@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the surrogate time-stepping hot path (BASELINE.json metric: rollout cell-updates/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...] [--dump-outputs DIR]
 
 One "step" = one time step of the rollout (7-channel input build -> conv surrogate -> curl/BC/
 un-scale head -> advection-diffusion update with the CFL dt) over one batch of synthetic T.
@@ -10,7 +10,9 @@ Default workload = BASELINE config 2: 512x512, batch 1, random-init primary netw
 With --gpus N every rank runs its own independent rollout (members differ in Ra and T0):
 no data-path collective, weak scaling, value = sum over ranks / max time over ranks.
 
-Prints ONE JSON line (rank 0).  `--impl reference` times the CPU port of the reference
+Prints ONE JSON line (rank 0).  With --dump-outputs DIR, rank 0 also writes what the timed rollout returned after its
+last timed step to DIR/<name>.npy (see dump_outputs); the inputs are seeded, so two builds can be compared output for
+output.  `--impl reference` times the CPU port of the reference
 (`oracle/ref_torch.py`, the reference is PyTorch and cannot travel to the GPU box) on the
 host cores, same metric and config.
 """
@@ -27,6 +29,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: nothing is written there
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -335,9 +338,22 @@ def launches_per_step(L_, R_, persistent_trunk=False):
     return 1 + 1 + (L_ if persistent_trunk else L_ * R_) + 3 + 2 * (L_ - 1) + 1 + 1
 
 
-def timed_rollout(net, H, W, B, rank, world, local, dev, K, Wm, flush, T0=None):
+def dump_outputs(path, ens):
+    """What a caller of EnsembleRollout holds after the last step: T and that step's u, v, p, V (float32 [B, H, W]) and each
+    member's dt (float64 [B]), one DIR/<name>.npy each.  Every rollout workload stays below 64 MB in all
+    (ensemble256: 32 members x 5 fields x 256 KiB = 40 MiB)."""
+    os.makedirs(path, exist_ok=True)
+    u, v, p, V = ens.fields()
+    out = {"T": ens.T, "u": u, "v": v, "p": p, "V": V, "dt": ens.last_dt()[(ens.n_done - 1) % 2]}
+    for name, t in out.items():
+        if t is not None:
+            np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
+
+
+def timed_rollout(net, H, W, B, rank, world, local, dev, K, Wm, flush, T0=None, dump=None):
     """Device-resident rollout of B members per rank: one CUDA graph per time step, L2 flushed (untimed) between steps,
-    per-step CUDA-event intervals summed.  Returns (device ms over K steps on this rank, wall s, finite, clock sampler)."""
+    per-step CUDA-event intervals summed.  Returns (device ms over K steps on this rank, wall s, finite, clock sampler).
+    With `dump` (a directory) the outputs of the last timed step are written there (dump_outputs)."""
     import torch.distributed as dist
 
     import pbml_mantle_convection_b200 as P
@@ -369,6 +385,8 @@ def timed_rollout(net, H, W, B, rank, world, local, dev, K, Wm, flush, T0=None):
         torch.cuda.synchronize()
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
     finite = bool(torch.isfinite(ens.T).all().item())
+    if dump:
+        dump_outputs(dump, ens)
     return dev_ms, wall, finite, clk
 
 
@@ -456,7 +474,8 @@ def run_ours(args, wl):
     net.up_staged = bool(args.up_staged)
     flush = torch.empty(256 * 1024 * 1024 // 4, dtype=torch.float32, device=dev)  # > 126 MB L2
     T0 = np.stack([P.synthetic_T0(H, W, seed=1 + rank * B + m) for m in range(B)])
-    dev_ms, wall, finite, clk = timed_rollout(net, H, W, B, rank, world, local, dev, K, Wm, flush, T0)
+    dev_ms, wall, finite, clk = timed_rollout(net, H, W, B, rank, world, local, dev, K, Wm, flush, T0,
+                                              dump=args.dump_outputs if rank == 0 else None)
 
     # ---- end to end through the drop-in TS call with HOST float64 tensors (advect_wi_gaia.py:590-616)
     ts = P.TS(net, P.ADNet(dev, CN_max=0.99), dev, ts=1, scale=True, p_pred=True, net="newfluidnet")
@@ -806,7 +825,11 @@ def main():
     ap.add_argument("--dt-sync", dest="dt_sync", default="flags", choices=["flags", "nccl"],
                     help="slab workloads with --halo p2p: global dt reduction inside the kernel (flags) or NCCL all_reduce per step")
     ap.add_argument("--no-sub-records", action="store_true", help="default workload: skip the slab8192 / ensemble256 sub-records")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="write the outputs of the last timed step of the GPU rollout to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.workload.startswith("slab")):
+        ap.error("--dump-outputs applies to the GPU rollout workloads (--impl ours, not slab)")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, wl)

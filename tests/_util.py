@@ -7,11 +7,30 @@ GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def load(name):
-    return dict(np.load(os.path.join(GOLDEN, name + ".npz"), allow_pickle=False))
+    """tests/golden/<name>.npz as a dict.  Weights that are exactly float32 values are stored as float32 to keep the files
+    small; they come back as the float64 arrays they were written from."""
+    d = dict(np.load(os.path.join(GOLDEN, name + ".npz"), allow_pickle=False))
+    return {k: v.astype(np.float64) if v.dtype == np.float32 else v for k, v in d.items()}
 
 
 def load_weights(name):
     return load(name + "_weights")
+
+
+def sample_index(H, W, n_interior, seed=0):
+    """Flat indices at which a full-size golden stores an H x W field: every boundary cell (the walls and the padding
+    modes act there) and `n_interior` interior cells drawn once with a fixed seed.  Sorted int32."""
+    ring = np.zeros((H, W), dtype=bool)
+    ring[0], ring[-1], ring[:, 0], ring[:, -1] = True, True, True, True
+    flat = np.flatnonzero(ring)
+    interior = np.flatnonzero(~ring)
+    pick = np.random.default_rng(seed).choice(interior, size=n_interior, replace=False)
+    return np.sort(np.concatenate([flat, pick])).astype(np.int32)
+
+
+def at(a, idx):
+    """The values of a 2-D field at the flat indices `idx` (how the full-size goldens store a field)."""
+    return np.asarray(a).reshape(-1)[idx]
 
 
 def split_weights(d, prefix="w::"):
@@ -57,14 +76,18 @@ LEARNED_CASES = ["learned_k5", "learned_k3_p", "learned_fluidnet"]
 
 
 def load_learned_case(tag):
-    """One case of tests/golden/learned.npz (whole learned-boundary networks): like load_unet_case."""
-    return load_unet_case(tag, "learned")
+    """One whole learned-boundary network case, tests/golden/<tag>.npz: like load_unet_case."""
+    return load_unet_case(tag)
 
 
-def load_unet_case(tag, file="unet"):
-    """One case of tests/golden/<file>.npz: (spec, input, {name: array for u, v, p, T}, state_dict as numpy)."""
-    g = load(file)
-    d = {k[len(tag) + 2:]: v for k, v in g.items() if k.startswith(tag + "::")}
+def load_unet_case(tag):
+    """One network case, tests/golden/<tag>.npz: (spec, input, {name: array for u, v, p, T}, state_dict as numpy).  The
+    input is not stored: it is redrawn from its seed exactly as make_golden.py drew it for the reference."""
+    import torch
+
+    d = load(tag)
     spec = spec_from_variant(d)
+    g = torch.Generator().manual_seed(int(d["inp_seed"]))
+    inp = torch.randn(*(int(n) for n in d["inp_shape"]), generator=g, dtype=torch.float64).numpy()
     outs = {n: d[n] for n in "uvpT" if n in d}
-    return spec, d["inp"], outs, split_weights(d)
+    return spec, inp, outs, split_weights(d)

@@ -42,6 +42,7 @@ def import_reference():
 
 P = import_reference()
 from oracle import ref_numpy as RN  # noqa: E402
+from tests._util import at, load_unet_case, sample_index  # noqa: E402
 
 RAQ, FKT, FKP = 6.79733173, 475523342.0, 2.58574662  # a CV simulation, load_fluidnet.ipynb:847
 
@@ -62,6 +63,22 @@ def make_net(spec: RN.NetSpec, seed=0, perturb_affine=True, cls=None):
                     p_.add_(0.2 * torch.randn(p_.shape, generator=g, dtype=p_.dtype))
     net.eval()
     return net
+
+
+def f32_if_exact(a):
+    """Store an array as float32 when that loses nothing (initial weights are float32 values widened by .double());
+    tests/_util.load widens it back."""
+    if a.dtype == np.float64 and a.size > 64 and np.array_equal(a.astype(np.float32).astype(np.float64), a):
+        return a.astype(np.float32)
+    return a
+
+
+def sample_fields(out, names, H, W, n_interior):
+    """Keep the full-size fields `names` of `out` only at sample_index(H, W, n_interior), stored as out["idx"]: every
+    golden file stays under 1 MB."""
+    out["idx"] = idx = sample_index(H, W, n_interior)
+    for k in names:
+        out[k] = at(out[k], idx)
 
 
 def set_grid(net, H, W):
@@ -170,7 +187,7 @@ def golden_ts_unmodified():
     yc = t64(yc_np).view(1, 1, H, W)
     x, dts, u, v, p, V = ts(t64(T0_np).view(1, 1, H, W), None, None, yc, t64(raq_nd), t64(fkt_nd), t64(fkp_nd),
                             t64(RAQ), t64(FKT), t64(FKP), xc, yc)
-    out = {"T0": T0_np, "xc": xc_np, "yc": yc_np, "params": np.array([RAQ, FKT, FKP]),
+    out = {"T0_seed": np.int64(1), "params": np.array([RAQ, FKT, FKP]),
            "T1": x[1][0, 0].numpy().copy(), "T5": x[5][0, 0].numpy().copy(),
            "dts": np.array([float(dts[i]) for i in range(1, 6)]),
            "u5": u[0, 0].numpy().copy(), "v5": v[0, 0].numpy().copy(), "p5": p[0, 0].numpy().copy(),
@@ -179,6 +196,7 @@ def golden_ts_unmodified():
     # numpy oracle, 1 step, vs TS
     Tn, dt_n, *_ = RN.ts_step(sd, spec, T0_np[None, None], xc_np, yc_np, RAQ, FKT, FKP)
     print(f"[ts128x506] numpy-oracle vs unmodified TS: T1 {np.abs(Tn[0,0]-out['T1']).max():.2e} dt {abs(dt_n-out['dts'][0])/out['dts'][0]:.2e}")
+    sample_fields(out, ["T1", "T5", "u5", "v5", "p5", "V5"], H, W, 15000)
     np.savez_compressed(os.path.join(HERE, "ts128x506.npz"), **out)
     np.savez_compressed(os.path.join(HERE, "ts128x506_weights.npz"), **sd)
 
@@ -279,6 +297,18 @@ def golden_ops():
     np.savez_compressed(os.path.join(HERE, "ops.npz"), **out)
 
 
+def save_case(tag, spec, inp_seed, inp, outputs, sd):
+    """One network case as tests/golden/<tag>.npz.  The input is stored as its seed and shape (tests/_util.load_unet_case
+    redraws it), the weights as float32 where that is exact."""
+    out = {"inp_seed": np.int64(inp_seed), "inp_shape": np.array(inp.shape, dtype=np.int64)}
+    out.update({n: t.numpy() for n, t in outputs if t is not None})
+    out["spec"] = np.array([spec.levels, spec.c_i, spec.c_h, spec.c_o, spec.repeats, spec.f, int(spec.use_symm), int(spec.p_pred)])
+    out["r_p"], out["loss_type"] = np.array(spec.r_p), np.array(spec.loss_type)
+    out["a_bound"] = np.float64(spec.a_bound)
+    out.update({"w::" + k: f32_if_exact(v_) for k, v_ in sd.items()})
+    np.savez_compressed(os.path.join(HERE, f"{tag}.npz"), **out)
+
+
 @torch.no_grad()
 def golden_unet():
     """The U-Net time-stepper surrogate (pytorch_networks_convae.py:1700-2068; SURVEY.md section 8f N4), small cases
@@ -291,7 +321,6 @@ def golden_unet():
         "unet_learned_k3": (RN.NetSpec(levels=3, c_i=10, c_h=8, c_o=3, r_p="learned", use_symm=False, repeats=2, f=3), 36, 50),
         "unet_learned_k5": (RN.NetSpec(levels=3, c_i=10, c_h=8, c_o=2, r_p="learned", use_symm=False, repeats=1, f=5, p_pred=False), 48, 58),
     }
-    out = {}
     for tag, (spec, H, W) in cases.items():
         net = make_net(spec, seed=5, cls=lambda *a, factor=2, **k: P.Unet(*a, **k))
         g = torch.Generator().manual_seed(9)
@@ -301,15 +330,7 @@ def golden_unet():
         res = RN.unet_forward(sd, spec, inp.numpy())
         print(f"[{tag}] numpy-oracle vs reference: " + " ".join(
             f"{n} {relerr(a, b.numpy()):.2e}" for n, a, b in zip("uvpT", res, (u, v, p_, T)) if b is not None))
-        out[f"{tag}::inp"] = inp.numpy()
-        for n, t in zip("uvpT", (u, v, p_, T)):
-            if t is not None:
-                out[f"{tag}::{n}"] = t.numpy()
-        out[f"{tag}::spec"] = np.array([spec.levels, spec.c_i, spec.c_h, spec.c_o, spec.repeats, spec.f, int(spec.use_symm), int(spec.p_pred)])
-        out[f"{tag}::r_p"], out[f"{tag}::loss_type"] = np.array(spec.r_p), np.array(spec.loss_type)
-        out[f"{tag}::a_bound"] = np.float64(spec.a_bound)
-        out.update({f"{tag}::w::" + k: v_ for k, v_ in sd.items()})
-    np.savez_compressed(os.path.join(HERE, "unet.npz"), **out)
+        save_case(tag, spec, 9, inp, zip("uvpT", (u, v, p_, T)), sd)
 
 
 @torch.no_grad()
@@ -321,7 +342,6 @@ def golden_learned():
         "learned_k3_p": (P.NewFluidNet, RN.NetSpec(levels=2, c_h=16, c_o=2, r_p="learned", use_symm=False, repeats=1, f=3), 36, 44),
         "learned_fluidnet": (P.FluidNet, RN.NetSpec(levels=2, c_h=8, c_o=2, r_p="learned", use_symm=False, repeats=2, f=3), 36, 44),
     }
-    out = {}
     for tag, (cls, spec, H, W) in cases.items():
         net = make_net(spec, seed=6, cls=cls)
         set_grid(net, H, W)
@@ -332,15 +352,7 @@ def golden_learned():
         res = RN.learned_net_forward(sd, spec, inp.numpy(), fluidnet=cls is P.FluidNet)
         print(f"[{tag}] numpy-oracle vs reference: " + " ".join(
             f"{n} {relerr(a, b.numpy()):.2e}" for n, a, b in zip("uvp", res, (u, v, p_)) if b is not None))
-        out[f"{tag}::inp"] = inp.numpy()
-        for n, t in zip("uvp", (u, v, p_)):
-            if t is not None:
-                out[f"{tag}::{n}"] = t.numpy()
-        out[f"{tag}::spec"] = np.array([spec.levels, spec.c_i, spec.c_h, spec.c_o, spec.repeats, spec.f, int(spec.use_symm), int(spec.p_pred)])
-        out[f"{tag}::r_p"], out[f"{tag}::loss_type"] = np.array(spec.r_p), np.array(spec.loss_type)
-        out[f"{tag}::a_bound"] = np.float64(spec.a_bound)
-        out.update({f"{tag}::w::" + k: v_ for k, v_ in sd.items()})
-    np.savez_compressed(os.path.join(HERE, "learned.npz"), **out)
+        save_case(tag, spec, 10, inp, zip("uvp", (u, v, p_)), sd)
 
 
 
@@ -429,14 +441,9 @@ def golden_noise():
         noise[tag] = {n: relerr(r.double().numpy(), g[n]) for n, r in zip("uvp", res) if r is not None}
     for file, cases, seed in (("learned", {"learned_k5": P.NewFluidNet, "learned_k3_p": P.NewFluidNet, "learned_fluidnet": P.FluidNet}, 6),
                               ("unet", {"unet_curl_p": None, "unet_curl_k5": None, "unet_mae": None, "unet_learned_k3": None, "unet_learned_k5": None}, 5)):
-        g = dict(np.load(os.path.join(HERE, file + ".npz")))
         for tag, cls in cases.items():
-            d = {k[len(tag) + 2:]: v for k, v in g.items() if k.startswith(tag + "::")}
-            s = d["spec"]
-            spec = RN.NetSpec(levels=int(s[0]), c_i=int(s[1]), c_h=int(s[2]), c_o=int(s[3]), repeats=int(s[4]), f=int(s[5]),
-                              use_symm=bool(s[6]), p_pred=bool(s[7]), r_p=str(d["r_p"]), loss_type=str(d["loss_type"]),
-                              a_bound=float(d["a_bound"]))
-            H, W = d["inp"].shape[-2:]
+            spec, inp, d, _w = load_unet_case(tag)
+            H, W = inp.shape[-2:]
             if file == "unet":
                 net = make_net(spec, seed=seed, cls=lambda *a, factor=2, **k: P.Unet(*a, **k))
                 net.float()
@@ -447,14 +454,15 @@ def golden_noise():
                 net = make_net(spec, seed=seed, cls=cls)
                 set_grid(net, H, W)
                 set_fp32(net)
-            res = net(torch.tensor(d["inp"], dtype=torch.float32))
+            res = net(torch.tensor(inp, dtype=torch.float32))
             noise[tag] = {n: relerr(r.double().numpy(), d[n]) for n, r in zip("uvpT", res) if r is not None and n in d}
     # rollouts: 128^2 (1 / 10 / 100 steps), 64x96 (1 / 10), 128x506 through the unmodified TS (5 steps)
     for tag, spec, H, W, keep in (("roll128", RN.NetSpec(), 128, 128, (1, 10, 100)), ("roll64x96", RN.NetSpec(levels=4), 64, 96, (1, 10)),
                                   ("ts128x506", RN.NetSpec(), 128, 506, (1, 5))):
         h64, h32, _ = _rollout_noise(spec, H, W, (RAQ, FKT, FKP), max(keep), RN.synthetic_T0(H, W, seed=1))
         g = dict(np.load(os.path.join(HERE, tag + ".npz")))
-        assert np.abs(h64[0]["T"] - g["T1"]).max() == 0.0, "noise run does not reproduce the stored golden"
+        T1 = at(h64[0]["T"], g["idx"]) if "idx" in g else h64[0]["T"]
+        assert np.abs(T1 - g["T1"]).max() == 0.0, "noise run does not reproduce the stored golden"
         noise[tag] = {f"step{i}": _field_noise(h64, h32, i - 1) for i in keep}
         mT64, Tp64, dTp64 = RN.diagnostics(h64[-1]["T"], RN.synthetic_grid(H, W)[1][:, 0])
         mT32, Tp32, dTp32 = RN.diagnostics(h32[-1]["T"], RN.synthetic_grid(H, W)[1][:, 0])
@@ -487,6 +495,7 @@ def golden_full_size():
     assert all(np.array_equal(sd[k], w128[k]) for k in sd), "roll512 must share roll128's weights"
     out = {"params": np.array([RAQ, FKT, FKP]), "T0_seed": np.int64(1), "u1": h64[0]["u"], "v1": h64[0]["v"], "p1": h64[0]["p"],
            "T1": h64[0]["T"], "T3": h64[2]["T"], "dts": np.array([h["dt"] for h in h64])}
+    sample_fields(out, ["u1", "v1", "p1", "T1", "T3"], H, W, 18000)
     np.savez_compressed(os.path.join(HERE, "roll512.npz"), **out)
     noise["roll512"] = {"step1": _field_noise(h64, h32, 0), "step3": _field_noise(h64, h32, 2)}
     print("[roll512]", noise["roll512"])
@@ -499,6 +508,7 @@ def golden_full_size():
                     f"m{m}_dts": np.array([h["dt"] for h in h64])})
         noise["ens256"][f"m{m}"] = _field_noise(h64, h32, 2)
         print(f"[ens256 m{m}]", noise["ens256"][f"m{m}"])
+    sample_fields(out, [f"m{m}_{n}3" for m in range(len(ENS256_PARAMS)) for n in "uvpT"], H, W, 5400)
     np.savez_compressed(os.path.join(HERE, "ens256.npz"), **out)
     path = os.path.join(HERE, "ref_fp32_noise.json")
     old = json.load(open(path)) if os.path.exists(path) else {}

@@ -1,5 +1,5 @@
 """Network-level parity of the rows SURVEY.md section 8f calls N1 and N4: whole learned-boundary networks and the U-Net
-drop-in against the vectors of the real reference (tests/golden/learned.npz, unet.npz), and the `net="unet"` branch of
+drop-in against the vectors of the real reference (tests/golden/learned_*.npz, unet_*.npz), and the `net="unet"` branch of
 TS.  Bound per field: max(1e-5, 1.5 x the reference's own fp32-vs-fp64 distance on the same case)
 (tests/golden/ref_fp32_noise.json).  Their host logic is also covered on the CPU (tests/test_host_logic_cpu.py)."""
 import numpy as np

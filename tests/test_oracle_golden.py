@@ -6,7 +6,7 @@ import torch
 
 from oracle import ref_numpy as RN
 from oracle import ref_torch as RT
-from tests._util import LEARNED_CASES, UNET_CASES, VARIANTS, load, load_learned_case, load_unet_case, load_weights, relerr, spec_from_variant, split_weights
+from tests._util import LEARNED_CASES, UNET_CASES, VARIANTS, at, load, load_learned_case, load_unet_case, load_weights, relerr, spec_from_variant, split_weights
 
 
 def test_ops_adnet():
@@ -89,16 +89,21 @@ def test_rollout_numpy_10_steps_small():
 
 
 def test_unmodified_TS_128x506():
+    """The reference's fields are stored at the sample indices g["idx"]."""
     g = load("ts128x506")
     spec = RN.NetSpec()
     W = RT.prepare_weights(load_weights("ts128x506"), spec)
     raq, fkt, fkp = g["params"]
-    T, dts, u, v, p, V, snaps = RT.rollout(W, spec, torch.tensor(g["T0"])[None, None], torch.tensor(g["xc"]),
-                                           torch.tensor(g["yc"]), float(raq), float(fkt), float(fkp), 5, keep=(1, 5))
-    assert np.abs(snaps[1][0, 0].numpy() - g["T1"]).max() < 1e-10
-    assert np.abs(snaps[5][0, 0].numpy() - g["T5"]).max() < 1e-9
-    assert relerr(u[0].numpy(), g["u5"]) < 1e-9 and relerr(p[0].numpy(), g["p5"]) < 1e-9
-    assert np.abs(V[0, 0].numpy() - g["V5"]).max() < 1e-12
+    xc, yc = RN.synthetic_grid(128, 506)
+    T0 = RN.synthetic_T0(128, 506, seed=int(g["T0_seed"]))
+    T, dts, u, v, p, V, snaps = RT.rollout(W, spec, torch.tensor(T0)[None, None], torch.tensor(xc), torch.tensor(yc),
+                                           float(raq), float(fkt), float(fkp), 5, keep=(1, 5))
+    idx = g["idx"]
+    assert np.abs(at(snaps[1][0, 0].numpy(), idx) - g["T1"]).max() < 1e-10
+    assert np.abs(at(snaps[5][0, 0].numpy(), idx) - g["T5"]).max() < 1e-9
+    assert relerr(at(u[0].numpy(), idx), g["u5"]) < 1e-9 and relerr(at(p[0].numpy(), idx), g["p5"]) < 1e-9
+    assert np.abs(at(V[0, 0].numpy(), idx) - g["V5"]).max() < 1e-12
+    assert np.allclose(dts, g["dts"], rtol=1e-9)
 
 
 @pytest.mark.parametrize("tag", UNET_CASES)
