@@ -56,8 +56,9 @@ enum { PBMC_LAYOUT_BLOCKED = 0, PBMC_LAYOUT_STAGED16 = 1 };
 enum { PBMC_HEAD_CURL = 0, PBMC_HEAD_MAE = 1 };
 /* pbmc_net.flags: PER_LAYER = never use the persistent trunk kernel; UP_STAGED = the bicubic kernel writes the up-sampled
  * levels as conv[1]'s fp16 hi|lo operand image (PBMC_LAYOUT_STAGED16) and conv[1] stages them with TMA bulk copies
- * (bit-identical results; measured neutral-to-slower, so off by default) */
-enum { PBMC_NET_TRUNK_PER_LAYER = 1, PBMC_NET_UP_STAGED = 2, PBMC_NET_TRUNK_BULK_LOADER = 4 };
+ * (bit-identical results; measured neutral-to-slower, so off by default); LEARNED = every conv is the learned 9-region
+ * convolution (r_p = "learned", see pbmc_net) */
+enum { PBMC_NET_TRUNK_PER_LAYER = 1, PBMC_NET_UP_STAGED = 2, PBMC_NET_TRUNK_BULK_LOADER = 4, PBMC_NET_LEARNED = 8 };
 /* pbmc_trunk_desc.loader: THREADS (default) = every worker loads its own pixels with ld.global.cg; BULK = TMA bulk copies
  * (cp.async.bulk + mbarrier transaction bytes): all raw rows of a layer are requested up front by one warp, land in the
  * stage slot their operand image will occupy and are converted in place.  Same results; measured SLOWER on B200 (77.9 vs
@@ -302,6 +303,14 @@ typedef struct {
   pbmc_layer conv0;
   pbmc_layer trunk[PBMC_MAX_LEVELS * PBMC_MAX_REPEATS]; /* [level][repeat] */
   pbmc_layer conv1, conv2, conv3;
+  /* flags & PBMC_NET_LEARNED only (NULL otherwise): the eight edge / corner filter sets of each layer in the wedge layout
+   * of pbmc_conv_edge9 (ops.pack_edge9_weights).  The layer's wpk / wpk_umma / wpk_row then hold the INTERIOR filters and
+   * its bias the learnable_bias. */
+  const float* wedge_conv0;
+  const float* wedge_trunk[PBMC_MAX_LEVELS * PBMC_MAX_REPEATS]; /* [level][repeat] */
+  const float* wedge_conv1;
+  const float* wedge_conv2;
+  const float* wedge_conv3;
 } pbmc_net;
 
 /* ------------------------------------------------------------------ A3/A5: the R FluidLayers of one pyramid level, ONE launch
@@ -341,6 +350,14 @@ size_t pbmc_workspace_bytes(const pbmc_net* net_h, int B, int H, int W);
  * < 0 on error.  Pure host computation: no GPU needed. */
 int pbmc_trunk_cta_budgets(const pbmc_net* net_h, int B, int H, int W, int* budgets);
 
+/* Learned-boundary networks (flags & PBMC_NET_LEARNED; r_p = "learned", every conv a BoundaryLearnedConvolution2D,
+ * pytorch_networks_convae.py:1022-1065, bc_x = bc_y = 1): every layer of the DAG is two launches on the same stream -- the
+ * interior filters through the conv kernels with zeros padding (pad_mode is not used), then the ring kernel of
+ * pbmc_conv_edge9 with the same sources, output and statistics.  The trunk always runs one launch per layer (the persistent
+ * kernel would consume each layer's GroupNorm statistics before the ring kernel repairs them) and the up-sampled levels stay
+ * blocked fp32 (PBMC_NET_UP_STAGED is ignored).  Supported when c_h <= 16, c_o <= 4, every source <= 128 channels and every
+ * pyramid level holds the reference's boundary strips (at least k rows and columns for k = 3, k + 1 for k = 5); otherwise
+ * pbmc_workspace_bytes returns 0 and pbmc_surrogate_forward / pbmc_rollout / pbmc_trunk_cta_budgets PBMC_ERR_UNSUPPORTED. */
 /* inp: blocked [B][ceil(c_i/4)][H][W][4] network input (A1's output, or a packed user tensor).
  * u,v,p plain [B][H][W] (mae head with p_pred: p too).  members may be NULL => scaler 1
  * (module-level NewFluidNet.forward does not un-scale).  uvmax may be NULL. */

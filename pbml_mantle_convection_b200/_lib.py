@@ -22,6 +22,7 @@ ACT_NONE, ACT_GELU = 0, 1
 HEAD_CURL, HEAD_MAE = 0, 1
 TRUNK_MODE = {"auto": 0, "per_layer": 1, "auto_bulk_loader": 4}  # pbmc_net.flags bits (PBMC_NET_TRUNK_*)
 NET_UP_STAGED = 2
+NET_LEARNED = 8
 CONV_IMPL = {"auto": 0, "ffma": 1, "umma_3xtf32": 2, "umma_bf16": 3, "umma_f16x2": 4,
              "row_f16x2": 5, "row_bf16": 6, "mux_f16x2": 7, "mux_bf16": 8}
 
@@ -53,7 +54,9 @@ class Net(C.Structure):
     _fields_ = [("levels", C.c_int), ("repeats", C.c_int), ("c_i", C.c_int), ("c_h", C.c_int), ("c_o", C.c_int),
                 ("ksize", C.c_int), ("pad_mode", C.c_int), ("head_kind", C.c_int), ("p_pred", C.c_int),
                 ("conv_impl", C.c_int), ("a_bound", C.c_float), ("flags", C.c_int), ("conv0", Layer),
-                ("trunk", Layer * (MAX_LEVELS * MAX_REPEATS)), ("conv1", Layer), ("conv2", Layer), ("conv3", Layer)]
+                ("trunk", Layer * (MAX_LEVELS * MAX_REPEATS)), ("conv1", Layer), ("conv2", Layer), ("conv3", Layer),
+                ("wedge_conv0", C.c_void_p), ("wedge_trunk", C.c_void_p * (MAX_LEVELS * MAX_REPEATS)),
+                ("wedge_conv1", C.c_void_p), ("wedge_conv2", C.c_void_p), ("wedge_conv3", C.c_void_p)]
 
 
 MAX_RANKS = 16

@@ -32,6 +32,7 @@ extern thread_local int g_conv_pdl_next;  // conv_mux.cu: the next mux launch us
 int build_input_enqueue(const float* T, const float* xc, const float* yc, const float* ycc, const pbmc_member* members, float* inp,
                         float* V, int B, int H, int W, void* zero, size_t zero_bytes, cudaStream_t st, bool pdl);  // pyramid.cu
 extern thread_local int g_stencil_pdl_next;  // stencil.cu: the next plain stencil launch uses programmatic dependent launch
+extern thread_local int g_edge9_pdl_next;    // conv_edge9.cu: the next ring launch uses programmatic dependent launch
 
 }  // namespace pbmc
 
@@ -212,12 +213,20 @@ int make_plan(const pbmc_net& n, int B, int H, int W, Plan& P) {
   if (n.levels < 1 || n.levels > PBMC_MAX_LEVELS || n.repeats < 1 || n.repeats > PBMC_MAX_REPEATS) return PBMC_ERR_UNSUPPORTED;
   if (n.c_h < 4 || n.c_h % 4 != 0 || n.c_i < 1 || n.c_o < 1 || n.c_o > 4) return PBMC_ERR_UNSUPPORTED;
   if (B <= 0 || H < 3 || W < 3) return PBMC_ERR_BAD_SHAPE;
+  const bool learned = (n.flags & PBMC_NET_LEARNED) != 0;
+  // learned 9-region convs: the ring kernel takes one 16-wide c_out tile and sources of <= 128 channels, and every level
+  // must hold the reference's boundary strips (pbmc_conv_edge9; the reference's strips would overlap otherwise)
+  const int strip = n.ksize == 5 ? 6 : n.ksize;
+  if (learned && (n.c_h > 16 || n.c_i > 128 || (n.ksize != 3 && n.ksize != 5) || n.levels + 1 > PBMC_MAX_SRC))
+    return PBMC_ERR_UNSUPPORTED;
+  if (learned && (H < strip || W < strip)) return PBMC_ERR_UNSUPPORTED;
   P.L = n.levels; P.R = n.repeats; P.CB = n.c_h / 4; P.CIB = (n.c_i + 3) / 4; P.COB3 = (n.c_o + 3) / 4;
   P.Hl[0] = H; P.Wl[0] = W;
   for (int l = 1; l < P.L; ++l) {
     P.Hl[l] = P.Hl[l - 1] / 2; P.Wl[l] = P.Wl[l - 1] / 2;
     if (P.Hl[l] < 1 || P.Wl[l] < 1) return PBMC_ERR_BAD_SHAPE;
-    if (n.pad_mode == PBMC_PAD_REFLECT && (P.Hl[l] <= n.ksize / 2 || P.Wl[l] <= n.ksize / 2)) return PBMC_ERR_BAD_SHAPE;
+    if (learned && (P.Hl[l] < strip || P.Wl[l] < strip)) return PBMC_ERR_UNSUPPORTED;
+    if (!learned && n.pad_mode == PBMC_PAD_REFLECT && (P.Hl[l] <= n.ksize / 2 || P.Wl[l] <= n.ksize / 2)) return PBMC_ERR_BAD_SHAPE;
   }
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes); return o; };
@@ -260,8 +269,24 @@ inline void fill_conv(pbmc_conv_desc& d, const pbmc_net& n, const pbmc_layer& L,
                       double* ostats, double* ochan, int epi_act) {
   memset(&d, 0, sizeof(d));
   d.B = B; d.H = H; d.W = W;
-  d.cout = L.cout; d.ksize = L.ksize; d.pad_mode = n.pad_mode; d.epi_act = epi_act; d.impl = n.conv_impl;
+  // a learned net's interior filters only produce the pixels whose window stays inside the image: zeros is the cheapest
+  d.cout = L.cout; d.ksize = L.ksize; d.pad_mode = (n.flags & PBMC_NET_LEARNED) ? PBMC_PAD_ZEROS : n.pad_mode; d.epi_act = epi_act; d.impl = n.conv_impl;
   d.wpk = L.wpk; d.wpk_umma = L.wpk_umma; d.wpk_row = L.wpk_row; d.bias = L.bias; d.out = out; d.out_stats = ostats; d.out_chan_sum = ochan;
+}
+
+// Second launch of a learned 9-region conv: the ring kernel (pbmc_conv_edge9) over the conv `d` just enqueued -- same
+// sources, output and statistics, which it repairs for the ring pixels
+inline int ring_enqueue(const pbmc_conv_desc& d, const float* wedge, cudaStream_t st, int pdl) {
+  pbmc_edge9_desc e;
+  memset(&e, 0, sizeof(e));
+  for (int s = 0; s < d.nsrc; ++s) e.src[s] = d.src[s];
+  e.nsrc = d.nsrc; e.B = d.B; e.H = d.H; e.W = d.W;
+  e.cout = d.cout; e.ksize = d.ksize; e.epi_act = d.epi_act;
+  e.wedge = wedge; e.bias = d.bias; e.out = d.out; e.out_stats = d.out_stats; e.out_chan_sum = d.out_chan_sum;
+  g_edge9_pdl_next = pdl;
+  const int rc = pbmc_conv_edge9(&e, st);
+  g_edge9_pdl_next = 0;
+  return rc;
 }
 }  // namespace
 
@@ -315,7 +340,9 @@ static bool level_cta_budgets(const pbmc_net& n, const Plan& P, int B, int H, in
   }
   // Persistent trunk kernels (csrc/conv_trunk.cu: the R layers of a level in one launch, grid barrier between layers)
   // need EVERY CTA of EVERY level resident at once: taken only when all levels have a budget and the budgets fit 148 SMs.
-  bool trunk_persistent = (n.flags & PBMC_NET_TRUNK_PER_LAYER) == 0 && CB == 4 && n.ksize == 3;
+  // Never for learned nets: the kernel consumes each layer's GroupNorm statistics at its grid barrier, before a ring
+  // kernel could repair them.
+  bool trunk_persistent = (n.flags & (PBMC_NET_TRUNK_PER_LAYER | PBMC_NET_LEARNED)) == 0 && CB == 4 && n.ksize == 3;
   // Their budgets are balanced on finish times, not on row counts: a level's kernel takes R x (the kernel's own per-layer
   // cost model, which moves in steps of a staging round of 5 rows), the coarse levels start after their pooling chain and
   // must still be up-sampled before conv[1] can begin.  Smallest common finish time whose CTA counts fit 148 SMs
@@ -421,7 +448,11 @@ static int surrogate_enqueue_on(pbmc_ctx* ctx, const pbmc_net& n, const Plan& P,
   //                         their SMs: 0.2011 -> 0.2003 ms/step in 10-step graphs); with one launch PER LAYER it cost
   //                         0.27 ms -- an early-resident CTA parked in griddepcontrol.wait took an SM from the other
   //                         levels' streams -- and stays off there
+  //  32  ring kernels of conv[0..3] (learned nets), each directly behind its interior conv: OFF -- measured slower on B200
+  //                         (paper network, 128x506, B = 1, 10-step graphs: 0.521 vs 0.474 ms/step; 32 x 256^2: 5.41 vs
+  //                         5.41 ms), so the ring kernels launch in plain stream order
   static const int chain_pdl = PBMC_DEV_KNOB("PBMC_CHAIN_PDL", 1 | 2 | 4 | 8 | 16);
+  const bool learned = (n.flags & PBMC_NET_LEARNED) != 0;
   auto F = [&](size_t off) { return reinterpret_cast<float*>(ws + off); };
   auto S = [&](int slot) { return reinterpret_cast<double*>(ws + P.stat_off(slot, B)); };
   double* chan_sum = reinterpret_cast<double*>(ws + P.chan_sum);
@@ -442,6 +473,7 @@ static int surrogate_enqueue_on(pbmc_ctx* ctx, const pbmc_net& n, const Plan& P,
     g_conv_pdl_next = 0;
     RC(rc0);
   }
+  if (learned) RC(ring_enqueue(d, n.wedge_conv0, st, chain_pdl & 32));
   PBMC_CUDA(cudaEventRecord(ctx->ev_fork[0], st));
 
   // pyramid levels (:1319-1327): level l runs on stream l (level 0 on the caller's stream)
@@ -467,7 +499,7 @@ static int surrogate_enqueue_on(pbmc_ctx* ctx, const pbmc_net& n, const Plan& P,
   // Off by default: measured neutral-to-slower in the whole step (512^2: 0.244-0.260 vs 0.241 ms; 32 x 256^2: 1.47 vs
   // 1.445 ms) -- conv[1] is paced by its MMA issue loop, not by its producers, and the operand-image writer of the
   // bicubic kernel stores 2 x 8 B per thread.  pbmc_net.flags & PBMC_NET_UP_STAGED turns it on (results are bit-identical).
-  up_staged = up_staged && (n.flags & PBMC_NET_UP_STAGED) != 0;
+  up_staged = up_staged && (n.flags & PBMC_NET_UP_STAGED) != 0 && !learned;  // the ring kernel reads blocked sources only
   const float* level_in[PBMC_MAX_LEVELS];
   level_in[0] = F(P.x0);
   for (int l = 0; l < L; ++l) {
@@ -521,6 +553,7 @@ static int surrogate_enqueue_on(pbmc_ctx* ctx, const pbmc_net& n, const Plan& P,
         g_conv_pdl_next = 0;
         RC(rct);
       }
+      if (learned) RC(ring_enqueue(d, n.wedge_trunk[l * PBMC_MAX_REPEATS + r], sl, 0));
     }
     if (l > 0) {
       pbmc_src us = make_src(F(P.ping[l][(R - 1) & 1]), CB, PBMC_XFORM_GN_GELU, S(1 + l * R + R - 1),
@@ -550,6 +583,7 @@ static int surrogate_enqueue_on(pbmc_ctx* ctx, const pbmc_net& n, const Plan& P,
     g_conv_pdl_next = 0;
     RC(rc1);
   }
+  if (learned) RC(ring_enqueue(d, n.wedge_conv1, st, chain_pdl & 32));
   // gn[0] + act folded into conv[2]'s load; conv[2] + act (:1336-1340)
   fill_conv(d, n, n.conv2, B, H, W, F(P.h2), nullptr, nullptr, PBMC_ACT_GELU);
   d.nsrc = 1;
@@ -560,6 +594,7 @@ static int surrogate_enqueue_on(pbmc_ctx* ctx, const pbmc_net& n, const Plan& P,
     g_conv_pdl_next = 0;
     RC(rc2);
   }
+  if (learned) RC(ring_enqueue(d, n.wedge_conv2, st, chain_pdl & 32));
   // conv[3] (:1342) with per-channel sums for the zero-mean (:1343)
   fill_conv(d, n, n.conv3, B, H, W, F(P.h3), nullptr, chan_sum, PBMC_ACT_NONE);
   d.nsrc = 1;
@@ -570,6 +605,7 @@ static int surrogate_enqueue_on(pbmc_ctx* ctx, const pbmc_net& n, const Plan& P,
     g_conv_pdl_next = 0;
     RC(rc3);
   }
+  if (learned) RC(ring_enqueue(d, n.wedge_conv3, st, chain_pdl & 32));
   g_conv_pdl_next = chain_pdl & 8;
   {
     const int rch = pbmc_head(F(P.h3), chan_sum, members, n.a_bound, n.head_kind, n.p_pred, u, v, p, uvmax, B, H, W, st);

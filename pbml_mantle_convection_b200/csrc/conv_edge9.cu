@@ -57,6 +57,10 @@ __global__ void __launch_bounds__(E9_THREADS) conv_edge9_kernel(const __grid_con
   const int H = p.H, W = p.W, k = p.k, pd = (k - 1) / 2, pad = k == 5 ? k + 1 : k, kk = k * k;
   const long ring = 2L * pd * W + 2L * pd * (H - 2 * pd);
   const size_t plane = (size_t)H * W;
+  // programmatic dependent launch (no-ops otherwise): everything below reads what the interior conv (or earlier) wrote;
+  // the next kernel of the chain does its own griddepcontrol.wait before it reads this kernel's output
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
 
   // GroupNorm coefficients of every transformed source
   for (int e = tid; e < p.nsrc * E9_MAXC; e += E9_THREADS) {
@@ -169,6 +173,10 @@ __global__ void __launch_bounds__(E9_THREADS) conv_edge9_kernel(const __grid_con
 
 }  // namespace pbmc
 
+namespace pbmc {
+thread_local int g_edge9_pdl_next = 0;  // set by api.cu right before the launch it applies to
+}  // namespace pbmc
+
 using namespace pbmc;
 
 extern "C" int pbmc_conv_edge9(const pbmc_edge9_desc* d, void* stream) {
@@ -200,8 +208,10 @@ extern "C" int pbmc_conv_edge9(const pbmc_edge9_desc* d, void* stream) {
   const long ring = 2L * pd * d->W + 2L * pd * (d->H - 2 * pd);
   const size_t smem = (size_t)E9_PX * d->ksize * d->ksize * 16 * sizeof(float);
   dim3 grid((unsigned)((ring + E9_PX - 1) / E9_PX), d->B);
+  const bool pdl = g_edge9_pdl_next != 0;
+  g_edge9_pdl_next = 0;
   if (grid.y > 65535) return PBMC_ERR_BAD_SHAPE;
-  conv_edge9_kernel<<<grid, E9_THREADS, smem, (cudaStream_t)stream>>>(p);
+  PBMC_CUDA(launch_maybe_pdl(conv_edge9_kernel, grid, dim3(E9_THREADS), smem, (cudaStream_t)stream, pdl, p));
   PBMC_CHECK_LAUNCH("conv_edge9_kernel");
   return PBMC_OK;
 }

@@ -16,7 +16,7 @@ from . import ops
 
 
 class _PackedLayer:
-    def __init__(self, w_full, bias, gamma, beta, src_channels, dev):
+    def __init__(self, w_full, bias, gamma, beta, src_channels, dev, w_edge=None):
         cout, _, k, _ = w_full.shape
         self.wpk = ops.pack_conv_weight(w_full.to(dev), src_channels)
         self.bias = ops.pad_vec(bias, cout, dev)
@@ -28,6 +28,8 @@ class _PackedLayer:
                          if ops.umma_supported(cout, src_channels) else None)
         self.wpk_row = (ops.pack_conv_weight_row(w_full.to(dev), src_channels)
                         if ops.row_supported(cout, k, src_channels) else None)
+        # learned 9-region conv: w_full is the interior filter bank, w_edge the eight edge / corner banks
+        self.wedge = ops.pack_edge9_weights([w.to(dev) for w in w_edge], src_channels) if w_edge is not None else None
 
     def c(self):
         s = L.Layer()
@@ -39,21 +41,25 @@ class _PackedLayer:
 
 
 class PackedNetwork:
-    """Repacked filters / bias / GroupNorm affine of every layer of a (non-learned) NewFluidNet: conv0, trunk[l][r],
-    conv1, conv2, conv3 as `_PackedLayer`s.  Needs no library context: the fused engine and the slab-decomposed
-    surrogate both start from it."""
+    """Repacked filters / bias / GroupNorm affine of every layer of a NewFluidNet: conv0, trunk[l][r], conv1, conv2, conv3
+    as `_PackedLayer`s (learned-boundary nets: interior filters, edge filter image `wedge` and learnable bias).  Needs no
+    library context: the fused engine and the slab-decomposed surrogate both start from it."""
 
 
 def pack_network(m, dev) -> PackedNetwork:
-    if m.r_p == "learned":
-        raise NotImplementedError("fused engine covers zeros/replicate/reflect padding; r_p='learned' "
-                                  "runs through BoundaryLearnedConvolution2D.forward")
-    from .symmetric_layers_torch import _check_conv_supported
+    from .symmetric_layers_torch import _check_conv_supported, full_weight
 
     f32 = lambda t: None if t is None else t.detach().to(dev, torch.float32)
 
+    def learned(conv, gamma, beta, src_channels):
+        # BoundaryLearnedConvolution2D: regions in conv._REGIONS order = interior, then ops.EDGE9_REGIONS
+        wf = [f32(full_weight(getattr(conv, name))) for name in conv._REGIONS]
+        return _PackedLayer(wf[0], f32(conv.learnable_bias).reshape(-1), gamma, beta, src_channels, dev, wf[1:])
+
     def fluid(fl, cin):
         conv, gn = fl.layers[0], fl.layers[1]
+        if m.r_p == "learned":
+            return learned(conv, f32(gn.weight), f32(gn.bias), [cin])
         _check_conv_supported(conv)  # dilation / stride / groups != 1 would silently compute another operator
         w = f32(conv.weight)
         if getattr(conv, "symmetry", None) is not None:
@@ -64,6 +70,11 @@ def pack_network(m, dev) -> PackedNetwork:
     pk.conv0 = fluid(m.conv[0], m.c_i)
     pk.trunk = [[fluid(m.convs[l][r], m.c_h) for r in range(m.repeats)] for l in range(m.levels)]
     c1, c2, c3 = m.conv[1], m.conv[2], m.conv[3]
+    if m.r_p == "learned":
+        pk.conv1 = learned(c1, f32(m.gn[0].weight), f32(m.gn[0].bias), [m.c_h] * m.levels + [m.c_i])
+        pk.conv2 = learned(c2, None, None, [m.c_h])
+        pk.conv3 = learned(c3, None, None, [m.c_h])
+        return pk
     for c in (c1, c2, c3):
         _check_conv_supported(c)
     pk.conv1 = _PackedLayer(f32(c1.weight), f32(c1.bias), f32(m.gn[0].weight), f32(m.gn[0].bias),
@@ -71,6 +82,23 @@ def pack_network(m, dev) -> PackedNetwork:
     pk.conv2 = _PackedLayer(f32(c2.weight), f32(c2.bias), None, None, [m.c_h], dev)
     pk.conv3 = _PackedLayer(f32(c3.weight), f32(c3.bias), None, None, [m.c_h], dev)
     return pk
+
+
+def shape_desc(m):
+    """pbmc_net of `m` with its shape fields and flags only (no weights): enough for the host-side queries
+    (pbmc_workspace_bytes, pbmc_trunk_cta_budgets), no device needed."""
+    n = L.Net()
+    n.levels, n.repeats, n.c_i, n.c_h, n.c_o = m.levels, m.repeats, m.c_i, m.c_h, m.c_o
+    learned = m.r_p == "learned"
+    n.ksize = m.conv[0].layers[0].k if learned else m.conv[0].layers[0].kernel_size[0]
+    n.pad_mode = 0 if learned else L.PAD[m.r_p]  # learned: not used (the interior convs run with zeros padding)
+    n.flags = L.NET_LEARNED if learned else 0
+    return n
+
+
+def fused_supported(m, B, H, W) -> bool:
+    """Whether the fused engine (pbmc_surrogate_forward / pbmc_rollout) takes network `m` at this size."""
+    return L.load().pbmc_workspace_bytes(C.byref(shape_desc(m)), B, H, W) > 0
 
 
 class SurrogateEngine:
@@ -124,20 +152,24 @@ class SurrogateEngine:
 
     def _build_desc(self):
         m = self.net_module
-        n = L.Net()
-        n.levels, n.repeats, n.c_i, n.c_h, n.c_o = m.levels, m.repeats, m.c_i, m.c_h, m.c_o
+        n = shape_desc(m)
         n.ksize = self.conv0.ksize
-        n.pad_mode = L.PAD[m.r_p]
         n.head_kind = L.HEAD_CURL if m.loss_type == "curl" else L.HEAD_MAE
         n.p_pred = int(bool(m.p_pred))
         n.conv_impl = L.CONV_IMPL[self.conv_impl]
-        n.flags = L.TRUNK_MODE[self.trunk_mode] | (L.NET_UP_STAGED if self.up_staged else 0)  
+        n.flags |= L.TRUNK_MODE[self.trunk_mode] | (L.NET_UP_STAGED if self.up_staged else 0)
         n.a_bound = float(m.a_bound)
         n.conv0 = self.conv0.c()
         for l in range(m.levels):
             for r in range(m.repeats):
                 n.trunk[l * L.MAX_REPEATS + r] = self.trunk[l][r].c()
         n.conv1, n.conv2, n.conv3 = self.conv1.c(), self.conv2.c(), self.conv3.c()
+        if m.r_p == "learned":
+            n.wedge_conv0 = L.ptr(self.conv0.wedge)
+            for l in range(m.levels):
+                for r in range(m.repeats):
+                    n.wedge_trunk[l * L.MAX_REPEATS + r] = L.ptr(self.trunk[l][r].wedge)
+            n.wedge_conv1, n.wedge_conv2, n.wedge_conv3 = (L.ptr(x.wedge) for x in (self.conv1, self.conv2, self.conv3))
         self.desc = n
 
     def set_conv_impl(self, impl):

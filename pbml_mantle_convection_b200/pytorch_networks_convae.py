@@ -21,7 +21,7 @@ import torch.nn as nn
 
 from . import _lib as L
 from . import ops
-from .engine import Grid, RolloutState, SurrogateEngine
+from .engine import Grid, RolloutState, SurrogateEngine, fused_supported
 from .symmetric_layers_torch import SymmetricConv2d, conv_module_forward, full_weight
 
 _ACTS = {"selu": nn.SELU, "tanh": nn.Tanh, "elu": nn.ELU, "silu": nn.SiLU, "relu": nn.ReLU, "gelu": nn.GELU}
@@ -742,7 +742,9 @@ class TS(nn.Module):
         grid = self._get_grid(xc, yc, ycc, dev)
         fl = lambda t: float(t)
         advect = self.ad is not None and self.net == "newfluidnet"
-        fused = isinstance(stokes, NewFluidNet) and stokes.r_p != "learned" and grid.separable
+        # learned-boundary nets: where the engine's ring kernel takes every level (else the per-step path below)
+        fused = (isinstance(stokes, NewFluidNet) and grid.separable
+                 and (stokes.r_p != "learned" or fused_supported(stokes, B, H, W)))
         cn_max = self.ad.CN_max if advect else 0.0
         n = self.ts
         if fused and advect:

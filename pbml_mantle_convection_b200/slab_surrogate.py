@@ -108,6 +108,9 @@ class SlabSurrogate:
     params: (RaQ, gamma, beta).  State: `T` (local [1, rows, W] float32, ghost rows valid)."""
 
     def __init__(self, net, H, W, x1d, y1d, params, comm, device, cn_max=0.99):
+        if net.r_p == "learned":
+            raise NotImplementedError("SlabSurrogate covers zeros / replicate / reflect padding; a learned-boundary network "
+                                      "(r_p='learned') runs on one GPU per grid (TS, EnsembleRollout)")
         self.net, self.comm, self.device = net, comm, torch.device(device)
         self.H, self.W, self.cn_max = H, W, float(cn_max)
         self.rank, self.world = comm.rank, comm.world
