@@ -376,6 +376,39 @@ int pbmc_rollout(pbmc_ctx* ctx, const pbmc_net* net_h, const pbmc_member* member
                  int nslots, int first_step, int n_steps, double* dt_seq, int dt_seq_rows, float* u, float* v, float* p, float* V,
                  void* workspace, size_t workspace_bytes, int B, int H, int W, void* stream);
 
+/* ------------------------------------------------------------------ run to a simulated end time
+ * The reference driver's loop per member (advect_wi_gaia.py:583-668): `while t < t_end` (and steps < max_steps), after
+ * every step t += dt, mean-T logged, and a snapshot whenever t > save_t (then save_t = t + save_every; save_t = 0 at the
+ * start).  One clock per member, in device memory, read and updated by the device after every step, so a captured k-step
+ * graph keeps working across replays.  A member that has stopped ("frozen") still goes through the surrogate (the batch
+ * shape is fixed) but its T stays bit-identical, its dt_seq rows are written as 0 and nothing is logged for it.
+ *   active    1 while the member takes steps: t < t_end && steps < max_steps (recomputed after every step)
+ *   snaps     snapshots taken so far; snapshot j lives in ring slot j % snap_slots
+ *   drained   snapshots the caller has read (the caller advances it); a due snapshot is skipped, and overflow set, when
+ *             snaps - drained == snap_slots: a full ring is never written past
+ *   part      scratch of the per-step mean-T reduction */
+#define PBMC_CLOCK_PARTS 64
+typedef struct {
+  double t, t_end, save_t, save_every;
+  int64_t steps, max_steps, snaps, drained;
+  int active, overflow;
+  double part[PBMC_CLOCK_PARTS];
+} pbmc_member_clock;
+
+/* pbmc_rollout plus a clock per member.  Behind every step's stencil, on the same stream:
+ *   meanT_seq  [dt_seq_rows][B] doubles, indexed like dt_seq: mean of the member's new T (float64, fixed summation order)
+ *   snap_ring  float [snap_slots][B][nch][H][W], nch = 4 (T, u, v, p) with p, else 3: T after the step, u, v, p of the step
+ *   snap_meta  [snap_slots][B][2] doubles = (step number, t) of each ring slot
+ * Refused before any CUDA call: NULL clock / dt_seq / meanT_seq / snap_ring / snap_meta (PBMC_ERR_NULL_POINTER),
+ * snap_slots < 1 (PBMC_ERR_BAD_SHAPE), per_member_dt = 0 with B > 1 (PBMC_ERR_UNSUPPORTED: freezing one member would
+ * change the others' batch-global dt). */
+int pbmc_rollout_clocked(pbmc_ctx* ctx, const pbmc_net* net_h, const pbmc_member* members, const float* xc, const float* yc,
+                         const float* ycc, const float* xcoef, const float* ycoef, double dx_min, double cn_max, int per_member_dt,
+                         float* T_seq, int nslots, int first_step, int n_steps, double* dt_seq, int dt_seq_rows, float* u, float* v,
+                         float* p, float* V, void* workspace, size_t workspace_bytes, int B, int H, int W,
+                         pbmc_member_clock* clock, double* meanT_seq, float* snap_ring, double* snap_meta, int snap_slots,
+                         void* stream);
+
 #ifdef __cplusplus
 }
 #endif

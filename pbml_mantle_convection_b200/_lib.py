@@ -79,7 +79,16 @@ class TrunkDesc(C.Structure):
                 ("impl", C.c_int), ("max_ctas", C.c_int), ("pre_zeroed", C.c_int), ("loader", C.c_int), ("reserved", C.c_int)]
 
 
-_STRUCTS = {"pbmc_edge9_desc": Edge9Desc, "pbmc_trunk_desc": TrunkDesc, "pbmc_slab_sync": SlabSync, "pbmc_member": Member, "pbmc_src": Src, "pbmc_conv_desc": ConvDesc, "pbmc_layer": Layer, "pbmc_net": Net}
+CLOCK_PARTS = 64
+
+
+class MemberClock(C.Structure):
+    _fields_ = [("t", C.c_double), ("t_end", C.c_double), ("save_t", C.c_double), ("save_every", C.c_double),
+                ("steps", C.c_int64), ("max_steps", C.c_int64), ("snaps", C.c_int64), ("drained", C.c_int64),
+                ("active", C.c_int), ("overflow", C.c_int), ("part", C.c_double * CLOCK_PARTS)]
+
+
+_STRUCTS = {"pbmc_member_clock": MemberClock, "pbmc_edge9_desc": Edge9Desc, "pbmc_trunk_desc": TrunkDesc, "pbmc_slab_sync": SlabSync, "pbmc_member": Member, "pbmc_src": Src, "pbmc_conv_desc": ConvDesc, "pbmc_layer": Layer, "pbmc_net": Net}
 
 # name -> (restype, argtypes); every symbol declared in include/pbmc.h
 _vp, _i, _d, _f, _sz = C.c_void_p, C.c_int, C.c_double, C.c_float, C.c_size_t
@@ -120,6 +129,8 @@ SIGNATURES = {
     "pbmc_surrogate_forward": (_i, [_vp, C.POINTER(Net), _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _i, _i, _i, _vp]),
     "pbmc_rollout": (_i, [_vp, C.POINTER(Net), _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _vp, _i, _i, _i, _vp, _i, _vp, _vp,
                           _vp, _vp, _vp, _sz, _i, _i, _i, _vp]),
+    "pbmc_rollout_clocked": (_i, [_vp, C.POINTER(Net), _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _vp, _i, _i, _i, _vp, _i, _vp,
+                                  _vp, _vp, _vp, _vp, _sz, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _vp]),
 }
 
 _lib = None

@@ -13,7 +13,7 @@ CSRC = os.path.join(PKG, "csrc")
 INCLUDE = os.path.join(ROOT, "include")
 LIB = os.path.join(PKG, "libpbmc.so")
 STAMP = os.path.join(PKG, "csrc", ".build_stamp")
-SOURCES = ["api.cu", "conv_ffma.cu", "conv_umma.cu", "conv_row.cu", "conv_mux.cu", "conv_trunk.cu", "conv_edge9.cu", "pyramid.cu", "head.cu", "stencil.cu"]
+SOURCES = ["api.cu", "conv_ffma.cu", "conv_umma.cu", "conv_row.cu", "conv_mux.cu", "conv_trunk.cu", "conv_edge9.cu", "pyramid.cu", "head.cu", "stencil.cu", "clock.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "--use_fast_math=false",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-O2", "--expt-relaxed-constexpr"]
 

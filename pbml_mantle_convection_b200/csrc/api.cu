@@ -33,6 +33,9 @@ int build_input_enqueue(const float* T, const float* xc, const float* yc, const 
                         float* V, int B, int H, int W, void* zero, size_t zero_bytes, cudaStream_t st, bool pdl);  // pyramid.cu
 extern thread_local int g_stencil_pdl_next;  // stencil.cu: the next plain stencil launch uses programmatic dependent launch
 extern thread_local int g_edge9_pdl_next;    // conv_edge9.cu: the next ring launch uses programmatic dependent launch
+int clock_enqueue(pbmc_member_clock* clk, const float* Tin, float* Tout, const float* u, const float* v, const float* p,
+                  double* dt_row, double* meanT_row, float* ring, double* meta, int slots, int B, int H, int W,
+                  cudaStream_t st);  // clock.cu
 
 }  // namespace pbmc
 
@@ -71,6 +74,7 @@ extern "C" size_t pbmc_sizeof(const char* name) {
   if (!strcmp(name, "pbmc_slab_sync")) return sizeof(pbmc_slab_sync);
   if (!strcmp(name, "pbmc_trunk_desc")) return sizeof(pbmc_trunk_desc);
   if (!strcmp(name, "pbmc_edge9_desc")) return sizeof(pbmc_edge9_desc);
+  if (!strcmp(name, "pbmc_member_clock")) return sizeof(pbmc_member_clock);
   return 0;
 }
 
@@ -645,12 +649,24 @@ __global__ void uvmax_batch_reduce_kernel(uint32_t* uv, int B) {
 }
 }  // namespace pbmc
 
-extern "C" int pbmc_rollout(pbmc_ctx* ctx, const pbmc_net* net, const pbmc_member* members, const float* xc,
-                            const float* yc, const float* ycc, const float* xcoef, const float* ycoef, double dx_min,
-                            double cn_max,
-                            int per_member_dt, float* T_seq, int nslots, int first_step, int n_steps, double* dt_seq,
-                            int dt_seq_rows, float* u, float* v, float* p, float* V, void* workspace, size_t workspace_bytes, int B, int H,
-                            int W, void* stream) {
+namespace {
+// The clock arguments of pbmc_rollout_clocked (clock == NULL: plain pbmc_rollout)
+struct ClockArgs {
+  pbmc_member_clock* clock;
+  double* meanT_seq;
+  float* snap_ring;
+  double* snap_meta;
+  int snap_slots;
+};
+}  // namespace
+
+// pbmc_rollout and pbmc_rollout_clocked: the same launches in the same order; a clock adds its two launches behind every
+// step's stencil
+static int rollout_impl(pbmc_ctx* ctx, const pbmc_net* net, const pbmc_member* members, const float* xc, const float* yc,
+                        const float* ycc, const float* xcoef, const float* ycoef, double dx_min, double cn_max,
+                        int per_member_dt, float* T_seq, int nslots, int first_step, int n_steps, double* dt_seq,
+                        int dt_seq_rows, float* u, float* v, float* p, float* V, void* workspace, size_t workspace_bytes,
+                        int B, int H, int W, const ClockArgs& clk, void* stream) {
   if (!ctx || !net || !members || !xc || !yc || !ycc || !xcoef || !ycoef || !T_seq || !u || !v || !workspace) return PBMC_ERR_NULL_POINTER;
   if (nslots < 2 || first_step < 1 || n_steps < 0 || !(dx_min > 0.0)) return PBMC_ERR_BAD_SHAPE;
   if (dt_seq != nullptr && dt_seq_rows < first_step + n_steps - 1) return PBMC_ERR_BAD_SHAPE;  // step i writes row i - 1
@@ -691,6 +707,10 @@ extern "C" int pbmc_rollout(pbmc_ctx* ctx, const pbmc_net* net, const pbmc_membe
                                           dt_seq ? dt_seq + (size_t)(i - 1) * B : nullptr, B, H, W, st);
       g_stencil_pdl_next = 0;
       RC(rcs);
+      // plain stream order behind the stencil; the next step's input build is PDL-launched behind the commit kernel
+      if (clk.clock)
+        RC(clock_enqueue(clk.clock, Tin, Tout, u, v, p, dt_seq + (size_t)(i - 1) * B, clk.meanT_seq + (size_t)(i - 1) * B,
+                         clk.snap_ring, clk.snap_meta, clk.snap_slots, B, H, W, st));
     }
     return PBMC_OK;
   };
@@ -699,4 +719,29 @@ extern "C" int pbmc_rollout(pbmc_ctx* ctx, const pbmc_net* net, const pbmc_membe
   cudaEventRecord(ctx->ev_out, st);
   cudaStreamWaitEvent(caller, ctx->ev_out, 0);
   return rc;
+}
+
+extern "C" int pbmc_rollout(pbmc_ctx* ctx, const pbmc_net* net, const pbmc_member* members, const float* xc,
+                            const float* yc, const float* ycc, const float* xcoef, const float* ycoef, double dx_min,
+                            double cn_max,
+                            int per_member_dt, float* T_seq, int nslots, int first_step, int n_steps, double* dt_seq,
+                            int dt_seq_rows, float* u, float* v, float* p, float* V, void* workspace, size_t workspace_bytes, int B, int H,
+                            int W, void* stream) {
+  const ClockArgs none = {nullptr, nullptr, nullptr, nullptr, 0};
+  return rollout_impl(ctx, net, members, xc, yc, ycc, xcoef, ycoef, dx_min, cn_max, per_member_dt, T_seq, nslots, first_step,
+                      n_steps, dt_seq, dt_seq_rows, u, v, p, V, workspace, workspace_bytes, B, H, W, none, stream);
+}
+
+extern "C" int pbmc_rollout_clocked(pbmc_ctx* ctx, const pbmc_net* net, const pbmc_member* members, const float* xc,
+                                    const float* yc, const float* ycc, const float* xcoef, const float* ycoef, double dx_min,
+                                    double cn_max, int per_member_dt, float* T_seq, int nslots, int first_step, int n_steps,
+                                    double* dt_seq, int dt_seq_rows, float* u, float* v, float* p, float* V, void* workspace,
+                                    size_t workspace_bytes, int B, int H, int W, pbmc_member_clock* clock, double* meanT_seq,
+                                    float* snap_ring, double* snap_meta, int snap_slots, void* stream) {
+  if (!clock || !dt_seq || !meanT_seq || !snap_ring || !snap_meta) return PBMC_ERR_NULL_POINTER;
+  if (snap_slots < 1) return PBMC_ERR_BAD_SHAPE;
+  if (!per_member_dt && B > 1) return PBMC_ERR_UNSUPPORTED;  // a frozen member would still set the others' batch-global dt
+  const ClockArgs clk = {clock, meanT_seq, snap_ring, snap_meta, snap_slots};
+  return rollout_impl(ctx, net, members, xc, yc, ycc, xcoef, ycoef, dx_min, cn_max, per_member_dt, T_seq, nslots, first_step,
+                      n_steps, dt_seq, dt_seq_rows, u, v, p, V, workspace, workspace_bytes, B, H, W, clk, stream);
 }

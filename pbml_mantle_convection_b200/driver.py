@@ -14,11 +14,14 @@ afterwards (`.ipynb_checkpoints/load_advection_results-checkpoint.ipynb:243-326`
 with the same cadence rules: a snapshot whenever `t > save_t` (then `save_t = t + save_every`), the pickles rewritten
 whenever `t > write_t` and once more at the end (`:654-677`).
 
-Two ways to advance:
+Three ways to advance:
   * `attempt(ts_net, ...)`  -- one `ts_net(...)` call per step exactly like `:590-593` (host tensors in, fields read
     back every step); any callable with `TS.forward`'s signature works (the drop-in `TS`, or the reference's own).
   * `attempt_resident(ens, ...)` -- an `EnsembleRollout` advances `check_every` steps per CUDA-graph replay with T, u, v
     and dt on the device; host work (time bookkeeping, cadence checks, snapshots) happens once per block.
+  * `attempt_ensemble(ens, ...)` -- every member of an `EnsembleRollout` runs to its own `t_end` on a device-side clock
+    (`EnsembleRollout.start_clock`): per-step t / mean-T and snapshots at the exact steps, the four pickles per member,
+    read back once per block of `check_every` steps.
 
 External energy solver (the `ML_STOKES` / `ML_PRE` modes and the `intervene_TS` interventions of mode "ML", `:486-505`,
 `:618-630`): the reference calls GAIA's `sim.doTimestep()` with the surrogate's velocities already written into the state
@@ -166,3 +169,59 @@ def attempt_resident(ens, xcc, ycc, t_end, out_dir, save_every=0.0, write_every=
             write_logs(out_dir, mode, snapshots, TS_vec, t_vec, T_vec)
     write_logs(out_dir, mode, snapshots, TS_vec, t_vec, T_vec)
     return t, n_step, (snapshots, TS_vec, t_vec, T_vec)
+
+
+def attempt_ensemble(ens, xcc, ycc, t_end, out_dir, save_every=0.0, write_every=0.0, mode="ML", t=0.0, n_step=0,
+                     check_every=10, max_steps=None):
+    """`attempt` for every member of a device-resident `EnsembleRollout` at once.  Member m runs `while t < t_end[m]` (and
+    n_step < max_steps) on its own device-side clock; t_end, save_every, t and n_step are scalars or one value per member.
+    Writes the reference's four pickles of member m into `out_dir/member_<m>/` with `attempt`'s cadence: the initial entry
+    and snapshot, one t_vec / T_vec entry per step the member took, snapshots at the steps where t > save_t.  Blocks of
+    `check_every` steps run as one CUDA-graph replay each, then the block's logs are drained; `t > write_t` is evaluated at
+    block ends (it decides when intermediate pickles are written, not their final content).  A TS_vec entry is the block's
+    wall time over the steps the member took in it.  Returns (t [B], n_step [B], [logs of member m]) with logs as in
+    `attempt`."""
+    B, H, W = ens.B, ens.H, ens.W
+    n = H * W
+    k = int(check_every)
+    logs = [_new_logs(mode) for _ in range(B)]
+    dirs = [os.path.join(out_dir, f"member_{m}") for m in range(B)]
+    T0 = ens.T.double().cpu().numpy().reshape(B, n)
+    t0 = np.broadcast_to(np.asarray(t, dtype=np.float64), (B,)).copy()
+    for m, (snapshots, TS_vec, t_vec, T_vec) in enumerate(logs):
+        T_vec[mode].append(np.copy(T0[m].mean()))
+        t_vec[mode].append(np.copy(t0[m]))
+        _snapshot(snapshots[mode], {"T": T0[m].copy(), "v": np.zeros((n, 3)), "P": np.zeros(n)})
+        snapshots[mode]["xcc"], snapshots[mode]["ycc"] = xcc, ycc
+    write_t = np.zeros(B)
+    write_every = np.broadcast_to(np.asarray(write_every, dtype=np.float64), (B,))
+    ens.start_clock(t_end, save_every=save_every, t0=t0, max_steps=max_steps, n_step=n_step, snap_slots=k)
+    t_now = t0.copy()
+    n_now = np.broadcast_to(np.asarray(n_step, dtype=np.int64), (B,)).copy()
+    while ens.any_active():
+        w0 = time.time()
+        ens.run(k, steps_per_graph=k)
+        blk = ens.drain()
+        wall = time.time() - w0
+        for m, d in enumerate(blk):
+            snapshots, TS_vec, t_vec, T_vec = logs[m]
+            taken = len(d["dt"])
+            for tm, mt in zip(d["t"], d["meanT"]):
+                t_vec[mode].append(np.copy(tm))
+                T_vec[mode].append(np.copy(mt))
+                TS_vec[mode].append(wall / taken)
+            for sn in d["snapshots"]:
+                st = {"T": sn["T"].astype(np.float64).reshape(n),
+                      "v": np.concatenate((sn["u"].astype(np.float64).reshape(-1, 1), sn["v"].astype(np.float64).reshape(-1, 1),
+                                           np.zeros((n, 1))), axis=1),
+                      "P": sn["p"].astype(np.float64).reshape(n) if sn["p"] is not None else np.zeros(n)}
+                _snapshot(snapshots[mode], st)
+            if taken:
+                t_now[m], n_now[m] = d["t"][-1], d["steps"][-1]
+            if taken and t_now[m] > write_t[m]:
+                write_t[m] = t_now[m] + write_every[m]
+                write_logs(dirs[m], mode, *logs[m])
+    for m in range(B):
+        write_logs(dirs[m], mode, *logs[m])
+    ens.stop_clock()
+    return t_now, n_now, logs

@@ -228,16 +228,22 @@ class SurrogateEngine:
                                                 L.stream_ptr(dev)), "pbmc_surrogate_forward")
         return u, v, p, uvmax
 
-    def rollout(self, state, first_step, n_steps):
-        """Enqueue n_steps time steps on `state` (a RolloutState).  No host sync."""
+    def rollout(self, state, first_step, n_steps, clock=None):
+        """Enqueue n_steps time steps on `state` (a RolloutState).  No host sync.  clock: a rollout.MemberClocks (the
+        per-member run-to-time clock, pbmc_rollout_clocked) or None (pbmc_rollout)."""
         self.refresh()
         s = state
         ws = self.workspace(s.B, s.H, s.W)
-        L.check(L.load().pbmc_rollout(self._ctx, C.byref(self.desc), L.ptr(s.members), L.ptr(s.xc), L.ptr(s.yc), L.ptr(s.ycc),
-                                      L.ptr(s.xcoef), L.ptr(s.ycoef), float(s.dx_min), float(s.cn_max), int(s.per_member_dt),
-                                      L.ptr(s.T_seq), s.nslots, int(first_step), int(n_steps), L.ptr(s.dt_seq), int(s.dt_seq.shape[0]), L.ptr(s.u),
-                                      L.ptr(s.v), L.ptr(s.p), L.ptr(s.V), L.ptr(ws), ws.numel(), s.B, s.H, s.W,
-                                      L.stream_ptr(self.device)), "pbmc_rollout")
+        args = (self._ctx, C.byref(self.desc), L.ptr(s.members), L.ptr(s.xc), L.ptr(s.yc), L.ptr(s.ycc), L.ptr(s.xcoef),
+                L.ptr(s.ycoef), float(s.dx_min), float(s.cn_max), int(s.per_member_dt), L.ptr(s.T_seq), s.nslots,
+                int(first_step), int(n_steps), L.ptr(s.dt_seq), int(s.dt_seq.shape[0]), L.ptr(s.u), L.ptr(s.v), L.ptr(s.p),
+                L.ptr(s.V), L.ptr(ws), ws.numel(), s.B, s.H, s.W)
+        if clock is None:
+            L.check(L.load().pbmc_rollout(*args, L.stream_ptr(self.device)), "pbmc_rollout")
+        else:
+            L.check(L.load().pbmc_rollout_clocked(*args, L.ptr(clock.clock), L.ptr(clock.meanT_seq), L.ptr(clock.ring),
+                                                  L.ptr(clock.meta), int(clock.slots), L.stream_ptr(self.device)),
+                    "pbmc_rollout_clocked")
 
 
 class Grid:

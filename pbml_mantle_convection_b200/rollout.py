@@ -5,12 +5,20 @@ This is the GAIA-free form of the reference's hot loop (advect_wi_gaia.py:583-66
 never leave the device; a whole block of time steps is one CUDA graph.  Each member keeps its
 own CFL time step (the reference runs one member per process; ADNet's batch-global amax,
 :556, is not inherited here -- use `per_member_dt=False` for that behaviour).
+
+Run to a simulated end time (`start_clock` / `drain`): each member carries a clock in device memory that the device
+advances after every step (pbmc_rollout_clocked): a member runs `while t < t_end` like the reference driver
+(advect_wi_gaia.py:583), logs mean-T after every step and takes its snapshots at the exact steps where `t > save_t`;
+once stopped it is frozen (T bit-identical, dt rows 0) while the others go on.  The host reads the logs once per block.
 """
 from __future__ import annotations
+
+import ctypes as C
 
 import numpy as np
 import torch
 
+from . import _lib as L
 from . import ops
 from .engine import Grid, RolloutState
 
@@ -36,6 +44,31 @@ def synthetic_T0(H, W, seed=1):
     return T
 
 
+_W = lambda name: getattr(L.MemberClock, name).offset // 8  # 8-byte word of a pbmc_member_clock field
+_T, _T_END, _SAVE_T, _SAVE_EVERY = _W("t"), _W("t_end"), _W("save_t"), _W("save_every")
+_STEPS, _MAX_STEPS, _SNAPS, _DRAINED = _W("steps"), _W("max_steps"), _W("snaps"), _W("drained")
+_ACTIVE, _OVERFLOW = 2 * _W("active"), 2 * _W("active") + 1  # int32 words
+_HDR = _W("part")  # the counters; the partial sums after them are device scratch
+_NO_LIMIT = 1 << 62
+
+
+class MemberClocks:
+    """Device buffers of a clocked rollout: one pbmc_member_clock per member (as a [B, words] float64 tensor, viewed as
+    int64 / int32 for the integer fields), meanT_seq (indexed like dt_seq) and the snapshot ring with its metadata."""
+
+    def __init__(self, B, H, W, rows, p_pred, slots, device):
+        words = C.sizeof(L.MemberClock) // 8
+        self.clock = torch.zeros(B, words, dtype=torch.float64, device=device)
+        self.meanT_seq = torch.zeros(rows, B, dtype=torch.float64, device=device)
+        self.nch = 4 if p_pred else 3
+        self.slots = int(slots)
+        self.ring = torch.zeros(self.slots, B, self.nch, H, W, dtype=torch.float32, device=device)
+        self.meta = torch.zeros(self.slots, B, 2, dtype=torch.float64, device=device)
+
+    def key(self):
+        return ("clock", self.clock.data_ptr(), self.meanT_seq.data_ptr(), self.ring.data_ptr(), self.meta.data_ptr(), self.slots)
+
+
 class EnsembleRollout:
     """B members on one GPU.  `params`: list of (RaQ, gamma=fkt, beta=fkp), one per member."""
 
@@ -57,6 +90,8 @@ class EnsembleRollout:
         self.time = torch.zeros(self.B, dtype=torch.float64, device=self.device)
         self._graphs = {}
         self._stream = torch.cuda.Stream(self.device)
+        self._clk = None      # MemberClocks while a clock runs (start_clock)
+        self._pending = None  # (first dt_seq row, steps) of the block not drained yet
 
     # ------------------------------------------------------------------ state
     def set_T(self, T0):
@@ -73,12 +108,15 @@ class EnsembleRollout:
         """Enqueue n time steps directly (no graph)."""
         done = 0
         self.engine = self.net._engine(self.device)  # picks up a changed net.conv_impl
+        if self._clk is not None and n > self.max_steps:
+            raise ValueError("a clocked rollout advances at most max_steps steps between two drain() calls")
         while done < n:
             # dt history is written relative to first_step (rows first-1 .. first-1+k-1 of max_steps + 1); restart the
             # index every call
             first = 1 + (self.n_done % 2)
             k = min(n - done, self.max_steps)
-            self.engine.rollout(self.state, first, k)
+            self._begin_block(first - 1, k)
+            self.engine.rollout(self.state, first, k, clock=self._clk)
             self.time += self.state.dt_seq[first - 1:first - 1 + k].sum(0)
             self.n_done += k
             done += k
@@ -93,14 +131,20 @@ class EnsembleRollout:
         par = self.n_done % 2
         # the graph bakes in packed-weight and workspace addresses and the conv implementation: key on them too
         key = (k, par) + self.engine.graph_key(self.B, self.H, self.W)
+        clk = self._clk
+        if clk is not None:
+            key = key + clk.key()  # a clocked graph: its own entry (t_end, save_every live in device memory)
         if key not in self._graphs:
             saved = self.state.T_seq.clone()
-            self.engine.rollout(self.state, 1 + par, 1)  # eager warm-up: module load + func attributes outside capture
+            saved_clock = clk.clock.clone() if clk is not None else None
+            self.engine.rollout(self.state, 1 + par, 1, clock=clk)  # eager warm-up: module load + func attributes outside capture
             self.state.T_seq.copy_(saved)
+            if clk is not None:
+                clk.clock.copy_(saved_clock)
             torch.cuda.synchronize(self.device)
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
-                self.engine.rollout(self.state, 1 + par, k)
+                self.engine.rollout(self.state, 1 + par, k, clock=clk)
             self._graphs[key] = g
         return self._graphs[key]
 
@@ -112,16 +156,22 @@ class EnsembleRollout:
         k = int(steps_per_graph)
         if n_steps % k:
             raise ValueError("n_steps must be a multiple of steps_per_graph")
+        if self._clk is not None and n_steps != k:
+            raise ValueError("a clocked rollout runs one block (n_steps == steps_per_graph) between two drain() calls")
         for _ in range(n_steps // k):
             par = self.n_done % 2
-            self.graph(k).replay()
+            g = self.graph(k)
+            self._begin_block(par, k)
+            g.replay()
             if track_time:
                 self.time += self.state.dt_seq[par:par + k].sum(0)
             self.n_done += k
 
     # ------------------------------------------------------------------ outputs
     def fields(self):
-        """(u, v, p, V) of the last step, float32 [B,H,W]."""
+        """(u, v, p, V) of the last step, float32 [B,H,W].  With a clock, a frozen member's entries are the surrogate's
+        output for its frozen T -- the velocities of a step it does not take, not those of its last step; its snapshots
+        hold the right ones."""
         s = self.state
         return s.u, s.v, s.p, s.V
 
@@ -135,3 +185,139 @@ class EnsembleRollout:
         y = self.grid.y1d64.to(self.device)
         dprof = (prof[:, 1:] - prof[:, :-1]) / (y[1:] - y[:-1])[None]
         return mean, prof, dprof
+
+    # ------------------------------------------------------------------ run to a simulated end time
+    def _per_member(self, x, dtype=np.float64):
+        return np.broadcast_to(np.asarray(x, dtype=dtype), (self.B,)).copy()
+
+    def start_clock(self, t_end, save_every=0.0, t0=None, max_steps=None, n_step=0, snap_slots=None, steps_per_graph=10):
+        """Give every member a clock (each argument a scalar or one value per member): the following steps run member m
+        `while t[m] < t_end[m] and steps[m] < max_steps[m]` (advect_wi_gaia.py:583), log mean-T after every step and take a
+        snapshot (T, u, v, p) whenever t > save_t (save_t = 0 at the start, then t + save_every).
+          t0         start time (default: `self.time`; given, it also becomes `self.time`)
+          n_step     step count at the start (the reference's n_step), max_steps an absolute limit on it (None: none)
+          snap_slots snapshot-ring slots per member (default steps_per_graph: a ring drained once per block never fills)
+        Then alternate `run(k, steps_per_graph=k)` (or `step(n)`) and `drain()` until `any_active()` is False."""
+        slots = int(snap_slots if snap_slots is not None else steps_per_graph)
+        if slots < 1:
+            raise ValueError("snap_slots must be >= 1")
+        if not self.state.per_member_dt and self.B > 1:
+            raise L.PbmcError("a clock needs per_member_dt=True when B > 1: with a batch-global dt a frozen member would "
+                              "still set the others' time step")
+        clk = self._clk
+        if clk is None or clk.slots != slots:
+            self._graphs = {k: g for k, g in self._graphs.items() if "clock" not in k}  # graphs of the old buffers
+            clk = MemberClocks(self.B, self.H, self.W, self.state.dt_seq.shape[0], self.state.p is not None, slots, self.device)
+        if t0 is None:
+            t0 = self.time.cpu().numpy()
+        t0 = self._per_member(t0)
+        steps0 = self._per_member(n_step, np.int64)
+        t_end, save_every = self._per_member(t_end), self._per_member(save_every)
+        max_steps = self._per_member(_NO_LIMIT if max_steps is None else max_steps, np.int64)
+        c = torch.zeros(clk.clock.shape, dtype=torch.float64)
+        c[:, _T], c[:, _T_END], c[:, _SAVE_T], c[:, _SAVE_EVERY] = (torch.from_numpy(a) for a in (t0, t_end, np.zeros(self.B), save_every))
+        ci = c.view(torch.int64)
+        ci[:, _STEPS], ci[:, _MAX_STEPS] = torch.from_numpy(steps0), torch.from_numpy(max_steps)
+        active = (t0 < t_end) & (steps0 < max_steps)
+        c.view(torch.int32)[:, _ACTIVE] = torch.from_numpy(active.astype(np.int32))
+        clk.clock.copy_(c)
+        self.time.copy_(torch.from_numpy(t0))
+        self._clk = clk
+        self._pending = None
+        self._host_t, self._host_steps, self._host_active = t0, steps0, active
+        self._t_end, self._max_steps = t_end, max_steps
+
+    def stop_clock(self):
+        """Back to unclocked stepping (the clocked graphs stay cached)."""
+        self._clk = None
+        self._pending = None
+
+    def set_t_end(self, t_end):
+        """New end time(s) between blocks: written to the device clock, no re-capture.  A stopped member whose t is now
+        below its t_end takes steps again."""
+        self._require_clock()
+        self._t_end = self._per_member(t_end)
+        self._host_active = (self._host_t < self._t_end) & (self._host_steps < self._max_steps)
+        self._clk.clock[:, _T_END].copy_(torch.from_numpy(self._t_end))
+        self._clk.clock.view(torch.int32)[:, _ACTIVE].copy_(torch.from_numpy(self._host_active.astype(np.int32)))
+
+    def set_save_every(self, save_every):
+        """New snapshot interval(s) between blocks (applies from the next snapshot on)."""
+        self._require_clock()
+        self._clk.clock[:, _SAVE_EVERY].copy_(torch.from_numpy(self._per_member(save_every)))
+
+    def any_active(self):
+        """Whether a member still takes steps, from the counters the last drain() read (no device access)."""
+        self._require_clock()
+        return bool(self._host_active.any())
+
+    def read_clock(self):
+        """The device clocks as numpy arrays: t, t_end, save_t, steps, snaps, drained, active, overflow (synchronises)."""
+        self._require_clock()
+        c = self._clk.clock[:, :_HDR].cpu()
+        ci, ci32 = c.view(torch.int64), c.view(torch.int32)
+        return {"t": c[:, _T].numpy(), "t_end": c[:, _T_END].numpy(), "save_t": c[:, _SAVE_T].numpy(),
+                "steps": ci[:, _STEPS].numpy(), "snaps": ci[:, _SNAPS].numpy(), "drained": ci[:, _DRAINED].numpy(),
+                "active": ci32[:, _ACTIVE].numpy() != 0, "overflow": ci32[:, _OVERFLOW].numpy() != 0}
+
+    def drain(self):
+        """Logs of the block run since the last drain, one dict per member:
+          dt, t, meanT  float64 [n] over the n steps the member took (t after each step, mean of T after each step)
+          steps         int64 [n], the step numbers
+          snapshots     list of dicts (step, t, T, u, v, p) in the order taken; fields float32 numpy [H,W] (p None without p_pred)
+        Copies only the counters, the block's rows and the filled ring slots to the host.  Raises if a member's snapshot
+        ring overflowed (a snapshot was due while every slot held an undrained one: drain more often or use more slots)."""
+        self._require_clock()
+        clk = self._clk
+        ck = self.read_clock()
+        if ck["overflow"].any():
+            bad = np.flatnonzero(ck["overflow"]).tolist()
+            raise L.PbmcError(f"snapshot ring overflow for members {bad}: a snapshot was due while all {clk.slots} slots held "
+                              "undrained snapshots (it was skipped); drain() after every block or pass a larger snap_slots")
+        n = ck["steps"] - self._host_steps
+        nmax = int(n.max()) if self.B else 0
+        if nmax > 0:
+            if self._pending is None or nmax > self._pending[1]:
+                raise L.PbmcError("clock counters do not match the block that was run")
+            lo = self._pending[0]
+            dts = self.state.dt_seq[lo:lo + nmax].cpu().numpy()
+            mts = clk.meanT_seq[lo:lo + nmax].cpu().numpy()
+        slot_idx, mem_idx = [], []
+        for m in range(self.B):
+            for j in range(int(ck["drained"][m]), int(ck["snaps"][m])):
+                slot_idx.append(j % clk.slots)
+                mem_idx.append(m)
+        if slot_idx:
+            si, mi = torch.tensor(slot_idx, device=self.device), torch.tensor(mem_idx, device=self.device)
+            ring = clk.ring[si, mi].cpu().numpy()
+            meta = clk.meta[si, mi].cpu().numpy()
+        out, r = [], 0
+        for m in range(self.B):
+            k = int(n[m])
+            d = {"dt": dts[:k, m].copy() if k else np.zeros(0), "meanT": mts[:k, m].copy() if k else np.zeros(0),
+                 "steps": np.arange(self._host_steps[m] + 1, ck["steps"][m] + 1, dtype=np.int64)}
+            # the device's own sequence of double additions t += dt, so d["t"][-1] == the clock's t bit for bit
+            d["t"] = np.cumsum(np.concatenate(([self._host_t[m]], d["dt"])))[1:]
+            snaps = []
+            for _ in range(int(ck["snaps"][m] - ck["drained"][m])):
+                f = ring[r]
+                snaps.append({"step": int(meta[r, 0]), "t": float(meta[r, 1]), "T": f[0], "u": f[1], "v": f[2],
+                              "p": f[3] if clk.nch == 4 else None})
+                r += 1
+            d["snapshots"] = snaps
+            out.append(d)
+        clk.clock.view(torch.int64)[:, _DRAINED].copy_(torch.from_numpy(ck["snaps"].copy()))
+        self._host_t, self._host_steps, self._host_active = ck["t"].copy(), ck["steps"].copy(), ck["active"].copy()
+        self._pending = None
+        return out
+
+    def _require_clock(self):
+        if self._clk is None:
+            raise RuntimeError("no clock: call start_clock() first")
+
+    def _begin_block(self, first_row, k):
+        if self._clk is None:
+            return
+        if self._pending is not None:
+            raise RuntimeError("drain() the previous block first: its per-step rows would be overwritten")
+        self._pending = (first_row, k)
