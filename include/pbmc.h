@@ -381,7 +381,8 @@ int pbmc_rollout(pbmc_ctx* ctx, const pbmc_net* net_h, const pbmc_member* member
  * every step t += dt, mean-T logged, and a snapshot whenever t > save_t (then save_t = t + save_every; save_t = 0 at the
  * start).  One clock per member, in device memory, read and updated by the device after every step, so a captured k-step
  * graph keeps working across replays.  A member that has stopped ("frozen") still goes through the surrogate (the batch
- * shape is fixed) but its T stays bit-identical, its dt_seq rows are written as 0 and nothing is logged for it.
+ * shape is fixed) but its T stays bit-identical, its dt_seq rows are written as 0 and nothing is logged for it
+ * (pbmc_rollout_queued puts the next queued member into the slot instead, while its queue has entries).
  *   active    1 while the member takes steps: t < t_end && steps < max_steps (recomputed after every step)
  *   snaps     snapshots taken so far; snapshot j lives in ring slot j % snap_slots
  *   drained   snapshots the caller has read (the caller advances it); a due snapshot is skipped, and overflow set, when
@@ -408,6 +409,48 @@ int pbmc_rollout_clocked(pbmc_ctx* ctx, const pbmc_net* net_h, const pbmc_member
                          float* p, float* V, void* workspace, size_t workspace_bytes, int B, int H, int W,
                          pbmc_member_clock* clock, double* meanT_seq, float* snap_ring, double* snap_meta, int snap_slots,
                          void* stream);
+
+/* ------------------------------------------------------------------ sweeps larger than the batch
+ * A queue of Q members run through the B slots of a clocked rollout: when a slot's member stops after step i (its clock
+ * goes from active to inactive) and the queue is not empty, the device puts the next queued member into that slot before
+ * step i + 1, inside the same captured graph.  Refill rule, fixed so that it can be tested: of the slots that stop after
+ * step i, the one with rank r (r = how many slots with a LOWER index also stop after step i) takes entry q = next + r if
+ * q < Q; then next += the number of slots refilled.  A refilled slot gets
+ *   T (the step's output slot) = T0[q] bit for bit, members[s] = params[q] bit for bit,
+ *   clock: t = t0[q], t_end[q], save_t = 0, save_every[q], steps = n_step0[q], max_steps[q], active = 1
+ * (snaps / drained / overflow belong to the slot's ring and carry on).  The finishing member's mean-T and its last
+ * snapshot are taken before the refill; the new member's first step is step i + 1.  A stopping slot with the queue
+ * empty freezes as in pbmc_rollout_clocked.  The caller places the first min(B, Q) entries into slots 0 .. in order
+ * (next = min(B, Q)); with Q < B the other slots start inactive.  Every queued member must be able to take a step
+ * (t0 < t_end, n_step0 < max_steps).  All members are device arrays; next is one int64 in device memory.
+ *   slot_member  [B]: queue entry in each slot (-1: none), rewritten on a refill
+ *   member_seq   [dt_seq_rows][B], indexed like dt_seq: the entry whose step row i - 1 logs, -1 if the slot took none
+ *   snap_member  [snap_slots][B]: the entry each ring slot's snapshot belongs to */
+typedef struct {
+  const float* T0;             /* [Q][H][W], 16-byte aligned */
+  const pbmc_member* params;   /* [Q] */
+  const double* t0;            /* [Q] */
+  const double* t_end;         /* [Q] */
+  const double* save_every;    /* [Q] */
+  const int64_t* n_step0;      /* [Q] */
+  const int64_t* max_steps;    /* [Q] */
+  int64_t* next;
+  int64_t* slot_member;
+  int64_t* member_seq;
+  int64_t* snap_member;
+  int64_t Q;
+} pbmc_member_queue;
+
+/* pbmc_rollout_clocked plus a member queue (host struct of device pointers): same launches, no extra one; the apply and
+ * commit kernels behind each step also make the refills.  members is rewritten by the device.  Refused before any CUDA
+ * call: what pbmc_rollout_clocked refuses, a NULL queue or NULL array in it (PBMC_ERR_NULL_POINTER), Q < 1
+ * (PBMC_ERR_BAD_SHAPE), a T0 that is not 16-byte aligned (PBMC_ERR_MISALIGNED). */
+int pbmc_rollout_queued(pbmc_ctx* ctx, const pbmc_net* net_h, pbmc_member* members, const float* xc, const float* yc,
+                        const float* ycc, const float* xcoef, const float* ycoef, double dx_min, double cn_max, int per_member_dt,
+                        float* T_seq, int nslots, int first_step, int n_steps, double* dt_seq, int dt_seq_rows, float* u, float* v,
+                        float* p, float* V, void* workspace, size_t workspace_bytes, int B, int H, int W,
+                        pbmc_member_clock* clock, double* meanT_seq, float* snap_ring, double* snap_meta, int snap_slots,
+                        const pbmc_member_queue* queue_h, void* stream);
 
 #ifdef __cplusplus
 }

@@ -88,7 +88,13 @@ class MemberClock(C.Structure):
                 ("active", C.c_int), ("overflow", C.c_int), ("part", C.c_double * CLOCK_PARTS)]
 
 
-_STRUCTS = {"pbmc_member_clock": MemberClock, "pbmc_edge9_desc": Edge9Desc, "pbmc_trunk_desc": TrunkDesc, "pbmc_slab_sync": SlabSync, "pbmc_member": Member, "pbmc_src": Src, "pbmc_conv_desc": ConvDesc, "pbmc_layer": Layer, "pbmc_net": Net}
+class MemberQueue(C.Structure):
+    _fields_ = [("T0", C.c_void_p), ("params", C.c_void_p), ("t0", C.c_void_p), ("t_end", C.c_void_p), ("save_every", C.c_void_p),
+                ("n_step0", C.c_void_p), ("max_steps", C.c_void_p), ("next", C.c_void_p), ("slot_member", C.c_void_p),
+                ("member_seq", C.c_void_p), ("snap_member", C.c_void_p), ("Q", C.c_int64)]
+
+
+_STRUCTS = {"pbmc_member_queue": MemberQueue, "pbmc_member_clock": MemberClock, "pbmc_edge9_desc": Edge9Desc, "pbmc_trunk_desc": TrunkDesc, "pbmc_slab_sync": SlabSync, "pbmc_member": Member, "pbmc_src": Src, "pbmc_conv_desc": ConvDesc, "pbmc_layer": Layer, "pbmc_net": Net}
 
 # name -> (restype, argtypes); every symbol declared in include/pbmc.h
 _vp, _i, _d, _f, _sz = C.c_void_p, C.c_int, C.c_double, C.c_float, C.c_size_t
@@ -131,6 +137,8 @@ SIGNATURES = {
                           _vp, _vp, _vp, _sz, _i, _i, _i, _vp]),
     "pbmc_rollout_clocked": (_i, [_vp, C.POINTER(Net), _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _vp, _i, _i, _i, _vp, _i, _vp,
                                   _vp, _vp, _vp, _vp, _sz, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _vp]),
+    "pbmc_rollout_queued": (_i, [_vp, C.POINTER(Net), _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _vp, _i, _i, _i, _vp, _i, _vp,
+                                 _vp, _vp, _vp, _vp, _sz, _i, _i, _i, _vp, _vp, _vp, _vp, _i, C.POINTER(MemberQueue), _vp]),
 }
 
 _lib = None

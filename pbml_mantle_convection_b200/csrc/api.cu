@@ -35,7 +35,7 @@ extern thread_local int g_stencil_pdl_next;  // stencil.cu: the next plain stenc
 extern thread_local int g_edge9_pdl_next;    // conv_edge9.cu: the next ring launch uses programmatic dependent launch
 int clock_enqueue(pbmc_member_clock* clk, const float* Tin, float* Tout, const float* u, const float* v, const float* p,
                   double* dt_row, double* meanT_row, float* ring, double* meta, int slots, int B, int H, int W,
-                  cudaStream_t st);  // clock.cu
+                  const pbmc_member_queue* queue, pbmc_member* members, int64_t* seq_row, cudaStream_t st);  // clock.cu
 
 }  // namespace pbmc
 
@@ -75,6 +75,7 @@ extern "C" size_t pbmc_sizeof(const char* name) {
   if (!strcmp(name, "pbmc_trunk_desc")) return sizeof(pbmc_trunk_desc);
   if (!strcmp(name, "pbmc_edge9_desc")) return sizeof(pbmc_edge9_desc);
   if (!strcmp(name, "pbmc_member_clock")) return sizeof(pbmc_member_clock);
+  if (!strcmp(name, "pbmc_member_queue")) return sizeof(pbmc_member_queue);
   return 0;
 }
 
@@ -660,13 +661,13 @@ struct ClockArgs {
 };
 }  // namespace
 
-// pbmc_rollout and pbmc_rollout_clocked: the same launches in the same order; a clock adds its two launches behind every
-// step's stencil
+// pbmc_rollout, pbmc_rollout_clocked and pbmc_rollout_queued: the same launches in the same order; a clock adds its two
+// launches behind every step's stencil, a queue (NULL except for pbmc_rollout_queued, whose members are mutable) none
 static int rollout_impl(pbmc_ctx* ctx, const pbmc_net* net, const pbmc_member* members, const float* xc, const float* yc,
                         const float* ycc, const float* xcoef, const float* ycoef, double dx_min, double cn_max,
                         int per_member_dt, float* T_seq, int nslots, int first_step, int n_steps, double* dt_seq,
                         int dt_seq_rows, float* u, float* v, float* p, float* V, void* workspace, size_t workspace_bytes,
-                        int B, int H, int W, const ClockArgs& clk, void* stream) {
+                        int B, int H, int W, const ClockArgs& clk, const pbmc_member_queue* queue, void* stream) {
   if (!ctx || !net || !members || !xc || !yc || !ycc || !xcoef || !ycoef || !T_seq || !u || !v || !workspace) return PBMC_ERR_NULL_POINTER;
   if (nslots < 2 || first_step < 1 || n_steps < 0 || !(dx_min > 0.0)) return PBMC_ERR_BAD_SHAPE;
   if (dt_seq != nullptr && dt_seq_rows < first_step + n_steps - 1) return PBMC_ERR_BAD_SHAPE;  // step i writes row i - 1
@@ -710,7 +711,8 @@ static int rollout_impl(pbmc_ctx* ctx, const pbmc_net* net, const pbmc_member* m
       // plain stream order behind the stencil; the next step's input build is PDL-launched behind the commit kernel
       if (clk.clock)
         RC(clock_enqueue(clk.clock, Tin, Tout, u, v, p, dt_seq + (size_t)(i - 1) * B, clk.meanT_seq + (size_t)(i - 1) * B,
-                         clk.snap_ring, clk.snap_meta, clk.snap_slots, B, H, W, st));
+                         clk.snap_ring, clk.snap_meta, clk.snap_slots, B, H, W, queue, const_cast<pbmc_member*>(members),
+                         queue ? queue->member_seq + (size_t)(i - 1) * B : nullptr, st));
     }
     return PBMC_OK;
   };
@@ -729,7 +731,16 @@ extern "C" int pbmc_rollout(pbmc_ctx* ctx, const pbmc_net* net, const pbmc_membe
                             int W, void* stream) {
   const ClockArgs none = {nullptr, nullptr, nullptr, nullptr, 0};
   return rollout_impl(ctx, net, members, xc, yc, ycc, xcoef, ycoef, dx_min, cn_max, per_member_dt, T_seq, nslots, first_step,
-                      n_steps, dt_seq, dt_seq_rows, u, v, p, V, workspace, workspace_bytes, B, H, W, none, stream);
+                      n_steps, dt_seq, dt_seq_rows, u, v, p, V, workspace, workspace_bytes, B, H, W, none, nullptr, stream);
+}
+
+// the refusals of a clocked rollout, shared by pbmc_rollout_clocked and pbmc_rollout_queued
+static int validate_clock(const pbmc_member_clock* clock, const double* dt_seq, const double* meanT_seq, const float* snap_ring,
+                          const double* snap_meta, int snap_slots, int per_member_dt, int B) {
+  if (!clock || !dt_seq || !meanT_seq || !snap_ring || !snap_meta) return PBMC_ERR_NULL_POINTER;
+  if (snap_slots < 1) return PBMC_ERR_BAD_SHAPE;
+  if (!per_member_dt && B > 1) return PBMC_ERR_UNSUPPORTED;  // a frozen member would still set the others' batch-global dt
+  return PBMC_OK;
 }
 
 extern "C" int pbmc_rollout_clocked(pbmc_ctx* ctx, const pbmc_net* net, const pbmc_member* members, const float* xc,
@@ -738,10 +749,29 @@ extern "C" int pbmc_rollout_clocked(pbmc_ctx* ctx, const pbmc_net* net, const pb
                                     double* dt_seq, int dt_seq_rows, float* u, float* v, float* p, float* V, void* workspace,
                                     size_t workspace_bytes, int B, int H, int W, pbmc_member_clock* clock, double* meanT_seq,
                                     float* snap_ring, double* snap_meta, int snap_slots, void* stream) {
-  if (!clock || !dt_seq || !meanT_seq || !snap_ring || !snap_meta) return PBMC_ERR_NULL_POINTER;
-  if (snap_slots < 1) return PBMC_ERR_BAD_SHAPE;
-  if (!per_member_dt && B > 1) return PBMC_ERR_UNSUPPORTED;  // a frozen member would still set the others' batch-global dt
+  RC(validate_clock(clock, dt_seq, meanT_seq, snap_ring, snap_meta, snap_slots, per_member_dt, B));
   const ClockArgs clk = {clock, meanT_seq, snap_ring, snap_meta, snap_slots};
   return rollout_impl(ctx, net, members, xc, yc, ycc, xcoef, ycoef, dx_min, cn_max, per_member_dt, T_seq, nslots, first_step,
-                      n_steps, dt_seq, dt_seq_rows, u, v, p, V, workspace, workspace_bytes, B, H, W, clk, stream);
+                      n_steps, dt_seq, dt_seq_rows, u, v, p, V, workspace, workspace_bytes, B, H, W, clk, nullptr, stream);
+}
+
+extern "C" int pbmc_rollout_queued(pbmc_ctx* ctx, const pbmc_net* net, pbmc_member* members, const float* xc, const float* yc,
+                                   const float* ycc, const float* xcoef, const float* ycoef, double dx_min, double cn_max,
+                                   int per_member_dt, float* T_seq, int nslots, int first_step, int n_steps, double* dt_seq,
+                                   int dt_seq_rows, float* u, float* v, float* p, float* V, void* workspace,
+                                   size_t workspace_bytes, int B, int H, int W, pbmc_member_clock* clock, double* meanT_seq,
+                                   float* snap_ring, double* snap_meta, int snap_slots, const pbmc_member_queue* queue,
+                                   void* stream) {
+  RC(validate_clock(clock, dt_seq, meanT_seq, snap_ring, snap_meta, snap_slots, per_member_dt, B));
+  if (!queue) return PBMC_ERR_NULL_POINTER;
+  const pbmc_member_queue& q = *queue;
+  if (!q.T0 || !q.params || !q.t0 || !q.t_end || !q.save_every || !q.n_step0 || !q.max_steps || !q.next || !q.slot_member ||
+      !q.member_seq || !q.snap_member)
+    return PBMC_ERR_NULL_POINTER;
+  if (q.Q < 1) return PBMC_ERR_BAD_SHAPE;
+  if (!aligned16(q.T0)) return PBMC_ERR_MISALIGNED;  // the refill copies T0 rows with 16-byte loads
+  if ((size_t)B * sizeof(int) > 48 * 1024) return PBMC_ERR_UNSUPPORTED;  // the commit kernel's [B] stop flags in shared memory
+  const ClockArgs clk = {clock, meanT_seq, snap_ring, snap_meta, snap_slots};
+  return rollout_impl(ctx, net, members, xc, yc, ycc, xcoef, ycoef, dx_min, cn_max, per_member_dt, T_seq, nslots, first_step,
+                      n_steps, dt_seq, dt_seq_rows, u, v, p, V, workspace, workspace_bytes, B, H, W, clk, &q, stream);
 }

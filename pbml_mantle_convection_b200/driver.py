@@ -22,6 +22,9 @@ Three ways to advance:
   * `attempt_ensemble(ens, ...)` -- every member of an `EnsembleRollout` runs to its own `t_end` on a device-side clock
     (`EnsembleRollout.start_clock`): per-step t / mean-T and snapshots at the exact steps, the four pickles per member,
     read back once per block of `check_every` steps.
+  * `attempt_sweep(ens, T0, params, ...)` -- the same for a sweep of Q members run through the B slots of an
+    `EnsembleRollout` (`EnsembleRollout.start_sweep`): a slot whose member stops takes the next queued member on the
+    device, so Q may exceed B and no slot idles while members wait.
 
 External energy solver (the `ML_STOKES` / `ML_PRE` modes and the `intervene_TS` interventions of mode "ML", `:486-505`,
 `:618-630`): the reference calls GAIA's `sim.doTimestep()` with the surrogate's velocities already written into the state
@@ -188,22 +191,56 @@ def attempt_ensemble(ens, xcc, ycc, t_end, out_dir, save_every=0.0, write_every=
     dirs = [os.path.join(out_dir, f"member_{m}") for m in range(B)]
     T0 = ens.T.double().cpu().numpy().reshape(B, n)
     t0 = np.broadcast_to(np.asarray(t, dtype=np.float64), (B,)).copy()
+    _initial_entries(logs, T0, t0, xcc, ycc, mode, n)
+    ens.start_clock(t_end, save_every=save_every, t0=t0, max_steps=max_steps, n_step=n_step, snap_slots=k)
+    return _run_blocks(ens, k, logs, dirs, t0, n_step, write_every, mode, n)
+
+
+def attempt_sweep(ens, T0, params, xcc, ycc, t_end, out_dir, save_every=0.0, write_every=0.0, mode="ML", t=0.0, n_step=0,
+                  check_every=10, max_steps=None):
+    """`attempt` for each of Q members run through the B slots of a device-resident `EnsembleRollout`
+    (`EnsembleRollout.start_sweep`; Q may be larger or smaller than B).  T0: [Q, H, W]; params: Q tuples (RaQ, gamma,
+    beta); t_end, save_every, t, n_step, max_steps: scalars or one value per member.  Member q's pickles go to
+    `out_dir/member_<q>/`, with `attempt_ensemble`'s cadence and content: the slot a member ran in, and when, make no
+    difference.  Returns (t [Q], n_step [Q], [logs of member q])."""
+    Q, H, W = len(params), ens.H, ens.W
+    n = H * W
+    k = int(check_every)
+    logs = [_new_logs(mode) for _ in range(Q)]
+    dirs = [os.path.join(out_dir, f"member_{q}") for q in range(Q)]
+    T0 = torch.as_tensor(T0).to("cpu", torch.float32).reshape(Q, H, W)  # what the device runs from
+    _initial_entries(logs, T0.double().numpy().reshape(Q, n), t, xcc, ycc, mode, n)
+    ens.start_sweep(T0, params, t_end, save_every=save_every, t0=t, max_steps=max_steps, n_step=n_step, snap_slots=k,
+                    steps_per_graph=k)
+    return _run_blocks(ens, k, logs, dirs, t, n_step, write_every, mode, n)
+
+
+def _initial_entries(logs, T0, t, xcc, ycc, mode, n):
+    """`attempt`'s entries before the first step, for every member: mean of T0, the start time, the T0 snapshot."""
+    t0 = np.broadcast_to(np.asarray(t, dtype=np.float64), (len(logs),))
     for m, (snapshots, TS_vec, t_vec, T_vec) in enumerate(logs):
         T_vec[mode].append(np.copy(T0[m].mean()))
         t_vec[mode].append(np.copy(t0[m]))
         _snapshot(snapshots[mode], {"T": T0[m].copy(), "v": np.zeros((n, 3)), "P": np.zeros(n)})
         snapshots[mode]["xcc"], snapshots[mode]["ycc"] = xcc, ycc
-    write_t = np.zeros(B)
-    write_every = np.broadcast_to(np.asarray(write_every, dtype=np.float64), (B,))
-    ens.start_clock(t_end, save_every=save_every, t0=t0, max_steps=max_steps, n_step=n_step, snap_slots=k)
-    t_now = t0.copy()
-    n_now = np.broadcast_to(np.asarray(n_step, dtype=np.int64), (B,)).copy()
+
+
+def _run_blocks(ens, k, logs, dirs, t, n_step, write_every, mode, n):
+    """Blocks of k steps (one graph replay each) until no member of the running clock or sweep is left; each drained
+    block (a list over the members, or a sweep's dict keyed by member) goes into the logs of its members.  A
+    TS_vec entry is the block's wall time over the steps the member took in it; `t > write_t` is evaluated at block
+    ends.  Writes every member's pickles at the end; returns (t, n_step, logs) per member."""
+    N = len(logs)
+    t_now = np.broadcast_to(np.asarray(t, dtype=np.float64), (N,)).copy()
+    n_now = np.broadcast_to(np.asarray(n_step, dtype=np.int64), (N,)).copy()
+    write_t = np.zeros(N)
+    write_every = np.broadcast_to(np.asarray(write_every, dtype=np.float64), (N,))
     while ens.any_active():
         w0 = time.time()
         ens.run(k, steps_per_graph=k)
         blk = ens.drain()
         wall = time.time() - w0
-        for m, d in enumerate(blk):
+        for m, d in (blk.items() if isinstance(blk, dict) else enumerate(blk)):
             snapshots, TS_vec, t_vec, T_vec = logs[m]
             taken = len(d["dt"])
             for tm, mt in zip(d["t"], d["meanT"]):
@@ -221,7 +258,7 @@ def attempt_ensemble(ens, xcc, ycc, t_end, out_dir, save_every=0.0, write_every=
             if taken and t_now[m] > write_t[m]:
                 write_t[m] = t_now[m] + write_every[m]
                 write_logs(dirs[m], mode, *logs[m])
-    for m in range(B):
+    for m in range(N):
         write_logs(dirs[m], mode, *logs[m])
     ens.stop_clock()
     return t_now, n_now, logs

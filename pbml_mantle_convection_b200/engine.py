@@ -228,9 +228,10 @@ class SurrogateEngine:
                                                 L.stream_ptr(dev)), "pbmc_surrogate_forward")
         return u, v, p, uvmax
 
-    def rollout(self, state, first_step, n_steps, clock=None):
+    def rollout(self, state, first_step, n_steps, clock=None, queue=None):
         """Enqueue n_steps time steps on `state` (a RolloutState).  No host sync.  clock: a rollout.MemberClocks (the
-        per-member run-to-time clock, pbmc_rollout_clocked) or None (pbmc_rollout)."""
+        per-member run-to-time clock, pbmc_rollout_clocked) or None (pbmc_rollout); queue (with a clock only): a
+        rollout.SweepQueue whose members refill the slots that stop (pbmc_rollout_queued)."""
         self.refresh()
         s = state
         ws = self.workspace(s.B, s.H, s.W)
@@ -240,6 +241,10 @@ class SurrogateEngine:
                 L.ptr(s.V), L.ptr(ws), ws.numel(), s.B, s.H, s.W)
         if clock is None:
             L.check(L.load().pbmc_rollout(*args, L.stream_ptr(self.device)), "pbmc_rollout")
+        elif queue is not None:
+            L.check(L.load().pbmc_rollout_queued(*args, L.ptr(clock.clock), L.ptr(clock.meanT_seq), L.ptr(clock.ring),
+                                                 L.ptr(clock.meta), int(clock.slots), C.byref(queue.desc),
+                                                 L.stream_ptr(self.device)), "pbmc_rollout_queued")
         else:
             L.check(L.load().pbmc_rollout_clocked(*args, L.ptr(clock.clock), L.ptr(clock.meanT_seq), L.ptr(clock.ring),
                                                   L.ptr(clock.meta), int(clock.slots), L.stream_ptr(self.device)),

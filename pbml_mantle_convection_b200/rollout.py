@@ -10,6 +10,10 @@ Run to a simulated end time (`start_clock` / `drain`): each member carries a clo
 advances after every step (pbmc_rollout_clocked): a member runs `while t < t_end` like the reference driver
 (advect_wi_gaia.py:583), logs mean-T after every step and takes its snapshots at the exact steps where `t > save_t`;
 once stopped it is frozen (T bit-identical, dt rows 0) while the others go on.  The host reads the logs once per block.
+
+Sweeps larger than the batch (`start_sweep`): Q members run through the B slots; when a slot's member stops, the device
+puts the next queued member into it inside the same graph (pbmc_rollout_queued), so no slot idles while the queue holds
+members.
 """
 from __future__ import annotations
 
@@ -69,6 +73,32 @@ class MemberClocks:
         return ("clock", self.clock.data_ptr(), self.meanT_seq.data_ptr(), self.ring.data_ptr(), self.meta.data_ptr(), self.slots)
 
 
+class SweepQueue:
+    """Device buffers of a sweep's member queue (pbmc_member_queue): the queued members' T0, parameter rows and clock
+    starts, `next`, the slot each member is in and the member_seq / snap_member tags.  `desc` is the C struct."""
+
+    def __init__(self, Q, B, H, W, rows, slots, device):
+        f64 = lambda n: torch.zeros(n, dtype=torch.float64, device=device)
+        i64 = lambda *n: torch.full(n, -1, dtype=torch.int64, device=device)
+        self.Q, self.B, self.slots = int(Q), int(B), int(slots)
+        self.T0 = torch.zeros(Q, H, W, dtype=torch.float32, device=device)
+        self.params = torch.zeros(Q, C.sizeof(L.Member) // 4, dtype=torch.float32, device=device)
+        self.t0, self.t_end, self.save_every = f64(Q), f64(Q), f64(Q)
+        self.n_step0, self.max_steps = i64(Q), i64(Q)
+        self.next, self.slot_member = i64(1), i64(B)
+        self.member_seq, self.snap_member = i64(rows, B), i64(self.slots, B)
+        d = self.desc = L.MemberQueue()
+        for name in ("T0", "params", "t0", "t_end", "save_every", "n_step0", "max_steps", "next", "slot_member", "member_seq",
+                     "snap_member"):
+            setattr(d, name, L.ptr(getattr(self, name)))
+        d.Q = self.Q
+
+    def key(self):
+        d = self.desc
+        return ("queue", d.T0, d.params, d.t0, d.t_end, d.save_every, d.n_step0, d.max_steps, d.next, d.slot_member,
+                d.member_seq, d.snap_member, d.Q)
+
+
 class EnsembleRollout:
     """B members on one GPU.  `params`: list of (RaQ, gamma=fkt, beta=fkp), one per member."""
 
@@ -91,7 +121,10 @@ class EnsembleRollout:
         self._graphs = {}
         self._stream = torch.cuda.Stream(self.device)
         self._clk = None      # MemberClocks while a clock runs (start_clock)
+        self._clocks = None   # the last MemberClocks (its buffers, and so its graphs, serve the next clock of that ring size)
         self._pending = None  # (first dt_seq row, steps) of the block not drained yet
+        self._queue = None    # SweepQueue of the last sweep (its buffers, and so its graphs, serve the next one of that shape)
+        self._sweep = None    # host bookkeeping while a sweep runs (start_sweep)
 
     # ------------------------------------------------------------------ state
     def set_T(self, T0):
@@ -116,7 +149,7 @@ class EnsembleRollout:
             first = 1 + (self.n_done % 2)
             k = min(n - done, self.max_steps)
             self._begin_block(first - 1, k)
-            self.engine.rollout(self.state, first, k, clock=self._clk)
+            self.engine.rollout(self.state, first, k, clock=self._clk, queue=self._run_queue())
             self.time += self.state.dt_seq[first - 1:first - 1 + k].sum(0)
             self.n_done += k
             done += k
@@ -131,20 +164,23 @@ class EnsembleRollout:
         par = self.n_done % 2
         # the graph bakes in packed-weight and workspace addresses and the conv implementation: key on them too
         key = (k, par) + self.engine.graph_key(self.B, self.H, self.W)
-        clk = self._clk
+        clk, qu = self._clk, self._run_queue()
         if clk is not None:
             key = key + clk.key()  # a clocked graph: its own entry (t_end, save_every live in device memory)
+        if qu is not None:
+            key = key + qu.key()  # a sweep's graph: refills only rewrite device memory
         if key not in self._graphs:
-            saved = self.state.T_seq.clone()
-            saved_clock = clk.clock.clone() if clk is not None else None
-            self.engine.rollout(self.state, 1 + par, 1, clock=clk)  # eager warm-up: module load + func attributes outside capture
-            self.state.T_seq.copy_(saved)
-            if clk is not None:
-                clk.clock.copy_(saved_clock)
+            # eager warm-up (module load + func attributes outside capture) on saved state: what a step may rewrite
+            saved = [self.state.T_seq] + ([clk.clock] if clk is not None else []) + \
+                    ([self.members, qu.next, qu.slot_member] if qu is not None else [])
+            copies = [t.clone() for t in saved]
+            self.engine.rollout(self.state, 1 + par, 1, clock=clk, queue=qu)
+            for t, c in zip(saved, copies):
+                t.copy_(c)
             torch.cuda.synchronize(self.device)
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
-                self.engine.rollout(self.state, 1 + par, k, clock=clk)
+                self.engine.rollout(self.state, 1 + par, k, clock=clk, queue=qu)
             self._graphs[key] = g
         return self._graphs[key]
 
@@ -197,17 +233,10 @@ class EnsembleRollout:
           t0         start time (default: `self.time`; given, it also becomes `self.time`)
           n_step     step count at the start (the reference's n_step), max_steps an absolute limit on it (None: none)
           snap_slots snapshot-ring slots per member (default steps_per_graph: a ring drained once per block never fills)
-        Then alternate `run(k, steps_per_graph=k)` (or `step(n)`) and `drain()` until `any_active()` is False."""
-        slots = int(snap_slots if snap_slots is not None else steps_per_graph)
-        if slots < 1:
-            raise ValueError("snap_slots must be >= 1")
-        if not self.state.per_member_dt and self.B > 1:
-            raise L.PbmcError("a clock needs per_member_dt=True when B > 1: with a batch-global dt a frozen member would "
-                              "still set the others' time step")
-        clk = self._clk
-        if clk is None or clk.slots != slots:
-            self._graphs = {k: g for k, g in self._graphs.items() if "clock" not in k}  # graphs of the old buffers
-            clk = MemberClocks(self.B, self.H, self.W, self.state.dt_seq.shape[0], self.state.p is not None, slots, self.device)
+        Then alternate `run(k, steps_per_graph=k)` (or `step(n)`) and `drain()` until `any_active()` is False.
+        The clock's device buffers (and so its captured graphs) outlive stop_clock(): the next start_clock() or
+        start_sweep() with the same ring size reuses them, re-initialised, and captures nothing new."""
+        clk = self._new_clock(snap_slots, steps_per_graph)
         if t0 is None:
             t0 = self.time.cpu().numpy()
         t0 = self._per_member(t0)
@@ -224,18 +253,95 @@ class EnsembleRollout:
         self.time.copy_(torch.from_numpy(t0))
         self._clk = clk
         self._pending = None
+        self._sweep = None
         self._host_t, self._host_steps, self._host_active = t0, steps0, active
         self._t_end, self._max_steps = t_end, max_steps
 
+    def _new_clock(self, snap_slots, steps_per_graph):
+        """The MemberClocks for a clock with this ring size: the current one when it fits (its graphs stay valid)."""
+        slots = int(snap_slots if snap_slots is not None else steps_per_graph)
+        if slots < 1:
+            raise ValueError("snap_slots must be >= 1")
+        if not self.state.per_member_dt and self.B > 1:
+            raise L.PbmcError("a clock needs per_member_dt=True when B > 1: with a batch-global dt a frozen member would "
+                              "still set the others' time step")
+        clk = self._clocks
+        if clk is None or clk.slots != slots:
+            self._graphs = {k: g for k, g in self._graphs.items() if "clock" not in k}  # graphs of the old buffers
+            clk = MemberClocks(self.B, self.H, self.W, self.state.dt_seq.shape[0], self.state.p is not None, slots, self.device)
+            self._clocks = clk
+        return clk
+
+    def start_sweep(self, T0, params, t_end, save_every=0.0, t0=0.0, max_steps=None, n_step=0, snap_slots=None,
+                    steps_per_graph=10):
+        """Run Q members (`params`: Q tuples (RaQ, gamma, beta); T0: [Q, H, W]) through this ensemble's B slots, each
+        `while t < t_end and steps < max_steps` on its own clock as in start_clock (t_end, save_every, t0, max_steps,
+        n_step: scalars or one value per member).  When a slot's member stops, the device puts the next queued member
+        into the slot before the following step (include/pbmc.h, pbmc_rollout_queued: of the slots stopping at one step,
+        the lower slot index takes the earlier member), inside the same graph.  Members that would take no step are
+        finished here and never enter the queue; the first B queued members start in slots 0 .. B - 1 in member order,
+        and with fewer queued members than slots the other slots stay frozen.  Then alternate `run(k, steps_per_graph=k)` and `drain()` until `any_active()` is False.
+        The slots' T and member rows are rewritten by the sweep (`members` holds the last members afterwards), and
+        `time` keeps summing each slot's dt rows: per-member times come from drain().  A second sweep with the same
+        number of queued members and ring size reuses the buffers and the captured graphs."""
+        Qa = len(params)
+        T0 = torch.as_tensor(T0).to(torch.float32).reshape(Qa, self.H, self.W)
+        bc = lambda x, dt=np.float64: np.broadcast_to(np.asarray(x, dtype=dt), (Qa,)).copy()
+        t0, t_end, save_every = bc(t0), bc(t_end), bc(save_every)
+        steps0 = bc(n_step, np.int64)
+        max_steps = bc(_NO_LIMIT if max_steps is None else max_steps, np.int64)
+        index = np.flatnonzero((t0 < t_end) & (steps0 < max_steps))  # queue entry -> member
+        Q = len(index)
+        clk = self._new_clock(snap_slots, steps_per_graph)
+        qu = self._queue
+        if Q and (qu is None or qu.Q != Q or qu.slots != clk.slots):
+            self._graphs = {k: g for k, g in self._graphs.items() if "queue" not in k}
+            qu = self._queue = SweepQueue(Q, self.B, self.H, self.W, self.state.dt_seq.shape[0], clk.slots, self.device)
+        n0 = min(self.B, Q)
+        active = np.arange(self.B) < n0
+        c = torch.zeros(clk.clock.shape, dtype=torch.float64)
+        if Q:
+            sel = torch.from_numpy(index)
+            qu.T0.copy_(T0[sel])
+            qu.params.copy_(ops.make_members([params[i] for i in index], self.device))
+            for name, a in (("t0", t0), ("t_end", t_end), ("save_every", save_every), ("n_step0", steps0), ("max_steps", max_steps)):
+                getattr(qu, name).copy_(torch.from_numpy(a[index]))
+            qu.next.fill_(n0)
+            qu.slot_member.copy_(torch.from_numpy(np.where(active, np.arange(self.B), -1)))
+            qu.member_seq.fill_(-1)
+            qu.snap_member.fill_(-1)
+            # slots without a member keep entry 0's T and row (finite input to the surrogate); their clocks stay inactive
+            fill = torch.from_numpy(np.minimum(np.arange(self.B), n0 - 1)).to(self.device)
+            self.state.T_seq[self.n_done % 2].copy_(qu.T0[fill])
+            self.members.copy_(qu.params[fill])
+            first = index[:n0]
+            c[:n0, _T], c[:n0, _T_END] = torch.from_numpy(t0[first]), torch.from_numpy(t_end[first])
+            c[:n0, _SAVE_EVERY] = torch.from_numpy(save_every[first])
+            ci = c.view(torch.int64)
+            ci[:n0, _STEPS], ci[:n0, _MAX_STEPS] = torch.from_numpy(steps0[first]), torch.from_numpy(max_steps[first])
+        c.view(torch.int32)[:, _ACTIVE] = torch.from_numpy(active.astype(np.int32))
+        clk.clock.copy_(c)
+        self.time.copy_(c[:, _T])
+        self._clk = clk
+        self._pending = None
+        self._sweep = {"index": index, "Q": Q, "next": n0, "t": t0, "steps": steps0}
+        self._host_active = active
+
     def stop_clock(self):
-        """Back to unclocked stepping (the clocked graphs stay cached)."""
+        """Back to unclocked stepping.  Also ends a sweep.  The clock's buffers and graphs stay cached for the next
+        start_clock() / start_sweep() with the same ring size."""
         self._clk = None
         self._pending = None
+        self._sweep = None
+
+    def _run_queue(self):
+        """The SweepQueue the next steps run with (None: no sweep, or a sweep whose members all finished on the host)."""
+        return self._queue if self._sweep is not None and self._sweep["Q"] else None
 
     def set_t_end(self, t_end):
         """New end time(s) between blocks: written to the device clock, no re-capture.  A stopped member whose t is now
         below its t_end takes steps again."""
-        self._require_clock()
+        self._require_clock(sweep=False)
         self._t_end = self._per_member(t_end)
         self._host_active = (self._host_t < self._t_end) & (self._host_steps < self._max_steps)
         self._clk.clock[:, _T_END].copy_(torch.from_numpy(self._t_end))
@@ -243,22 +349,35 @@ class EnsembleRollout:
 
     def set_save_every(self, save_every):
         """New snapshot interval(s) between blocks (applies from the next snapshot on)."""
-        self._require_clock()
+        self._require_clock(sweep=False)
         self._clk.clock[:, _SAVE_EVERY].copy_(torch.from_numpy(self._per_member(save_every)))
 
     def any_active(self):
-        """Whether a member still takes steps, from the counters the last drain() read (no device access)."""
+        """Whether a member still takes steps (in a sweep: or waits in the queue), from the counters the last drain()
+        read (no device access)."""
         self._require_clock()
-        return bool(self._host_active.any())
+        sw = self._sweep
+        return bool(self._host_active.any()) or (sw is not None and sw["next"] < sw["Q"])
 
     def read_clock(self):
-        """The device clocks as numpy arrays: t, t_end, save_t, steps, snaps, drained, active, overflow (synchronises)."""
+        """The device clocks as numpy arrays: t, t_end, save_t, steps, snaps, drained, active, overflow (synchronises).
+        In a sweep (one clock per slot) also slot_member (the member in each slot, -1: none) and next (queued members
+        placed so far)."""
         self._require_clock()
         c = self._clk.clock[:, :_HDR].cpu()
         ci, ci32 = c.view(torch.int64), c.view(torch.int32)
-        return {"t": c[:, _T].numpy(), "t_end": c[:, _T_END].numpy(), "save_t": c[:, _SAVE_T].numpy(),
-                "steps": ci[:, _STEPS].numpy(), "snaps": ci[:, _SNAPS].numpy(), "drained": ci[:, _DRAINED].numpy(),
-                "active": ci32[:, _ACTIVE].numpy() != 0, "overflow": ci32[:, _OVERFLOW].numpy() != 0}
+        out = {"t": c[:, _T].numpy(), "t_end": c[:, _T_END].numpy(), "save_t": c[:, _SAVE_T].numpy(),
+               "steps": ci[:, _STEPS].numpy(), "snaps": ci[:, _SNAPS].numpy(), "drained": ci[:, _DRAINED].numpy(),
+               "active": ci32[:, _ACTIVE].numpy() != 0, "overflow": ci32[:, _OVERFLOW].numpy() != 0}
+        if self._sweep is not None:
+            qu = self._run_queue()
+            out["slot_member"] = self._member_of(qu.slot_member.cpu().numpy() if qu is not None else np.full(self.B, -1))
+            out["next"] = int(qu.next.item()) if qu is not None else 0
+        return out
+
+    def _member_of(self, entries):
+        """Queue entries (-1: none) -> member indices of the sweep (-1: none)."""
+        return np.append(self._sweep["index"], -1)[entries]
 
     def drain(self):
         """Logs of the block run since the last drain, one dict per member:
@@ -266,7 +385,9 @@ class EnsembleRollout:
           steps         int64 [n], the step numbers
           snapshots     list of dicts (step, t, T, u, v, p) in the order taken; fields float32 numpy [H,W] (p None without p_pred)
         Copies only the counters, the block's rows and the filled ring slots to the host.  Raises if a member's snapshot
-        ring overflowed (a snapshot was due while every slot held an undrained one: drain more often or use more slots)."""
+        ring overflowed (a snapshot was due while every slot held an undrained one: drain more often or use more slots).
+        In a sweep: a dict {member index: logs} over the members that took a step in the block, each with the fields
+        above plus `finished` (the member has stopped); t is the cumsum of the member's dt from its own t0."""
         self._require_clock()
         clk = self._clk
         ck = self.read_clock()
@@ -274,6 +395,8 @@ class EnsembleRollout:
             bad = np.flatnonzero(ck["overflow"]).tolist()
             raise L.PbmcError(f"snapshot ring overflow for members {bad}: a snapshot was due while all {clk.slots} slots held "
                               "undrained snapshots (it was skipped); drain() after every block or pass a larger snap_slots")
+        if self._sweep is not None:
+            return self._drain_sweep(ck)
         n = ck["steps"] - self._host_steps
         nmax = int(n.max()) if self.B else 0
         if nmax > 0:
@@ -282,15 +405,7 @@ class EnsembleRollout:
             lo = self._pending[0]
             dts = self.state.dt_seq[lo:lo + nmax].cpu().numpy()
             mts = clk.meanT_seq[lo:lo + nmax].cpu().numpy()
-        slot_idx, mem_idx = [], []
-        for m in range(self.B):
-            for j in range(int(ck["drained"][m]), int(ck["snaps"][m])):
-                slot_idx.append(j % clk.slots)
-                mem_idx.append(m)
-        if slot_idx:
-            si, mi = torch.tensor(slot_idx, device=self.device), torch.tensor(mem_idx, device=self.device)
-            ring = clk.ring[si, mi].cpu().numpy()
-            meta = clk.meta[si, mi].cpu().numpy()
+        _, ring, meta = self._ring_entries(ck)
         out, r = [], 0
         for m in range(self.B):
             k = int(n[m])
@@ -311,9 +426,66 @@ class EnsembleRollout:
         self._pending = None
         return out
 
-    def _require_clock(self):
+    def _ring_entries(self, ck):
+        """(slot, ring slot) of every undrained snapshot, slot-major, oldest first, and their ring / meta contents."""
+        clk = self._clk
+        pairs = [(m, j % clk.slots) for m in range(self.B) for j in range(int(ck["drained"][m]), int(ck["snaps"][m]))]
+        if not pairs:
+            return pairs, None, None
+        mi = torch.tensor([m for m, _ in pairs], device=self.device)
+        si = torch.tensor([j for _, j in pairs], device=self.device)
+        return pairs, clk.ring[si, mi].cpu().numpy(), clk.meta[si, mi].cpu().numpy()
+
+    def _drain_sweep(self, ck):
+        sw, clk, qu = self._sweep, self._clk, self._run_queue()
+        out = {}
+        if qu is None:
+            self._pending = None
+            return out
+        pairs, ring, meta = self._ring_entries(ck)
+        steps = {}
+        if self._pending is not None:
+            lo, k = self._pending
+            seq = self._member_of(qu.member_seq[lo:lo + k].cpu().numpy())
+            dts = self.state.dt_seq[lo:lo + k].cpu().numpy()
+            mts = clk.meanT_seq[lo:lo + k].cpu().numpy()
+            for m in np.unique(seq[seq >= 0]):
+                j, s = np.nonzero(seq == m)  # row-major: in step order (a member runs in one slot)
+                steps[int(m)] = (dts[j, s].copy(), mts[j, s].copy())
+        snaps = {}
+        if pairs:
+            owner = self._member_of(qu.snap_member.cpu().numpy())
+            for r, (s, j) in enumerate(pairs):
+                f = ring[r]
+                snaps.setdefault(int(owner[j, s]), []).append(
+                    {"step": int(meta[r, 0]), "t": float(meta[r, 1]), "T": f[0], "u": f[1], "v": f[2],
+                     "p": f[3] if clk.nch == 4 else None})
+        running = set(ck["slot_member"][ck["active"]].tolist())
+        for m in sorted(set(steps) | set(snaps)):
+            dt, mt = steps.get(m, (np.zeros(0), np.zeros(0)))
+            h_t, h_n = sw["t"][m], sw["steps"][m]
+            d = {"dt": dt, "meanT": mt, "steps": np.arange(h_n + 1, h_n + 1 + len(dt), dtype=np.int64)}
+            d["t"] = np.cumsum(np.concatenate(([h_t], dt)))[1:]  # the device's own additions: == its clock bit for bit
+            d["snapshots"] = snaps.get(m, [])
+            d["finished"] = m not in running
+            if len(dt):
+                sw["t"][m], sw["steps"][m] = d["t"][-1], d["steps"][-1]
+            out[m] = d
+        occupied = ck["slot_member"] >= 0
+        who = ck["slot_member"][occupied]
+        if not (np.array_equal(sw["steps"][who], ck["steps"][occupied]) and np.array_equal(sw["t"][who], ck["t"][occupied])):
+            raise L.PbmcError("clock counters do not match the block that was run")
+        clk.clock.view(torch.int64)[:, _DRAINED].copy_(torch.from_numpy(ck["snaps"].copy()))
+        sw["next"] = ck["next"]
+        self._host_active = ck["active"].copy()
+        self._pending = None
+        return out
+
+    def _require_clock(self, sweep=True):
         if self._clk is None:
             raise RuntimeError("no clock: call start_clock() first")
+        if not sweep and self._sweep is not None:
+            raise RuntimeError("a sweep's per-member t_end and save_every are fixed by start_sweep()")
 
     def _begin_block(self, first_row, k):
         if self._clk is None:
