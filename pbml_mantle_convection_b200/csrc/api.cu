@@ -20,19 +20,23 @@ void set_last_cuda_error(cudaError_t e, const char* where) {
 int conv_ffma_dispatch(const pbmc_conv_desc& d, cudaStream_t st);
 int conv_umma_dispatch(const pbmc_conv_desc& d, cudaStream_t st);  // conv_umma.cu
 bool conv_umma_supported(const pbmc_conv_desc& d);
-int conv_row_dispatch(const pbmc_conv_desc& d, cudaStream_t st);  // conv_row.cu
+// pdl: launch with programmatic stream serialization (the kernel waits for its predecessor with griddepcontrol.wait)
+int conv_row_dispatch(const pbmc_conv_desc& d, cudaStream_t st, bool pdl);  // conv_row.cu
 bool conv_row_supported(const pbmc_conv_desc& d);
-int conv_mux_dispatch(const pbmc_conv_desc& d, cudaStream_t st);  // conv_mux.cu
+int conv_mux_dispatch(const pbmc_conv_desc& d, cudaStream_t st, bool pdl);  // conv_mux.cu
 bool conv_mux_supported(const pbmc_conv_desc& d);
 bool conv_mux_one_wave(const pbmc_conv_desc& d);
-int conv_trunk_dispatch(const pbmc_trunk_desc& t, cudaStream_t st);  // conv_trunk.cu
+int conv_trunk_dispatch(const pbmc_trunk_desc& t, cudaStream_t st, bool pdl);  // conv_trunk.cu
 bool conv_trunk_supported(const pbmc_trunk_desc& t);
 double conv_trunk_layer_cost(int rpc);
-extern thread_local int g_conv_pdl_next;  // conv_mux.cu: the next mux launch uses programmatic dependent launch
+int head_enqueue(const float* y, const double* chan_sum, const pbmc_member* members, float a_bound, int head_kind, int p_pred,
+                 float* u, float* v, float* p, uint32_t* uvmax, int B, int H, int W, cudaStream_t st, bool pdl);  // head.cu
 int build_input_enqueue(const float* T, const float* xc, const float* yc, const float* ycc, const pbmc_member* members, float* inp,
                         float* V, int B, int H, int W, void* zero, size_t zero_bytes, cudaStream_t st, bool pdl);  // pyramid.cu
-extern thread_local int g_stencil_pdl_next;  // stencil.cu: the next plain stencil launch uses programmatic dependent launch
-extern thread_local int g_edge9_pdl_next;    // conv_edge9.cu: the next ring launch uses programmatic dependent launch
+int advect_diffuse_enqueue(const float* T, const float* u, const float* v, const float* x, const float* y,
+                           const pbmc_member* members, const uint32_t* uvmax_in, int member_stride, double dx_min, double cn_max,
+                           double dt_fixed, float* T_out, uint32_t* uvmax_out, double* dt_out, int B, int H, int W, cudaStream_t st,
+                           bool pdl);  // stencil.cu
 int clock_enqueue(pbmc_member_clock* clk, const float* Tin, float* Tout, const float* u, const float* v, const float* p,
                   double* dt_row, double* meanT_row, float* ring, double* meta, int slots, int B, int H, int W,
                   const pbmc_member_queue* queue, pbmc_member* members, int64_t* seq_row, cudaStream_t st);  // clock.cu
@@ -109,7 +113,7 @@ static int validate_conv(const pbmc_conv_desc& d) {
   return PBMC_OK;
 }
 
-static int conv_enqueue(const pbmc_conv_desc& d, cudaStream_t st) {
+static int conv_enqueue(const pbmc_conv_desc& d, cudaStream_t st, bool pdl) {
   int rc = validate_conv(d);
   if (rc != PBMC_OK) return rc;
   int impl = d.impl;
@@ -133,7 +137,7 @@ static int conv_enqueue(const pbmc_conv_desc& d, cudaStream_t st) {
     if (conv_mux_supported(d)) {
       pbmc_conv_desc e = d;
       e.impl = impl;
-      return conv_mux_dispatch(e, st);
+      return conv_mux_dispatch(e, st, pdl);
     }
     impl = impl == PBMC_CONV_MUX_F16X2 ? PBMC_CONV_ROW_F16X2 : PBMC_CONV_ROW_BF16;  // multi-source / 5x5: row kernel
   }
@@ -141,8 +145,9 @@ static int conv_enqueue(const pbmc_conv_desc& d, cudaStream_t st) {
     if (!d.wpk_row || !conv_row_supported(d)) return PBMC_ERR_UNSUPPORTED;
     pbmc_conv_desc e = d;
     e.impl = impl;
-    return conv_row_dispatch(e, st);
+    return conv_row_dispatch(e, st, pdl);
   }
+  // FFMA and UMMA never take pdl: their kernels do not execute griddepcontrol.wait
   if (impl == PBMC_CONV_FFMA) return conv_ffma_dispatch(d, st);
   if (impl == PBMC_CONV_UMMA_3XTF32 || impl == PBMC_CONV_UMMA_BF16 || impl == PBMC_CONV_UMMA_F16X2) {
     if (!d.wpk_umma || !conv_umma_supported(d)) return PBMC_ERR_UNSUPPORTED;
@@ -157,7 +162,7 @@ extern "C" int pbmc_conv_fwd(const pbmc_conv_desc* d, void* stream) {
   if (!d) return PBMC_ERR_NULL_POINTER;
   int rc = check_device_ptr(d->out);
   if (rc != PBMC_OK) return rc;
-  return conv_enqueue(*d, (cudaStream_t)stream);
+  return conv_enqueue(*d, (cudaStream_t)stream, false);
 }
 
 extern "C" int pbmc_trunk_fwd(const pbmc_trunk_desc* t, void* stream) {
@@ -167,7 +172,7 @@ extern "C" int pbmc_trunk_fwd(const pbmc_trunk_desc* t, void* stream) {
   if (!t->ping[0]) return PBMC_ERR_NULL_POINTER;
   int rc = check_device_ptr(t->ping[0]);
   if (rc != PBMC_OK) return rc;
-  return conv_trunk_dispatch(*t, (cudaStream_t)stream);
+  return conv_trunk_dispatch(*t, (cudaStream_t)stream, false);
 }
 extern "C" int pbmc_trunk_supported(const pbmc_trunk_desc* t) { return t && t->layers && conv_trunk_supported(*t) ? 1 : 0; }
 
@@ -281,17 +286,14 @@ inline void fill_conv(pbmc_conv_desc& d, const pbmc_net& n, const pbmc_layer& L,
 
 // Second launch of a learned 9-region conv: the ring kernel (pbmc_conv_edge9) over the conv `d` just enqueued -- same
 // sources, output and statistics, which it repairs for the ring pixels
-inline int ring_enqueue(const pbmc_conv_desc& d, const float* wedge, cudaStream_t st, int pdl) {
+inline int ring_enqueue(const pbmc_conv_desc& d, const float* wedge, cudaStream_t st) {
   pbmc_edge9_desc e;
   memset(&e, 0, sizeof(e));
   for (int s = 0; s < d.nsrc; ++s) e.src[s] = d.src[s];
   e.nsrc = d.nsrc; e.B = d.B; e.H = d.H; e.W = d.W;
   e.cout = d.cout; e.ksize = d.ksize; e.epi_act = d.epi_act;
   e.wedge = wedge; e.bias = d.bias; e.out = d.out; e.out_stats = d.out_stats; e.out_chan_sum = d.out_chan_sum;
-  g_edge9_pdl_next = pdl;
-  const int rc = pbmc_conv_edge9(&e, st);
-  g_edge9_pdl_next = 0;
-  return rc;
+  return pbmc_conv_edge9(&e, st);
 }
 }  // namespace
 
@@ -408,20 +410,6 @@ static bool level_cta_budgets(const pbmc_net& n, const Plan& P, int B, int H, in
       }
     }
   }
-#ifdef PBMC_DEV_BUILD
-  {
-    // developer knob: PBMC_BUDGETS="116,24,6,3,2,1" overrides the per-level CTA budgets
-    static const char* bud = getenv("PBMC_BUDGETS");
-    if (bud != nullptr && L > 1) {
-      const char* q = bud;
-      for (int l = 0; l < L && *q; ++l) {
-        cta_budget[l] = atoi(q);
-        while (*q && *q != ',') ++q;
-        if (*q == ',') ++q;
-      }
-    }
-  }
-#endif
   {
     int total = 0;
     for (int l = 0; l < L && trunk_persistent; ++l) {
@@ -444,19 +432,18 @@ static int surrogate_enqueue_on(pbmc_ctx* ctx, const pbmc_net& n, const Plan& P,
                                 const pbmc_member* members, float* u, float* v, float* p, uint32_t* uvmax, int B, int H,
                                 int W, cudaStream_t st, bool pre_zeroed) {
   const int L = P.L, R = P.R, CB = P.CB;
-  // Programmatic dependent launch on the critical chain (PBMC_CHAIN_PDL overrides the mask in a developer build; default all):
-  //   1  conv[2], conv[3]   on: nothing else runs then; the next conv's set-up overlaps the previous one's drain
-  //   4  conv[1]            on  (0.2348 -> 0.2331 -> 0.2311 ms/step at 512^2 with 1, then 1 | 4)
-  //   8  head kernel        on
-  //  16  conv[0]            on in a rollout (behind the input-build kernel, no memset node in between)
-  //   2  level-0 trunk      on for the persistent kernel (one launch behind conv[0]; its 96 CTAs leave the other levels
-  //                         their SMs: 0.2011 -> 0.2003 ms/step in 10-step graphs); with one launch PER LAYER it cost
-  //                         0.27 ms -- an early-resident CTA parked in griddepcontrol.wait took an SM from the other
-  //                         levels' streams -- and stays off there
-  //  32  ring kernels of conv[0..3] (learned nets), each directly behind its interior conv: OFF -- measured slower on B200
-  //                         (paper network, 128x506, B = 1, 10-step graphs: 0.521 vs 0.474 ms/step; 32 x 256^2: 5.41 vs
-  //                         5.41 ms), so the ring kernels launch in plain stream order
-  static const int chain_pdl = PBMC_DEV_KNOB("PBMC_CHAIN_PDL", 1 | 2 | 4 | 8 | 16);
+  // Programmatic dependent launch (pdl) on the critical chain:
+  //   conv[2], conv[3]   on: nothing else runs then; the next conv's set-up overlaps the previous one's drain
+  //   conv[1]            on  (0.2348 -> 0.2331 -> 0.2311 ms/step at 512^2 with conv[2..3], then also conv[1])
+  //   head kernel        on
+  //   conv[0]            on in a rollout (behind the input-build kernel, no memset node in between)
+  //   level-0 trunk      on for the persistent kernel (one launch behind conv[0]; its 96 CTAs leave the other levels
+  //                      their SMs: 0.2011 -> 0.2003 ms/step in 10-step graphs); with one launch PER LAYER it cost
+  //                      0.27 ms -- an early-resident CTA parked in griddepcontrol.wait took an SM from the other
+  //                      levels' streams -- and stays off there
+  //   ring kernels of conv[0..3] (learned nets), each directly behind its interior conv: OFF -- measured slower on B200
+  //                      (paper network, 128x506, B = 1, 10-step graphs: 0.521 vs 0.474 ms/step; 32 x 256^2: 5.41 vs
+  //                      5.41 ms), so the ring kernels launch in plain stream order
   const bool learned = (n.flags & PBMC_NET_LEARNED) != 0;
   auto F = [&](size_t off) { return reinterpret_cast<float*>(ws + off); };
   auto S = [&](int slot) { return reinterpret_cast<double*>(ws + P.stat_off(slot, B)); };
@@ -472,13 +459,8 @@ static int surrogate_enqueue_on(pbmc_ctx* ctx, const pbmc_net& n, const Plan& P,
   fill_conv(d, n, n.conv0, B, H, W, F(P.x0), S(0), nullptr, PBMC_ACT_NONE);
   d.nsrc = 1;
   d.src[0] = make_src(inp, P.CIB, PBMC_XFORM_NONE, nullptr, nullptr, 0.0);
-  g_conv_pdl_next = pre_zeroed ? (chain_pdl & 16) : 0;  // rollout: directly behind the input-build kernel
-  {
-    const int rc0 = conv_enqueue(d, st);
-    g_conv_pdl_next = 0;
-    RC(rc0);
-  }
-  if (learned) RC(ring_enqueue(d, n.wedge_conv0, st, chain_pdl & 32));
+  RC(conv_enqueue(d, st, pre_zeroed));  // rollout: directly behind the input-build kernel
+  if (learned) RC(ring_enqueue(d, n.wedge_conv0, st));
   PBMC_CUDA(cudaEventRecord(ctx->ev_fork[0], st));
 
   // pyramid levels (:1319-1327): level l runs on stream l (level 0 on the caller's stream)
@@ -533,12 +515,7 @@ static int surrogate_enqueue_on(pbmc_ctx* ctx, const pbmc_net& n, const Plan& P,
       t.max_ctas = L > 1 ? cta_budget[l] : 148;
       t.pre_zeroed = 1;  // the statistics / counter region was zeroed by the memset at the top of the forward
       t.loader = (n.flags & PBMC_NET_TRUNK_BULK_LOADER) ? PBMC_TRUNK_LOADER_BULK : PBMC_TRUNK_LOADER_THREADS;
-      g_conv_pdl_next = l == 0 ? (chain_pdl & 2) : 0;  // level 0 runs on the main stream, directly behind conv[0]
-      {
-        const int rct = conv_trunk_dispatch(t, sl);
-        g_conv_pdl_next = 0;
-        RC(rct);
-      }
+      RC(conv_trunk_dispatch(t, sl, l == 0));  // level 0 runs on the main stream, directly behind conv[0]
     }
     for (int r = 0; r < R && !trunk_persistent; ++r) {
       const pbmc_layer& Lr = n.trunk[l * PBMC_MAX_REPEATS + r];
@@ -552,13 +529,8 @@ static int surrogate_enqueue_on(pbmc_ctx* ctx, const pbmc_net& n, const Plan& P,
         d.src[0] = make_src(F(P.ping[l][(r - 1) & 1]), CB, PBMC_XFORM_GN_GELU, S(1 + l * R + r - 1),
                             &n.trunk[l * PBMC_MAX_REPEATS + r - 1], invc);
       }
-      g_conv_pdl_next = 0;  // one launch per layer: never (see the mask above)
-      {
-        const int rct = conv_enqueue(d, sl);
-        g_conv_pdl_next = 0;
-        RC(rct);
-      }
-      if (learned) RC(ring_enqueue(d, n.wedge_trunk[l * PBMC_MAX_REPEATS + r], sl, 0));
+      RC(conv_enqueue(d, sl, false));  // one launch per layer: never (see above)
+      if (learned) RC(ring_enqueue(d, n.wedge_trunk[l * PBMC_MAX_REPEATS + r], sl));
     }
     if (l > 0) {
       pbmc_src us = make_src(F(P.ping[l][(R - 1) & 1]), CB, PBMC_XFORM_GN_GELU, S(1 + l * R + R - 1),
@@ -582,42 +554,21 @@ static int surrogate_enqueue_on(pbmc_ctx* ctx, const pbmc_net& n, const Plan& P,
     if (up_staged) d.src[l].layout = PBMC_LAYOUT_STAGED16;
   }
   d.src[L] = make_src(inp, P.CIB, PBMC_XFORM_NONE, nullptr, nullptr, 0.0);
-  g_conv_pdl_next = chain_pdl & 4;
-  {
-    const int rc1 = conv_enqueue(d, st);
-    g_conv_pdl_next = 0;
-    RC(rc1);
-  }
-  if (learned) RC(ring_enqueue(d, n.wedge_conv1, st, chain_pdl & 32));
+  RC(conv_enqueue(d, st, true));
+  if (learned) RC(ring_enqueue(d, n.wedge_conv1, st));
   // gn[0] + act folded into conv[2]'s load; conv[2] + act (:1336-1340)
   fill_conv(d, n, n.conv2, B, H, W, F(P.h2), nullptr, nullptr, PBMC_ACT_GELU);
   d.nsrc = 1;
   d.src[0] = make_src(F(P.h1), CB, PBMC_XFORM_GN_GELU, S(1 + L * R), &n.conv1, 1.0 / (4.0 * H * W));
-  g_conv_pdl_next = chain_pdl & 1;
-  {
-    const int rc2 = conv_enqueue(d, st);
-    g_conv_pdl_next = 0;
-    RC(rc2);
-  }
-  if (learned) RC(ring_enqueue(d, n.wedge_conv2, st, chain_pdl & 32));
+  RC(conv_enqueue(d, st, true));
+  if (learned) RC(ring_enqueue(d, n.wedge_conv2, st));
   // conv[3] (:1342) with per-channel sums for the zero-mean (:1343)
   fill_conv(d, n, n.conv3, B, H, W, F(P.h3), nullptr, chan_sum, PBMC_ACT_NONE);
   d.nsrc = 1;
   d.src[0] = make_src(F(P.h2), CB, PBMC_XFORM_NONE, nullptr, nullptr, 0.0);
-  g_conv_pdl_next = chain_pdl & 1;
-  {
-    const int rc3 = conv_enqueue(d, st);
-    g_conv_pdl_next = 0;
-    RC(rc3);
-  }
-  if (learned) RC(ring_enqueue(d, n.wedge_conv3, st, chain_pdl & 32));
-  g_conv_pdl_next = chain_pdl & 8;
-  {
-    const int rch = pbmc_head(F(P.h3), chan_sum, members, n.a_bound, n.head_kind, n.p_pred, u, v, p, uvmax, B, H, W, st);
-    g_conv_pdl_next = 0;
-    RC(rch);
-  }
-  return PBMC_OK;
+  RC(conv_enqueue(d, st, true));
+  if (learned) RC(ring_enqueue(d, n.wedge_conv3, st));
+  return head_enqueue(F(P.h3), chan_sum, members, n.a_bound, n.head_kind, n.p_pred, u, v, p, uvmax, B, H, W, st, true);
 }
 
 extern "C" int pbmc_trunk_cta_budgets(const pbmc_net* net, int B, int H, int W, int* budgets) {
@@ -688,7 +639,6 @@ static int rollout_impl(pbmc_ctx* ctx, const pbmc_net* net, const pbmc_member* m
   cudaStream_t st = ctx->s[0];
   PBMC_CUDA(cudaEventRecord(ctx->ev_in, caller));
   PBMC_CUDA(cudaStreamWaitEvent(st, ctx->ev_in, 0));
-  static const int tail_pdl = PBMC_DEV_KNOB("PBMC_TAIL_PDL", 3);  // 1 stencil behind head, 2 input build behind stencil
   auto steps = [&]() -> int {
     for (int i = first_step; i < first_step + n_steps; ++i) {
       const float* Tin = T_seq + (size_t)((i - 1) % nslots) * field;
@@ -697,17 +647,15 @@ static int rollout_impl(pbmc_ctx* ctx, const pbmc_net* net, const pbmc_member* m
       // programmatic dependent launch: behind the previous step's stencil (not for the call's first step: whatever
       // precedes it in the stream is not ours)
       RC(build_input_enqueue(Tin, xc, yc, ycc, members, reinterpret_cast<float*>(ws + P.inp), last ? V : nullptr, B, H, W, ws + P.stats,
-                             P.stats_bytes, st, (tail_pdl & 2) && i > first_step));
+                             P.stats_bytes, st, i > first_step));
       RC(surrogate_enqueue_on(ctx, *net, P, ws, reinterpret_cast<float*>(ws + P.inp), members, u, v, p, uvmax, B, H, W, st, true));
       if (!per_member_dt && B > 1) {
         uvmax_batch_reduce_kernel<<<1, 32, 0, st>>>(uvmax, B);
         PBMC_CHECK_LAUNCH("uvmax_batch_reduce_kernel");
       }
-      g_stencil_pdl_next = (tail_pdl & 1) && (per_member_dt || B == 1);  // directly behind the head kernel
-      const int rcs = pbmc_advect_diffuse(Tin, u, v, xcoef, ycoef, members, uvmax, per_member_dt ? 1 : 0, dx_min, cn_max, 0.0, Tout, nullptr,
-                                          dt_seq ? dt_seq + (size_t)(i - 1) * B : nullptr, B, H, W, st);
-      g_stencil_pdl_next = 0;
-      RC(rcs);
+      // programmatic dependent launch when the stencil is directly behind the head kernel (no batch reduction between)
+      RC(advect_diffuse_enqueue(Tin, u, v, xcoef, ycoef, members, uvmax, per_member_dt ? 1 : 0, dx_min, cn_max, 0.0, Tout, nullptr,
+                                dt_seq ? dt_seq + (size_t)(i - 1) * B : nullptr, B, H, W, st, per_member_dt || B == 1));
       // plain stream order behind the stencil; the next step's input build is PDL-launched behind the commit kernel
       if (clk.clock)
         RC(clock_enqueue(clk.clock, Tin, Tout, u, v, p, dt_seq + (size_t)(i - 1) * B, clk.meanT_seq + (size_t)(i - 1) * B,

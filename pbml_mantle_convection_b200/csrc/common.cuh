@@ -33,15 +33,6 @@ void set_last_cuda_error(cudaError_t e, const char* where);
     }                                                    \
   } while (0)
 
-// Developer knobs (environment variables read at dispatch time) exist only in a development build
-// (PBMC_EXTRA_NVCC_FLAGS=-DPBMC_DEV_BUILD python -m pbml_mantle_convection_b200.build --force): the product library
-// never calls getenv -- what it runs is decided by the C-ABI arguments alone.
-#ifdef PBMC_DEV_BUILD
-#define PBMC_DEV_KNOB(name, dflt) (getenv(name) ? atoi(getenv(name)) : (dflt))
-#else
-#define PBMC_DEV_KNOB(name, dflt) (dflt)
-#endif
-
 // Kernel launch with optional programmatic stream serialization: the kernel may become resident while its predecessor in
 // the stream drains and must execute griddepcontrol.wait before it touches anything the predecessor (or, transitively,
 // anything earlier) wrote or still reads.  Without the attribute griddepcontrol.* are no-ops.

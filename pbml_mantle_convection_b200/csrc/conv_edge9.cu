@@ -173,10 +173,6 @@ __global__ void __launch_bounds__(E9_THREADS) conv_edge9_kernel(const __grid_con
 
 }  // namespace pbmc
 
-namespace pbmc {
-thread_local int g_edge9_pdl_next = 0;  // set by api.cu right before the launch it applies to
-}  // namespace pbmc
-
 using namespace pbmc;
 
 extern "C" int pbmc_conv_edge9(const pbmc_edge9_desc* d, void* stream) {
@@ -208,10 +204,8 @@ extern "C" int pbmc_conv_edge9(const pbmc_edge9_desc* d, void* stream) {
   const long ring = 2L * pd * d->W + 2L * pd * (d->H - 2 * pd);
   const size_t smem = (size_t)E9_PX * d->ksize * d->ksize * 16 * sizeof(float);
   dim3 grid((unsigned)((ring + E9_PX - 1) / E9_PX), d->B);
-  const bool pdl = g_edge9_pdl_next != 0;
-  g_edge9_pdl_next = 0;
   if (grid.y > 65535) return PBMC_ERR_BAD_SHAPE;
-  PBMC_CUDA(launch_maybe_pdl(conv_edge9_kernel, grid, dim3(E9_THREADS), smem, (cudaStream_t)stream, pdl, p));
+  conv_edge9_kernel<<<grid, E9_THREADS, smem, (cudaStream_t)stream>>>(p);
   PBMC_CHECK_LAUNCH("conv_edge9_kernel");
   return PBMC_OK;
 }

@@ -28,14 +28,9 @@
 
 namespace pbmc {
 
-#ifndef CM_NSETS
-#define CM_NSETS 5
-#endif
-constexpr int CM_SETS = CM_NSETS;                  // groups of 4 warps
+constexpr int CM_SETS = 5;                         // groups of 4 warps
 constexpr int CM_WORKERS = 4 * CM_SETS;            // 20 worker warps
-#ifndef CM_NMMA
-#define CM_NMMA 2
-#endif
+constexpr int CM_NMMA = 2;
 constexpr int CM_MMA_WARP = CM_WORKERS;            // + the MMA issuers (row ri by issuer ri % CM_NMMA; the first one owns TMEM)
 constexpr int CM_THREADS = (CM_WORKERS + CM_NMMA) * 32;
 constexpr int CM_MAXR = 24;                        // input rows per CTA (all resident in shared memory)
@@ -43,13 +38,8 @@ constexpr int CM_ND = 10;                          // TMEM accumulator ring
 constexpr int CM_N = 48;                           // (dy, c_out)
 constexpr int CM_PLANE = 136;                      // positions per K-chunk plane (128 + 2 halo, rounded up to 8)
 constexpr int CM_HDR = 2048;
-// registers are granted to a CTA in units of 4 warps: 21 warps count as 24 -> 80 per thread; 17 warps as 20 -> 96
-#ifndef CM_MAXNREG
-#define CM_MAXNREG (CM_NSETS >= 5 ? 80 : 96)
-#endif
-#ifndef CM_PREFETCH
-#define CM_PREFETCH (CM_NSETS < 5)  // a second row buffer needs the 96-register budget
-#endif
+// registers are granted to a CTA in units of 4 warps: 22 warps count as 24 -> 80 per thread
+constexpr int CM_MAXNREG = 80;
 
 struct ConvMuxParams {
   const float* in;      // [B][nblk][H][W][4]
@@ -67,17 +57,8 @@ struct ConvMuxParams {
   double* out_stats;
   double* out_chan_sum;
   unsigned long long* trace;  // developer timeline (PBMC_ROW_TRACE builds only), else NULL
-  int dbg_flags;
-  int stagger;  // TS kernel: start delay per worker group, clocks
 };
 
-// developer experiments (trace builds only; results become WRONG): 1 = no proxy fence after staging a row, 2 = no global loads,
-// 4 = GroupNorm coefficients from immediates instead of ld.shared, 8 = no MMAs (commit only), 16 = no GELU
-#ifdef PBMC_ROW_TRACE
-#define CM_DBG(flag) ((p.dbg_flags & (flag)) != 0)
-#else
-#define CM_DBG(flag) false
-#endif
 #ifdef PBMC_ROW_TRACE
 #define CM_TR(slot)                                                                                  \
   do {                                                                                               \
@@ -150,7 +131,7 @@ __global__ void __maxnreg__(CM_MAXNREG) conv_mux_kernel(const __grid_constant__ 
     const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
     R.v0 = R.v1 = R.v2 = R.v3 = z;
     R.h = 0.f;
-    if (col_ok && sy >= 0 && !CM_DBG(2)) {
+    if (col_ok && sy >= 0) {
       const float* c = cbase + ro;
       R.v0 = ldg4(c);
       if (nb > 1) R.v1 = ldg4(c + pstride);
@@ -224,21 +205,16 @@ __global__ void __maxnreg__(CM_MAXNREG) conv_mux_kernel(const __grid_constant__ 
         for (int j = 0; j < 4; j += 2) {
           if (j < nb) {
             float4 a0, b0, a1, b1;
-            if (CM_DBG(4)) {
-              a0 = a1 = make_float4(1.01f, 0.99f, 1.02f, 0.98f);
-              b0 = b1 = make_float4(0.01f, -0.01f, 0.02f, -0.02f);
-            } else {
             asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(a0.x), "=f"(a0.y), "=f"(a0.z), "=f"(a0.w) : "r"(xfa_addr + j * 16));
             asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(b0.x), "=f"(b0.y), "=f"(b0.z), "=f"(b0.w) : "r"(xfb_addr + j * 16));
             asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(a1.x), "=f"(a1.y), "=f"(a1.z), "=f"(a1.w) : "r"(xfa_addr + j * 16 + 16));
             asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(b1.x), "=f"(b1.y), "=f"(b1.z), "=f"(b1.w) : "r"(xfb_addr + j * 16 + 16));
-            }
             float x8[8];
             x8[0] = fmaf(v[4 * j + 0], a0.x, b0.x); x8[1] = fmaf(v[4 * j + 1], a0.y, b0.y);
             x8[2] = fmaf(v[4 * j + 2], a0.z, b0.z); x8[3] = fmaf(v[4 * j + 3], a0.w, b0.w);
             x8[4] = fmaf(v[4 * j + 4], a1.x, b1.x); x8[5] = fmaf(v[4 * j + 5], a1.y, b1.y);
             x8[6] = fmaf(v[4 * j + 6], a1.z, b1.z); x8[7] = fmaf(v[4 * j + 7], a1.w, b1.w);
-            if (!CM_DBG(16)) gelu_erf2n<4>(x8);
+            gelu_erf2n<4>(x8);
             if (all_keep) {
 #pragma unroll
               for (int e = 0; e < 8; ++e) v[4 * j + e] = x8[e];
@@ -283,7 +259,7 @@ __global__ void __maxnreg__(CM_MAXNREG) conv_mux_kernel(const __grid_constant__ 
           asm volatile("st.shared.b16 [%0], %1;" ::"r"(ha), "h"(__bfloat16_as_ushort(__float2bfloat16_rn(hv))) : "memory");
         }
       }
-      if (!CM_DBG(1)) fence_proxy_async_smem();
+      fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) mbar_arrive(a_full((uint32_t)ri));
       if (tr_lane) CM_TR(102 + g * 64 + 4 * (ri / CM_SETS));
@@ -375,28 +351,6 @@ __global__ void __maxnreg__(CM_MAXNREG) conv_mux_kernel(const __grid_constant__ 
         if (tr_lane) CM_TR(1202 + 3 * yo);
       };
       int ri = g, yo = g;
-#if CM_PREFETCH
-      // two row buffers: the loads of the row after next are issued as soon as a buffer has been staged (96 registers)
-      Row rb;
-      if (ri + CM_SETS < nin) load_row(ri + CM_SETS, rb);
-      while (ri < nin) {
-        stage_row(ri, ra);
-        if (ri + 2 * CM_SETS < nin) load_row(ri + 2 * CM_SETS, ra);
-        ri += CM_SETS;
-        if (yo < nrows && epi_ready(yo)) {
-          epi_row(yo);
-          yo += CM_SETS;
-        }
-        if (ri >= nin) break;
-        stage_row(ri, rb);
-        if (ri + 2 * CM_SETS < nin) load_row(ri + 2 * CM_SETS, rb);
-        ri += CM_SETS;
-        if (yo < nrows && epi_ready(yo)) {
-          epi_row(yo);
-          yo += CM_SETS;
-        }
-      }
-#else
       while (ri < nin) {
         stage_row(ri, ra);
         ri += CM_SETS;
@@ -406,7 +360,6 @@ __global__ void __maxnreg__(CM_MAXNREG) conv_mux_kernel(const __grid_constant__ 
           yo += CM_SETS;
         }
       }
-#endif
       for (; yo < nrows; yo += CM_SETS) epi_row(yo);
     };
     if (cout_blks == 4 && !epi_gelu && !want_cs)
@@ -461,7 +414,7 @@ __global__ void __maxnreg__(CM_MAXNREG) conv_mux_kernel(const __grid_constant__ 
         const uint32_t dcol = tmem_base + ds * (uint32_t)N;
         const uint64_t a_s = a_desc0 + (uint64_t)((uint32_t)ri * (uint32_t)(STAGE_BYTES >> 4));
 #pragma unroll
-        for (int dx = 0; dx < KS && !CM_DBG(8); ++dx) {
+        for (int dx = 0; dx < KS; ++dx) {
           const uint64_t a_hi = a_s + (uint64_t)dx;  // one position = 16 B
           const uint64_t b_hi = b_desc0 + (uint64_t)(dx * PARTS * (B_TILE >> 4));
           umma_ss<1>(dcol, a_hi, b_hi, IDESC, (uint32_t)dx);
@@ -487,16 +440,6 @@ __global__ void __maxnreg__(CM_MAXNREG) conv_mux_kernel(const __grid_constant__ 
   }
 }
 
-}  // namespace pbmc
-
-#if CM_NSETS == 5 && defined(PBMC_DEV_BUILD)
-#include "conv_mux_ts.cuh"  // TMEM-operand variant: correct, measured slower (DESIGN.md section 4); development builds only
-#endif
-
-namespace pbmc {
-
-thread_local int g_conv_pdl_next = 0;  // set by api.cu right before the launch it applies to
-
 #ifdef PBMC_ROW_TRACE
 static unsigned long long* g_mux_trace = nullptr;
 extern "C" void pbmc_debug_set_mux_trace(void* dev_buf) { g_mux_trace = reinterpret_cast<unsigned long long*>(dev_buf); }
@@ -505,8 +448,6 @@ extern "C" void pbmc_debug_set_mux_trace(void* dev_buf) { g_mux_trace = reinterp
 // Output rows per CTA: minimise waves x (fixed cost + staging rounds + epilogue rounds), in clocks measured with
 // tools/muxtrace.py (a staging round = 5 groups x 1 row, an epilogue round = 5 rows).
 static int choose_rpc_mux(int units, int H, int max_ctas, bool gelu) {
-  static const int forced = PBMC_DEV_KNOB("PBMC_MUX_RPC", 0);  // developer knob
-  if (forced > 0) return forced < H ? (forced < CM_MAXR - 2 ? forced : CM_MAXR - 2) : (H < CM_MAXR - 2 ? H : CM_MAXR - 2);
   const long avail = max_ctas > 0 ? max_ctas : 148;
   int best = 1;
   double best_cost = 1e30;
@@ -521,7 +462,7 @@ static int choose_rpc_mux(int units, int H, int max_ctas, bool gelu) {
 }
 
 template <int PARTS>
-static int launch_mux(ConvMuxParams& p, int max_ctas, cudaStream_t st) {
+static int launch_mux(ConvMuxParams& p, int max_ctas, cudaStream_t st, bool pdl) {
   constexpr int STAGE_BYTES = PARTS * 2 * CM_PLANE * 16, B_GROUP = 3 * PARTS * (2 * CM_N * 16);
   static bool attr_set = false;
   if (!attr_set) {
@@ -534,59 +475,12 @@ static int launch_mux(ConvMuxParams& p, int max_ctas, cudaStream_t st) {
   if (smem > 227 * 1024) return PBMC_ERR_UNSUPPORTED;
   dim3 grid(cdiv(p.H, p.rpc), nstrips, p.B);
   if (grid.y > 65535 || grid.z > 65535) return PBMC_ERR_BAD_SHAPE;
-  // Programmatic dependent launch for the convs that api.cu marks (conv[2], conv[3]: no other stream is busy then, so
-  // an early-resident CTA waiting in griddepcontrol.wait starves nobody): the set-up (barriers, TMEM, filters) runs
-  // while the producer kernel drains; the kernel reads its producer's outputs only after griddepcontrol.wait.
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = dim3(CM_THREADS);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = g_conv_pdl_next ? 1 : 0;
-  g_conv_pdl_next = 0;
-  PBMC_CUDA(cudaLaunchKernelEx(&cfg, conv_mux_kernel<PARTS>, p));
+  // With programmatic dependent launch the set-up (barriers, TMEM, filters) runs while the producer kernel drains; the
+  // kernel reads its producer's outputs only after griddepcontrol.wait.
+  PBMC_CUDA(launch_maybe_pdl(conv_mux_kernel<PARTS>, grid, dim3(CM_THREADS), smem, st, pdl, p));
   PBMC_CHECK_LAUNCH("conv_mux_kernel");
   return PBMC_OK;
 }
-
-// TS variant: nothing but the filters in shared memory, so any number of rows per CTA; cost in clocks per CTA =
-// fixed + (rows + halo) x per-row (tools/muxtrace.py)
-static int choose_rpc_ts(int units, int H, int max_ctas) {
-  static const int forced = PBMC_DEV_KNOB("PBMC_MUX_RPC", 0);  // developer knob
-  if (forced > 0) return forced < H ? forced : H;
-  const long avail = max_ctas > 0 ? max_ctas : 148;
-  int best = 1;
-  double best_cost = 1e30;
-  for (int r = 1; r <= 96 && r <= H; ++r) {
-    const long ctas = (long)units * cdiv(H, r);
-    const long waves = (ctas + avail - 1) / avail;
-    const double cost = (double)waves * (5000.0 + (r + 2) * 550.0);
-    if (cost < best_cost - 1e-9) { best_cost = cost; best = r; }
-  }
-  return best;
-}
-
-#if CM_NSETS == 5 && defined(PBMC_DEV_BUILD)
-template <int PARTS>
-static int launch_ts(ConvMuxParams& p, int max_ctas, cudaStream_t st) {
-  constexpr int B_GROUP = 3 * PARTS * (2 * CM_N * 16);
-  const int nstrips = cdiv(p.W, 128);
-  p.rpc = choose_rpc_ts(nstrips * p.B, p.H, max_ctas);
-  const size_t smem = CT_BS + (size_t)B_GROUP;
-  dim3 grid(cdiv(p.H, p.rpc), nstrips, p.B);
-  if (grid.y > 65535 || grid.z > 65535) return PBMC_ERR_BAD_SHAPE;
-  conv_ts_kernel<PARTS><<<grid, CM_THREADS, smem, st>>>(p);
-  PBMC_CHECK_LAUNCH("conv_ts_kernel");
-  return PBMC_OK;
-}
-#else  // the TMEM-operand variant is written for five worker groups (one operand slot per group)
-template <int PARTS>
-static int launch_ts(ConvMuxParams&, int, cudaStream_t) { return PBMC_ERR_UNSUPPORTED; }
-#endif
 
 // AUTO picks the mux kernel only when its whole grid is resident at once (<= one CTA per SM of the budget): it was
 // built for the short strips of a single 512^2 field; for batches that run in waves the pipelined row kernel is faster
@@ -608,7 +502,7 @@ bool conv_mux_supported(const pbmc_conv_desc& d) {
 
 // wpk_row holds two operand images back to back (ops.pack_conv_weight_row), one 16-channel group here:
 //   [fp16 hi|lo : 3 * 2 * 1536 B][bf16 : 3 * 1536 B]
-int conv_mux_dispatch(const pbmc_conv_desc& d, cudaStream_t st) {
+int conv_mux_dispatch(const pbmc_conv_desc& d, cudaStream_t st, bool pdl) {
   ConvMuxParams p;
   const pbmc_src& S = d.src[0];
   p.in = S.ptr; p.stats = S.stats; p.gamma = S.gamma; p.beta = S.beta; p.inv_count = S.inv_count;
@@ -619,9 +513,6 @@ int conv_mux_dispatch(const pbmc_conv_desc& d, cudaStream_t st) {
   p.rpc = 1;
   p.bias = d.bias; p.out = d.out; p.out_stats = d.out_stats; p.out_chan_sum = d.out_chan_sum;
   p.trace = nullptr;
-  p.dbg_flags = PBMC_DEV_KNOB("PBMC_MUX_DBG_FLAGS", 0);
-  static const int stagger = PBMC_DEV_KNOB("PBMC_MUX_STAGGER", 0);  // developer knob
-  p.stagger = stagger;
 #ifdef PBMC_ROW_TRACE
   p.trace = g_mux_trace;
 #endif
@@ -629,15 +520,13 @@ int conv_mux_dispatch(const pbmc_conv_desc& d, cudaStream_t st) {
   if (!base) return PBMC_ERR_NULL_POINTER;
   if (!aligned16(base)) return PBMC_ERR_MISALIGNED;
   const size_t off_bf16 = (size_t)3 * 2 * (2 * CM_N * 16);
-  // PBMC_MUX_TS=1 (developer knob): A operand in TMEM instead of shared memory (conv_mux_ts.cuh; correct, measured slower)
-  static const int use_ts = PBMC_DEV_KNOB("PBMC_MUX_TS", 0);
   if (d.impl == PBMC_CONV_MUX_F16X2) {
     p.wpk = base;
-    return use_ts ? launch_ts<2>(p, d.max_ctas, st) : launch_mux<2>(p, d.max_ctas, st);
+    return launch_mux<2>(p, d.max_ctas, st, pdl);
   }
   if (d.impl == PBMC_CONV_MUX_BF16) {
     p.wpk = base + off_bf16;
-    return use_ts ? launch_ts<1>(p, d.max_ctas, st) : launch_mux<1>(p, d.max_ctas, st);
+    return launch_mux<1>(p, d.max_ctas, st, pdl);
   }
   return PBMC_ERR_UNSUPPORTED;
 }

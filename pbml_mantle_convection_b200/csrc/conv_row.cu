@@ -22,7 +22,7 @@
 // Warp roles:  epilogue sets of 4 warps (output rows dealt round-robin; TMEM lane quarter = warp & 3),
 // then the producers (NPG groups of 128 threads, one thread per position plus the k-1 halo positions,
 // round-robin over stages, loads two stages ahead), last warp = MMA issuer (one elected lane) + TMEM allocator.
-// Tried and withdrawn for the several-groups variant (round 2; tools/conv1_time.py, tools/exp_conv1_mem.sh): raw fp32 rows
+// Tried and withdrawn for the several-groups variant (round 2; tools/conv1_time.py): raw fp32 rows
 // streamed by cp.async.bulk into a second shared-memory ring so that the producers neither compute addresses nor hold
 // prefetch registers.  Bit-identical, and no faster: 66.6 us with one copying lane, 58.5 us with one lane per channel plane,
 // 59.4 us with a 12-stage ring, against 58.3 us for the register-prefetch producers -- half of the producers' time then
@@ -43,13 +43,11 @@
 
 namespace pbmc {
 
-extern thread_local int g_conv_pdl_next;  // conv_mux.cu: set by api.cu right before the launch it applies to
-
 // Role split (template parameter NPG of the kernel): 5 sets of 4 warps are divided between epilogue and producers.
 //   NPG = 3: two epilogue sets (alternate output rows) + three producer groups -- one 16-channel group per row, where an
 //            output row is due after every stage;
 //   NPG = 4: one epilogue set + four producer groups -- several groups per row (conv[1]: 7 stages per output row), where
-//            the epilogue idles and the producers' serial per-stage chain sets the pace (tools/exp_conv1.sh).
+//            the epilogue idles and the producers' serial per-stage chain sets the pace.
 constexpr int CR_SETS = 5;
 constexpr int CR_MMA_WARP = 4 * CR_SETS;      // warps 0 .. 4*EPI_SETS-1 epilogue, then 4*NPG producer warps, then the MMA issuer
 constexpr int CR_TMA_WARP = CR_MMA_WARP + 1;  // one lane bulk-copies the stages of operand-image (STAGED16) sources
@@ -72,8 +70,6 @@ struct ConvRowParams {
   float* out;
   double* out_stats;
   double* out_chan_sum;
-  int dbg_dx;  // developer experiment: byte offset per dx tap (16 = correct)
-  int dbg_flags;  // developer experiment bits, see CR_DBG
   unsigned long long* trace;  // developer timeline (PBMC_ROW_TRACE builds only), else NULL
 };
 
@@ -110,16 +106,6 @@ struct RowGeom {
   static_assert(ND * DN <= 512, "TMEM has 512 columns");
   static_assert(ND >= KS + 1, "the MMA must be able to run ahead of the epilogue");
 };
-
-// Developer experiments (PBMC_ROW_TRACE builds only; results become WRONG): skip parts of the pipeline to see what
-// bounds it.  1 no MMA issue, 2 no global loads, 4 no STS, 8 no LDTM, 16 no STG, 32 no proxy fence.
-// Finding (B200, 32 x 256^2, plain 16->16): all of them skipped still costs 60 % of the full kernel's time --
-// the per-stage barrier protocol + addressing on single warps (~330 instructions, ~7 clk each) is the bound.
-#ifdef PBMC_ROW_TRACE
-#define CR_DBG(flag) ((p.dbg_flags & (flag)) != 0)
-#else
-#define CR_DBG(flag) false
-#endif
 
 #ifdef PBMC_ROW_TRACE
 #define CR_TR(slot)                                                                              \
@@ -300,7 +286,7 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
         uint32_t sl = s_lo;
 #pragma unroll
         for (int dy = 0; dy < KS; ++dy) {
-          if (!CR_DBG(8)) tmem_ld16_issue(lane_addr + sl * (uint32_t)DN + (uint32_t)(dy * 16), r[dy]);
+          tmem_ld16_issue(lane_addr + sl * (uint32_t)DN + (uint32_t)(dy * 16), r[dy]);
           if (++sl == (uint32_t)ND) sl = 0;
         }
 #pragma unroll
@@ -317,7 +303,7 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
           }
         }
         if ((tid & 127) == 0) CR_TR(1201 + 3 * yo);
-        if (col_in && !CR_DBG(16)) {
+        if (col_in) {
 #pragma unroll
           for (int qb = 0; qb < 4; ++qb) {
             if (LEAN || qb < cout_blks) {
@@ -480,7 +466,7 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
       const int sy = pad_index(y0 - P + ri, H, p.pad_mode);
       const RowGroup gi = gtab[g];
       B.ok = sy >= 0;
-      const bool ok = col_ok && sy >= 0 && !CR_DBG(2);
+      const bool ok = col_ok && sy >= 0;
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         B.v[j] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -553,8 +539,7 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
       if (tr_lane) CR_TR(101 + pg * 300 + 4 * (st / CR_NPG));
       mbar_wait_parked(a_empty(slot), (((uint32_t)st / NSTAGE) & 1u) ^ 1u);
       if (tr_lane) CR_TR(102 + pg * 300 + 4 * (st / CR_NPG));
-      if (CR_DBG(4)) {
-      } else if (PARTS == 2) {
+      if (PARTS == 2) {
         uint4 h0, l0, h1, l1;
         split_f16(v, h0, l0);
         split_f16(v + 8, h1, l1);
@@ -583,7 +568,7 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
           }
         }
       }
-      if (!CR_DBG(32)) fence_proxy_async_smem();
+      fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) mbar_arrive(a_full(slot));
       if (tr_lane) CR_TR(103 + pg * 300 + 4 * (st / CR_NPG));
@@ -658,8 +643,7 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
         auto sts = [](uint32_t addr, uint4 q) {
           asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(q.x), "r"(q.y), "r"(q.z), "r"(q.w) : "memory");
         };
-        if (CR_DBG(4)) {
-        } else if (PARTS == 2) {
+        if (PARTS == 2) {
           uint4 h0, l0, h1, l1;
           split_f16(v, h0, l0);
           split_f16(v + 8, h1, l1);
@@ -683,7 +667,7 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
           }
         }
         if (tr_lane) CR_TR(104 + pg * 300 + 8 * (st / CR_NPG));
-        if (!CR_DBG(32)) fence_proxy_async_smem();
+        fence_proxy_async_smem();
         if (tr_lane) CR_TR(105 + pg * 300 + 8 * (st / CR_NPG));
         __syncwarp();
         if (lane == 0) mbar_arrive(a_full(slot));
@@ -738,7 +722,7 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
           B.v0 = B.v1 = B.v2 = B.v3 = z;
           B.h = 0.f;
           const float* cb = gi.base + coff + ro;
-          if (col_ok && sy >= 0 && !CR_DBG(2)) {
+          if (col_ok && sy >= 0) {
             B.v0 = ldg4(cb);
             if (gi.nb > 1) B.v1 = ldg4(cb + pstride);
             if (gi.nb > 2) B.v2 = ldg4(cb + 2 * pstride);
@@ -776,8 +760,7 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
           auto sts = [](uint32_t addr, uint4 q) {
             asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(q.x), "r"(q.y), "r"(q.z), "r"(q.w) : "memory");
           };
-          if (CR_DBG(4)) {
-          } else if (PARTS == 2) {
+          if (PARTS == 2) {
             uint4 h0, l0, h1, l1;
             split_f16(v, h0, l0);
             split_f16(v + 8, h1, l1);
@@ -801,7 +784,7 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
             }
           }
           if (tr_lane && st / CR_NPG < 37) CR_TR(104 + pg * 300 + 8 * (st / CR_NPG));
-          if (!CR_DBG(32)) fence_proxy_async_smem();
+          fence_proxy_async_smem();
           if (tr_lane && st / CR_NPG < 37) CR_TR(105 + pg * 300 + 8 * (st / CR_NPG));
           __syncwarp();
           if (lane == 0) mbar_arrive(a_full(slot));
@@ -865,11 +848,6 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
     const bool leader = elect_one();
     constexpr uint32_t A_LBO = PLANE * 16, B_LBO = (MERGE ? 2 * N : N) * 16, SBO = 128;
     const uint64_t a_desc0 = umma_desc(smem_u32(As), A_LBO, SBO), b_desc0 = umma_desc(smem_u32(Bs), B_LBO, SBO);
-#ifdef PBMC_ROW_TRACE
-    const uint32_t dx_step = (uint32_t)p.dbg_dx >> 4;
-#else
-    constexpr uint32_t dx_step = 1;  // one position = 16 B
-#endif
     const uint32_t smask = *stg_mask;
     auto sel = [&](int g, uint32_t pk, uint32_t tk, uint32_t& full, uint32_t& par, uint32_t& sidx, uint32_t& empty) {
       if ((smask >> g) & 1u) {
@@ -900,9 +878,8 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
             const uint64_t b_s = b_desc0 + (uint64_t)((uint32_t)g * (uint32_t)(G::B_GROUP >> 4));
 #pragma unroll
             for (int dx = 0; dx < KS; ++dx) {
-              const uint64_t a_hi = a_s + (uint64_t)(dx * dx_step);
+              const uint64_t a_hi = a_s + (uint64_t)dx;  // one position = 16 B
               const uint64_t b_hi = b_s + (uint64_t)(dx * PARTS * (G::B_TILE >> 4));
-              if (CR_DBG(1)) continue;
               if (MERGE) {
                 umma_ss<1>(dcol, a_hi, b_hi, IDESC2, (uint32_t)(g | dx));                          // A_hi x [W_hi ; W_lo] -> 96 columns
                 umma_ss<1>(dcol, a_hi + (uint64_t)(G::PART_BYTES >> 4), b_hi, IDESC, 1u);          // A_lo x W_hi -> the first 48
@@ -945,9 +922,8 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
             const uint64_t b_s = b_desc0 + (uint64_t)((uint32_t)g * (uint32_t)(G::B_GROUP >> 4));
   #pragma unroll
             for (int dx = 0; dx < KS; ++dx) {
-              const uint64_t a_hi = a_s + (uint64_t)(dx * dx_step);
+              const uint64_t a_hi = a_s + (uint64_t)dx;  // one position = 16 B
               const uint64_t b_hi = b_s + (uint64_t)(dx * PARTS * (G::B_TILE >> 4));
-              if (CR_DBG(1)) continue;
               if (MERGE) {
                 umma_ss<1>(dcol, a_hi, b_hi, IDESC2, (uint32_t)(g | dx));                          // A_hi x [W_hi ; W_lo] -> 96 columns
                 umma_ss<1>(dcol, a_hi + (uint64_t)(G::PART_BYTES >> 4), b_hi, IDESC, 1u);          // A_lo x W_hi -> the first 48
@@ -1019,8 +995,6 @@ extern "C" void pbmc_debug_set_row_trace(void* dev_buf) { g_row_trace = reinterp
 
 // rows per CTA: minimise waves * (rows + halo + fixed per-CTA cost in row units)
 static int choose_rpc(int units, int H, int ks, int max_ctas) {
-  static const int forced = PBMC_DEV_KNOB("PBMC_ROW_RPC", 0);  // developer knob
-  if (forced > 0) return forced < H ? forced : H;
   if (max_ctas > 0) {
     // a share of the GPU: the fewest rows per CTA that stay within the CTA budget (the conv runs next to others)
     for (int r = 1; r <= H; ++r)
@@ -1038,7 +1012,7 @@ static int choose_rpc(int units, int H, int ks, int max_ctas) {
 }
 
 template <int KS, int PARTS, int NPG>
-static int launch_row_npg(ConvRowParams& p, cudaStream_t st) {
+static int launch_row_npg(ConvRowParams& p, cudaStream_t st, bool pdl) {
   using G = RowGeom<KS, PARTS>;
   const size_t smem = CR_SMEM_HDR + (size_t)p.ngroups * G::B_GROUP + (size_t)(G::NSTAGE + (p.has_staged ? CR_NT : 0)) * G::STAGE_BYTES +
                       (size_t)p.cin_ch * 8;
@@ -1052,32 +1026,16 @@ static int launch_row_npg(ConvRowParams& p, cudaStream_t st) {
   p.rpc = choose_rpc(nstrips * p.B, p.H, KS, p.max_ctas);
   dim3 grid(cdiv(p.H, p.rpc), nstrips, p.B);
   if (grid.y > 65535 || grid.z > 65535) return PBMC_ERR_BAD_SHAPE;
-  // Programmatic dependent launch is wired but OFF: measured 0.269 vs 0.243 ms/step at 512^2 -- a dependent CTA that
-  // becomes resident early sits in griddepcontrol.wait holding an SM (a conv CTA owns one), which starves the
-  // other pyramid levels' streams.  (With PDL off griddepcontrol.wait / launch_dependents are no-ops.)
-  static const int pdl = PBMC_DEV_KNOB("PBMC_ROW_PDL", 0);  // developer knob
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = dim3(CR_THREADS);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = (pdl || g_conv_pdl_next) ? 1 : 0;
-  g_conv_pdl_next = 0;
-  PBMC_CUDA(cudaLaunchKernelEx(&cfg, conv_row_kernel<KS, PARTS, NPG>, p));
+  PBMC_CUDA(launch_maybe_pdl(conv_row_kernel<KS, PARTS, NPG>, grid, dim3(CR_THREADS), smem, st, pdl, p));
   PBMC_CHECK_LAUNCH("conv_row_kernel");
   return PBMC_OK;
 }
 
 template <int KS, int PARTS>
-static int launch_row(ConvRowParams& p, cudaStream_t st) {
+static int launch_row(ConvRowParams& p, cudaStream_t st, bool pdl) {
   // several K groups per input row (conv[1]): four producer groups, one epilogue set; else three and two
-  static const int forced = PBMC_DEV_KNOB("PBMC_ROW_NPG", 0);  // developer knob
-  const bool heavy = forced ? forced == 4 : p.ngroups >= 3;
-  return heavy ? launch_row_npg<KS, PARTS, 4>(p, st) : launch_row_npg<KS, PARTS, 3>(p, st);
+  const bool heavy = p.ngroups >= 3;
+  return heavy ? launch_row_npg<KS, PARTS, 4>(p, st, pdl) : launch_row_npg<KS, PARTS, 3>(p, st, pdl);
 }
 
 static int row_groups(const pbmc_conv_desc& d) {
@@ -1104,7 +1062,7 @@ bool conv_row_supported(const pbmc_conv_desc& d) {
 
 // wpk_row holds two operand images back to back (ops.pack_conv_weight_row):
 //   [fp16 hi|lo : groups * k * 2 * (2*N*16) B][bf16 : groups * k * (2*N*16) B]
-int conv_row_dispatch(const pbmc_conv_desc& d, cudaStream_t st) {
+int conv_row_dispatch(const pbmc_conv_desc& d, cudaStream_t st, bool pdl) {
   ConvRowParams p;
   int cin = 0;
   for (int s = 0; s < d.nsrc; ++s) {
@@ -1121,8 +1079,6 @@ int conv_row_dispatch(const pbmc_conv_desc& d, cudaStream_t st) {
   p.has_staged = 0;
   for (int s = 0; s < d.nsrc; ++s) p.has_staged |= d.src[s].layout == PBMC_LAYOUT_STAGED16;
   p.trace = nullptr;
-  p.dbg_dx = PBMC_DEV_KNOB("PBMC_ROW_DBG_DX", 16);
-  p.dbg_flags = PBMC_DEV_KNOB("PBMC_ROW_DBG_FLAGS", 0);
 #ifdef PBMC_ROW_TRACE
   p.trace = g_row_trace;
 #endif
@@ -1143,11 +1099,11 @@ int conv_row_dispatch(const pbmc_conv_desc& d, cudaStream_t st) {
   const size_t off_bf16 = (size_t)p.ngroups * d.ksize * 2 * (2 * n * 16);
   if (d.impl == PBMC_CONV_ROW_F16X2) {
     p.wpk = base;
-    return d.ksize == 3 ? launch_row<3, 2>(p, st) : launch_row<5, 2>(p, st);
+    return d.ksize == 3 ? launch_row<3, 2>(p, st, pdl) : launch_row<5, 2>(p, st, pdl);
   }
   if (d.impl == PBMC_CONV_ROW_BF16) {
     p.wpk = base + off_bf16;
-    return d.ksize == 3 ? launch_row<3, 1>(p, st) : launch_row<5, 1>(p, st);
+    return d.ksize == 3 ? launch_row<3, 1>(p, st, pdl) : launch_row<5, 1>(p, st, pdl);
   }
   return PBMC_ERR_UNSUPPORTED;
 }

@@ -29,15 +29,10 @@
 
 namespace pbmc {
 
-extern thread_local int g_conv_pdl_next;  // conv_mux.cu: set by api.cu right before the launch it applies to
-
-// Six groups (-DPBMC_CT_SETS=6: 832 threads at 72 registers, three staging rounds instead of four at 16 input rows) were
-// measured against five (tools/exp_ct_sets.sh): 68.6 vs 68.6 us per 4-layer launch at 148 CTAs, 85.1 vs 85.0 at 96 -- fewer
-// rounds, each slower by the same factor: the staging rounds are bound by issued instructions, not by their number.
-#ifndef PBMC_CT_SETS
-#define PBMC_CT_SETS 5
-#endif
-constexpr int CT_SETS = PBMC_CT_SETS;            // groups of 4 worker warps
+// Six groups (832 threads at 72 registers, three staging rounds instead of four at 16 input rows) were measured against
+// five: 68.6 vs 68.6 us per 4-layer launch at 148 CTAs, 85.1 vs 85.0 at 96 -- fewer rounds, each slower by the same
+// factor: the staging rounds are bound by issued instructions, not by their number.
+constexpr int CT_SETS = 5;                       // groups of 4 worker warps
 constexpr int CT_WORKERS = 4 * CT_SETS;          // 20 worker warps
 constexpr int CT_NMMA = 2;                       // MMA issuer warps (alternate rows); the first one owns TMEM
 constexpr int CT_MMA_WARP = CT_WORKERS;
@@ -558,7 +553,7 @@ bool conv_trunk_supported(const pbmc_trunk_desc& t) {
 }
 
 template <int PARTS, bool BULK>
-static int launch_trunk(ConvTrunkParams& p, cudaStream_t st) {
+static int launch_trunk(ConvTrunkParams& p, cudaStream_t st, bool pdl) {
   constexpr int STAGE_BYTES = PARTS * 2 * CT_PLANE * 16, B_GROUP = 3 * PARTS * (2 * CT_N * 16);
   static bool attr_set = false;
   if (!attr_set) {
@@ -568,15 +563,13 @@ static int launch_trunk(ConvTrunkParams& p, cudaStream_t st) {
   const size_t smem = CT_HDR + (size_t)2 * B_GROUP + (size_t)(p.rpc + 2) * STAGE_BYTES;
   if (smem > 227 * 1024) return PBMC_ERR_UNSUPPORTED;
   dim3 grid(cdiv(p.H, p.rpc), cdiv(p.W, 128), p.B);
-  const bool pdl = g_conv_pdl_next != 0;
-  g_conv_pdl_next = 0;
   PBMC_CUDA(launch_maybe_pdl(conv_trunk_kernel<PARTS, BULK>, grid, dim3(CT_THREADS), smem, st, pdl, p));
   PBMC_CHECK_LAUNCH("conv_trunk_kernel");
   return PBMC_OK;
 }
 
 // wpk_row of a layer: [fp16 hi|lo : 3 * 2 * 1536 B][bf16 : 3 * 1536 B] (ops.pack_conv_weight_row, one 16-channel group)
-int conv_trunk_dispatch(const pbmc_trunk_desc& t, cudaStream_t st) {
+int conv_trunk_dispatch(const pbmc_trunk_desc& t, cudaStream_t st, bool pdl) {
   if (!conv_trunk_supported(t)) return PBMC_ERR_UNSUPPORTED;
   if (!t.src0.ptr || !t.ping[0] || !t.ping[1] || !t.stats || !t.sync) return PBMC_ERR_NULL_POINTER;
   if (!aligned16(t.src0.ptr) || !aligned16(t.ping[0]) || !aligned16(t.ping[1])) return PBMC_ERR_MISALIGNED;
@@ -610,8 +603,8 @@ int conv_trunk_dispatch(const pbmc_trunk_desc& t, cudaStream_t st) {
     PBMC_CUDA(cudaMemsetAsync(t.sync, 0, (size_t)t.B * sizeof(unsigned int), st));
     PBMC_CUDA(cudaMemsetAsync(t.stats, 0, (size_t)t.R * t.B * 8 * sizeof(double), st));
   }
-  if (bf16) return launch_trunk<1, false>(p, st);
-  return t.loader == PBMC_TRUNK_LOADER_BULK ? launch_trunk<2, true>(p, st) : launch_trunk<2, false>(p, st);
+  if (bf16) return launch_trunk<1, false>(p, st, pdl);
+  return t.loader == PBMC_TRUNK_LOADER_BULK ? launch_trunk<2, true>(p, st, pdl) : launch_trunk<2, false>(p, st, pdl);
 }
 
 }  // namespace pbmc

@@ -356,17 +356,12 @@ int conv_umma_dispatch(const pbmc_conv_desc& d, cudaStream_t st) {
     p.wpk = base;
     return d.ksize == 3 ? launch_umma<3, 64, 15, 8, CU_TF32X3>(p, st) : launch_umma<5, 64, 15, 8, CU_TF32X3>(p, st);
   }
-  static const int tile_cfg = PBMC_DEV_KNOB("PBMC_UMMA_TILE", 0);  // developer knob
   if (d.impl == PBMC_CONV_UMMA_F16X2) {
     p.wpk = base + off_f16;
-    if (d.ksize == 3 && tile_cfg == 1) return launch_umma<3, 64, 7, 4, CU_F16X2>(p, st);
-    if (d.ksize == 3 && tile_cfg == 2) return launch_umma<3, 128, 7, 8, CU_F16X2>(p, st);
     return d.ksize == 3 ? launch_umma<3, 64, 15, 8, CU_F16X2>(p, st) : launch_umma<5, 64, 15, 8, CU_F16X2>(p, st);
   }
   if (d.impl == PBMC_CONV_UMMA_BF16) {
     p.wpk = base + off_bf16;
-    if (d.ksize == 3 && tile_cfg == 1) return launch_umma<3, 64, 7, 4, CU_BF16>(p, st);
-    if (d.ksize == 3 && tile_cfg == 2) return launch_umma<3, 128, 7, 8, CU_BF16>(p, st);
     return d.ksize == 3 ? launch_umma<3, 64, 15, 8, CU_BF16>(p, st) : launch_umma<5, 64, 15, 8, CU_BF16>(p, st);
   }
   return PBMC_ERR_UNSUPPORTED;

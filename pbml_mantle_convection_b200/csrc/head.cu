@@ -9,8 +9,6 @@
 
 namespace pbmc {
 
-extern thread_local int g_conv_pdl_next;  // conv_mux.cu: set by api.cu right before the launch it applies to
-
 __global__ void __launch_bounds__(256) head_kernel(const float* __restrict__ y, const double* __restrict__ chan_sum,
                                                    const pbmc_member* __restrict__ mem, float a_bound, int head_kind,
                                                    int p_pred, float* __restrict__ u, float* __restrict__ v,
@@ -69,30 +67,24 @@ __global__ void __launch_bounds__(256) head_kernel(const float* __restrict__ y, 
   }
 }
 
-}  // namespace pbmc
-
-using namespace pbmc;
-
-extern "C" int pbmc_head(const float* y, const double* chan_sum, const pbmc_member* members, float a_bound,
-                         int head_kind, int p_pred, float* u, float* v, float* p, uint32_t* uvmax, int B, int H, int W,
-                         void* stream) {
+int head_enqueue(const float* y, const double* chan_sum, const pbmc_member* members, float a_bound, int head_kind, int p_pred,
+                 float* u, float* v, float* p, uint32_t* uvmax, int B, int H, int W, cudaStream_t st, bool pdl) {
   if (!y || !chan_sum || !u || !v) return PBMC_ERR_NULL_POINTER;
   if (B <= 0 || H < 3 || W < 3) return PBMC_ERR_BAD_SHAPE;
   if (head_kind != PBMC_HEAD_CURL && head_kind != PBMC_HEAD_MAE) return PBMC_ERR_UNSUPPORTED;
   if (!aligned16(y)) return PBMC_ERR_MISALIGNED;
   dim3 grid(cdiv(W, 32), cdiv(H, 8), B);
   if (grid.y > 65535 || grid.z > 65535) return PBMC_ERR_BAD_SHAPE;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = dim3(32, 8);
-  cfg.stream = (cudaStream_t)stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pbmc::g_conv_pdl_next ? 1 : 0;
-  pbmc::g_conv_pdl_next = 0;
-  PBMC_CUDA(cudaLaunchKernelEx(&cfg, head_kernel, y, chan_sum, members, a_bound, head_kind, p_pred, u, v, p, uvmax, H, W));
+  PBMC_CUDA(launch_maybe_pdl(head_kernel, grid, dim3(32, 8), 0, st, pdl, y, chan_sum, members, a_bound, head_kind, p_pred, u, v, p,
+                             uvmax, H, W));
   PBMC_CHECK_LAUNCH("head_kernel");
   return PBMC_OK;
+}
+
+}  // namespace pbmc
+
+extern "C" int pbmc_head(const float* y, const double* chan_sum, const pbmc_member* members, float a_bound,
+                         int head_kind, int p_pred, float* u, float* v, float* p, uint32_t* uvmax, int B, int H, int W,
+                         void* stream) {
+  return pbmc::head_enqueue(y, chan_sum, members, a_bound, head_kind, p_pred, u, v, p, uvmax, B, H, W, (cudaStream_t)stream, false);
 }

@@ -556,14 +556,11 @@ extern "C" int pbmc_stencil_coefs(const double* coord, int n, double wall_lo, do
   return PBMC_OK;
 }
 
-namespace pbmc {
-thread_local int g_stencil_pdl_next = 0;  // set by api.cu (pbmc_rollout) right before the launch it applies to
-}
-
+// pdl: the plain (non-slab) marching kernel is launched with programmatic stream serialization
 static int advect_diffuse_launch(const float* T, const float* u, const float* v, const float* x, const float* y,
                                  const pbmc_member* members, const uint32_t* uvmax_in, int member_stride, double dx_min,
                                  double cn_max, double dt_fixed, float* T_out, uint32_t* uvmax_out, double* dt_out, int B, int H,
-                                 int W, int has_up, int has_down, float* peer_up, float* peer_down, void* stream,
+                                 int W, int has_up, int has_down, float* peer_up, float* peer_down, void* stream, bool pdl,
                                  const SlabSyncArgs* sync = nullptr) {
   if (!T || !u || !v || !x || !y || !T_out) return PBMC_ERR_NULL_POINTER;
   if (!(dt_fixed > 0.0) && !uvmax_in && !sync) return PBMC_ERR_NULL_POINTER;
@@ -573,8 +570,7 @@ static int advect_diffuse_launch(const float* T, const float* u, const float* v,
   StencilParams p{T, u, v, x, y, members, uvmax_in, uvmax_out, T_out, dt_out, dx_min, cn_max, dt_fixed, member_stride, H, W,
                   has_up ? 1 : 0, has_down ? H - 1 : H, has_up ? 1 : -1, has_down ? H - 2 : -1, peer_up, peer_down};
   const bool vec = (W % 4 == 0) && aligned16(T) && aligned16(u) && aligned16(v) && aligned16(T_out);
-  static const int tiled = PBMC_DEV_KNOB("PBMC_STENCIL_TILED", 0);  // developer knob: old kernel
-  if (vec && aligned16(x) && (!tiled || slab)) {
+  if (vec && aligned16(x)) {
     if ((peer_up && !aligned16(peer_up)) || (peer_down && !aligned16(peer_down))) return PBMC_ERR_MISALIGNED;
     // Rows per warp.  The grid runs in waves of (resident CTAs per SM) x (SMs) CTAs and every CTA takes the same time
     // (~ rpw + a few rows of fixed cost), so the sweep time is waves x (rpw + c): pick the rpw in [4, 128] that minimises it
@@ -606,8 +602,6 @@ static int advect_diffuse_launch(const float* T, const float* u, const float* v,
     if (sync != nullptr) {
       stencil_march_kernel<true><<<grid, 128, 0, (cudaStream_t)stream>>>(p, rpw, *sync);
     } else {
-      const bool pdl = g_stencil_pdl_next != 0;
-      g_stencil_pdl_next = 0;
       PBMC_CUDA(launch_maybe_pdl(stencil_march_kernel<false>, grid, dim3(128), 0, (cudaStream_t)stream, pdl, p, rpw, SlabSyncArgs{}));
     }
     PBMC_CHECK_LAUNCH("stencil_march_kernel");
@@ -625,12 +619,22 @@ static int advect_diffuse_launch(const float* T, const float* u, const float* v,
   return PBMC_OK;
 }
 
+namespace pbmc {
+int advect_diffuse_enqueue(const float* T, const float* u, const float* v, const float* x, const float* y,
+                           const pbmc_member* members, const uint32_t* uvmax_in, int member_stride, double dx_min, double cn_max,
+                           double dt_fixed, float* T_out, uint32_t* uvmax_out, double* dt_out, int B, int H, int W, cudaStream_t st,
+                           bool pdl) {
+  return advect_diffuse_launch(T, u, v, x, y, members, uvmax_in, member_stride, dx_min, cn_max, dt_fixed, T_out, uvmax_out,
+                               dt_out, B, H, W, 0, 0, nullptr, nullptr, st, pdl);
+}
+}  // namespace pbmc
+
 extern "C" int pbmc_advect_diffuse(const float* T, const float* u, const float* v, const float* x, const float* y,
                                    const pbmc_member* members, const uint32_t* uvmax_in, int member_stride,
                                    double dx_min, double cn_max, double dt_fixed, float* T_out, uint32_t* uvmax_out,
                                    double* dt_out, int B, int H, int W, void* stream) {
-  return advect_diffuse_launch(T, u, v, x, y, members, uvmax_in, member_stride, dx_min, cn_max, dt_fixed, T_out, uvmax_out,
-                               dt_out, B, H, W, 0, 0, nullptr, nullptr, stream);
+  return advect_diffuse_enqueue(T, u, v, x, y, members, uvmax_in, member_stride, dx_min, cn_max, dt_fixed, T_out, uvmax_out,
+                                dt_out, B, H, W, (cudaStream_t)stream, false);
 }
 
 extern "C" int pbmc_advect_diffuse_slab(const float* T, const float* u, const float* v, const float* x, const float* y,
@@ -640,7 +644,7 @@ extern "C" int pbmc_advect_diffuse_slab(const float* T, const float* u, const fl
                                         void* stream) {
   if ((peer_up_ghost_row && !has_up) || (peer_down_ghost_row && !has_down)) return PBMC_ERR_BAD_SHAPE;
   return advect_diffuse_launch(T, u, v, x, y, members, uvmax_in, 0, dx_min, cn_max, dt_fixed, T_out, uvmax_out, dt_out, 1, H, W,
-                               has_up, has_down, peer_up_ghost_row, peer_down_ghost_row, stream);
+                               has_up, has_down, peer_up_ghost_row, peer_down_ghost_row, stream, false);
 }
 
 static int make_sync_args(pbmc_slab_sync* self, pbmc_slab_sync* const* peers_h, int rank, int world, SlabSyncArgs& a) {
@@ -683,7 +687,7 @@ extern "C" int pbmc_advect_diffuse_slab_sync(const float* T, const float* u, con
   const int rc = make_sync_args(self, peers_h, rank, world, a);
   if (rc != PBMC_OK) return rc;
   return advect_diffuse_launch(T, u, v, x, y, members, nullptr, 0, dx_min, cn_max, 0.0, T_out, nullptr, dt_out, 1, H, W, has_up,
-                               has_down, peer_up_ghost_row, peer_down_ghost_row, stream, &a);
+                               has_down, peer_up_ghost_row, peer_down_ghost_row, stream, false, &a);
 }
 
 extern "C" int pbmc_uvmax(const float* u, const float* v, uint32_t* uvmax, int member_stride, int B, int H, int W,

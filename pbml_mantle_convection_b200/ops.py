@@ -202,9 +202,9 @@ def finalize_nchw(src: Source, Cc: int) -> torch.Tensor:
 
 # ------------------------------------------------------------------ conv
 def conv_fwd(sources, wpk, bias, cout, ksize, pad_mode, epi_act=L.ACT_NONE, want_stats=False, want_chan_sum=False,
-             impl="auto", wpk_umma=None, out=None, stats=None, csum=None, wpk_row=None):
+             impl="auto", wpk_umma=None, out=None, stats=None, csum=None, wpk_row=None, max_ctas=0):
     """Returns (out_blocked, stats|None, chan_sum|None).  `out`/`stats`/`csum` may be preallocated
-    (statistics ACCUMULATE into the given buffers, as in the C ABI)."""
+    (statistics ACCUMULATE into the given buffers, as in the C ABI).  `max_ctas`: CTA budget (0 = the whole GPU)."""
     t0 = sources[0].t
     B, _, H, W, _ = t0.shape
     dev = t0.device
@@ -221,7 +221,7 @@ def conv_fwd(sources, wpk, bias, cout, ksize, pad_mode, epi_act=L.ACT_NONE, want
         d.src[i] = s.c()
     d.B, d.H, d.W, d.cout, d.ksize = B, H, W, int(cout), int(ksize)
     d.pad_mode = L.PAD[pad_mode] if isinstance(pad_mode, str) else int(pad_mode)
-    d.epi_act, d.impl = int(epi_act), L.CONV_IMPL[impl]
+    d.epi_act, d.impl, d.max_ctas = int(epi_act), L.CONV_IMPL[impl], int(max_ctas)
     d.wpk, d.wpk_umma, d.bias, d.out = L.ptr(wpk), L.ptr(wpk_umma), L.ptr(bias), L.ptr(out)
     d.wpk_row = L.ptr(wpk_row)
     d.out_stats, d.out_chan_sum = L.ptr(stats), L.ptr(csum)

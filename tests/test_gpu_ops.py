@@ -254,44 +254,30 @@ def test_conv_mux_fused_groupnorm_gelu_and_epilogue_gelu(H, W, pad):
     assert relerr(ops.unpack_nchw(out, 16).cpu().numpy(), ref) < 5e-6
 
 
-@pytest.mark.parametrize("ts", [0, 1])
-@pytest.mark.parametrize("rpc", [1, 2, 3, 7, 22])
-def test_conv_mux_any_rows_per_cta(rpc, ts):
-    """Rows per CTA is a scheduling choice: same result for any of them, with the A operand staged in shared memory
-    (ts=0, default) and in tensor memory (ts=1, csrc/conv_mux_ts.cuh: accumulator / operand rings wrap from 6 rows on)."""
-    import os, subprocess, sys
-    code = (
-        "import numpy as np, torch\n"
-        "from oracle import ref_numpy as RN\n"
-        "from pbml_mantle_convection_b200 import ops\n"
-        "r=np.random.default_rng(5); x=r.standard_normal((1,16,37,150)); w=r.standard_normal((16,16,3,3))/12; b=r.standard_normal(16)\n"
-        "cu=lambda a: torch.tensor(np.ascontiguousarray(a),dtype=torch.float32,device='cuda:0')\n"
-        "o,_,_=ops.conv_fwd([ops.Source(ops.pack_nchw(cu(x)))],ops.pack_conv_weight(cu(w),[16]),ops.pad_vec(cu(b),16,'cuda:0'),16,3,'replicate',impl='mux_f16x2',wpk_row=ops.pack_conv_weight_row(cu(w),[16]))\n"
-        "y=ops.unpack_nchw(o,16).cpu().numpy(); ref=RN.conv2d_same(x,w,b,'replicate')\n"
-        "e=np.linalg.norm(y-ref)/np.linalg.norm(ref); print(e); assert e<3e-6\n")
-    env = dict(os.environ, PBMC_MUX_RPC=str(rpc), PBMC_MUX_TS=str(ts))
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    res = subprocess.run([sys.executable, "-c", code], cwd=root, env=env, capture_output=True, text=True, timeout=300)
-    assert res.returncode == 0, res.stdout + res.stderr
+def _conv_37x150(impl, max_ctas):
+    """One 16 -> 16 3x3 conv of a 37 x 150 field (two 128-column strips) under a CTA budget, against the float64 oracle."""
+    r = rng(5)
+    x, w, b = r.standard_normal((1, 16, 37, 150)), r.standard_normal((16, 16, 3, 3)) / 12, r.standard_normal(16)
+    out, _, _ = ops.conv_fwd([ops.Source(ops.pack_nchw(cu(x)))], ops.pack_conv_weight(cu(w), [16]), ops.pad_vec(cu(b), 16, DEV),
+                             16, 3, "replicate", impl=impl, wpk_row=ops.pack_conv_weight_row(cu(w), [16]), max_ctas=max_ctas)
+    err = relerr(ops.unpack_nchw(out, 16).cpu().numpy(), RN.conv2d_same(x, w, b, "replicate"))
+    assert err < 3e-6, err
 
 
-@pytest.mark.parametrize("rpc", [1, 2, 5, 64])
-def test_conv_row_any_rows_per_cta(rpc, monkeypatch):
+# CTA budget -> the rows per CTA that choose_rpc_mux (csrc/conv_mux.cu) picks for 2 strips x 37 rows: 1, 2, 3, 4, 5, 6, 7, 8,
+# 10, 13 and 19 rows, i.e. one to five staging rounds of the five worker groups and a TMEM accumulator ring (10) that wraps
+@pytest.mark.parametrize("max_ctas", [148, 38, 26, 20, 16, 14, 12, 10, 8, 6, 2])
+def test_conv_mux_any_rows_per_cta(max_ctas):
+    """Rows per CTA is a scheduling choice: the mux kernel gives the same result for any of them."""
+    _conv_37x150("mux_f16x2", max_ctas)
+
+
+# CTA budget -> rows per CTA of choose_rpc (csrc/conv_row.cu), the smallest r with 2 * ceil(37 / r) <= budget: 1, 2, 3, 10 and
+# 37 rows; from 7 rows on the 8-stage operand ring wraps, from 9 rows on the 10-accumulator ring as well
+@pytest.mark.parametrize("max_ctas", [148, 38, 26, 8, 2])
+def test_conv_row_any_rows_per_cta(max_ctas):
     """The strip decomposition (rows per CTA) is a scheduling choice: results must not depend on it."""
-    import os, subprocess, sys
-    code = (
-        "import numpy as np, torch\n"
-        "from oracle import ref_numpy as RN\n"
-        "from pbml_mantle_convection_b200 import ops\n"
-        "r=np.random.default_rng(5); x=r.standard_normal((1,16,37,150)); w=r.standard_normal((16,16,3,3))/12; b=r.standard_normal(16)\n"
-        "cu=lambda a: torch.tensor(np.ascontiguousarray(a),dtype=torch.float32,device='cuda:0')\n"
-        "o,_,_=ops.conv_fwd([ops.Source(ops.pack_nchw(cu(x)))],ops.pack_conv_weight(cu(w),[16]),ops.pad_vec(cu(b),16,'cuda:0'),16,3,'replicate',impl='row_f16x2',wpk_row=ops.pack_conv_weight_row(cu(w),[16]))\n"
-        "y=ops.unpack_nchw(o,16).cpu().numpy(); ref=RN.conv2d_same(x,w,b,'replicate')\n"
-        "e=np.linalg.norm(y-ref)/np.linalg.norm(ref); print(e); assert e<3e-6\n")
-    env = dict(os.environ, PBMC_ROW_RPC=str(rpc))
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    res = subprocess.run([sys.executable, "-c", code], cwd=root, env=env, capture_output=True, text=True, timeout=300)
-    assert res.returncode == 0, res.stdout + res.stderr
+    _conv_37x150("row_f16x2", max_ctas)
 
 
 def test_conv_gelu_epilogue():

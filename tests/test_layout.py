@@ -31,3 +31,14 @@ def test_gpu_side_files_do_not_read_reference():
         if f.endswith("make_golden.py") or f.endswith("test_layout.py"):
             continue
         assert ("/root/" + "reference") not in open(f).read(), f
+
+
+def test_library_reads_no_environment_and_keeps_no_launch_switches():
+    """What libpbmc runs is decided by its C-ABI arguments alone, and whether a launch is programmatic-dependent by the
+    arguments of the function that makes it."""
+    csrc = os.path.join(ROOT, "pbml_mantle_convection_b200", "csrc")
+    for f in sorted(os.listdir(csrc)):
+        if f.endswith((".cu", ".cuh", ".h")):
+            src = open(os.path.join(csrc, f)).read()
+            for word in ("getenv", "PBMC_DEV_", "_pdl_next"):
+                assert word not in src, f"{f} contains {word}"

@@ -45,5 +45,5 @@ for _ in range(30):
     b.synchronize()
     ts.append(a.elapsed_time(b) * 1e3)
 ts.sort()
-print(f"conv[1] {H}x{W} {impl} flags={os.environ.get('PBMC_ROW_DBG_FLAGS', '0')}: median {ts[len(ts) // 2]:.1f} us, best {ts[0]:.1f} us "
+print(f"conv[1] {H}x{W} {impl}: median {ts[len(ts) // 2]:.1f} us, best {ts[0]:.1f} us "
       f"({'no flush' if noflush else 'L2 flushed'}{', aliased sources' if alias else ''}, ), checksum {float(o.double().sum()):.6e}", flush=True)

@@ -128,8 +128,7 @@ def main():
     if not torch.cuda.is_available():
         sys.exit("needs a CUDA device: these are device timings")
     name, lim = card()
-    res = {"card": name, "power_limit_and_max_sm_clock": lim, "l2_flushed": False, "steps": a.steps,
-           "chain_pdl_env": os.environ.get("PBMC_CHAIN_PDL")}
+    res = {"card": name, "power_limit_and_max_sm_clock": lim, "l2_flushed": False, "steps": a.steps}
     print(f"card: {name}; power limit, max SM clock: {lim}; L2 not flushed between steps", flush=True)
     net = paper_net()
     H, W = 128, 506
