@@ -44,7 +44,11 @@ typedef enum {
 } pbmc_status;
 
 enum { PBMC_PAD_ZEROS = 0, PBMC_PAD_REPLICATE = 1, PBMC_PAD_REFLECT = 2 };
-enum { PBMC_XFORM_NONE = 0, PBMC_XFORM_GN_GELU = 1, PBMC_XFORM_GN = 2, PBMC_XFORM_GELU = 3 };
+/* PBMC_XFORM_SCALE: the raw source times 2^-s, s per sample from `stats` (sum, sum^2 per block, as a conv epilogue
+ * accumulates them) so that the source's rms lies in [1/2, 1); the conv's epilogue multiplies by 2^s again -- exact, and
+ * the fp16 hi+lo split then sees an order-1 operand whatever the source's magnitude.  Single-source convs on the MUX_*
+ * kernel only (pbmc_conv_fwd refuses it for every other implementation and shape; the pyramid operators refuse it). */
+enum { PBMC_XFORM_NONE = 0, PBMC_XFORM_GN_GELU = 1, PBMC_XFORM_GN = 2, PBMC_XFORM_GELU = 3, PBMC_XFORM_SCALE = 4 };
 enum { PBMC_ACT_NONE = 0, PBMC_ACT_GELU = 1 };
 /* Source layouts.  BLOCKED: float [B][nblk][H][W][4].  STAGED16: the tensor-core operand image of a 16-channel
  * tensor, ready to be copied into shared memory by the TMA engine with no thread touching it:
@@ -68,6 +72,11 @@ enum { PBMC_TRUNK_LOADER_THREADS = 0, PBMC_TRUNK_LOADER_BULK = 1 };
 /* conv implementation selector: FFMA = fp32 CUDA cores; UMMA_* = tcgen05 tensor cores:
  * 3XTF32 / F16X2 split every operand into hi + lo (tf32 resp. fp16) and issue 3 passes --
  * fp32-grade accuracy; BF16 = single pass with bf16 operands (looser, stated bound).
+ * Operand range of the fp16 split: the weights are prescaled per layer (see the operand images below), so any weight
+ * scale is fp32-grade; a source is split as it is read, which covers GroupNorm(+GELU) sources (order 1) and raw sources
+ * with |x| < 2^15 at an absolute error floor of about 2^-25 (fp16's subnormal lo part); PBMC_XFORM_SCALE sources at any
+ * magnitude.  The fused network reads conv[3]'s source, conv[2]'s unnormalised GELU output, as a SCALE source where conv[3]
+ * runs on the mux kernel, and otherwise runs conv[3] on 3XTF32 when AUTO or an F16X2 implementation is asked for.
  * ROW_* = the row-streaming warp-specialised tcgen05 kernel (csrc/conv_row.cu; vertical taps folded
  * into the MMA's N dimension), F16X2 = fp16 hi+lo 3-pass (fp32-grade), BF16 = single bf16 pass.
  * MUX_* = the time-multiplexed row kernel (csrc/conv_mux.cu: the same GEMM, all warps stage rows, then all
@@ -134,7 +143,11 @@ typedef struct {
  * Epilogue: + bias, optional GELU (:1339-1340), raw output, and per-(b, block) sum / sum^2
  * accumulated into out_stats (double, must be zeroed by the caller) for the next GroupNorm,
  * or per-channel sums for the zero-mean at :1343 (out_chan_sum, [B][cout_blks*4] doubles).
- * Packed weights: float [ceil(cout/16)][cin_blks][k*k][4][16]  (see pbmc_pack helpers in Python). */
+ * Packed weights: float [ceil(cout/16)][cin_blks][k*k][4][16]  (see pbmc_pack helpers in Python).
+ * Tensor-core operand images (wpk_umma: tf32 hi|lo, fp16 hi|lo, bf16 images; wpk_row: fp16 hi|lo, bf16 images; layouts
+ * in ops.pack_conv_weight_umma / ops.pack_conv_weight_row) hold the filters times 2^e, one e per layer chosen so that
+ * max|w| * 2^e lies in [2^14, 2^15) (e = 0 for all-zero filters), and end in a 16-byte tail float[4] = {2^-e, 0, 0, 0};
+ * the epilogue computes fmaf(acc, 2^-e, bias).  A power-of-two scale of the weights is therefore exact on every path. */
 typedef struct {
   pbmc_src src[PBMC_MAX_SRC];
   int nsrc;

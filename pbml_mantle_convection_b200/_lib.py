@@ -16,7 +16,7 @@ LIB_PATH = os.path.join(_PKG, "libpbmc.so")
 
 MAX_SRC, MAX_LEVELS, MAX_REPEATS = 8, 8, 8
 PAD = {"zeros": 0, "constant": 0, "replicate": 1, "reflect": 2}
-XFORM_NONE, XFORM_GN_GELU, XFORM_GN, XFORM_GELU = 0, 1, 2, 3
+XFORM_NONE, XFORM_GN_GELU, XFORM_GN, XFORM_GELU, XFORM_SCALE = 0, 1, 2, 3, 4
 LAYOUT_BLOCKED, LAYOUT_STAGED16 = 0, 1
 ACT_NONE, ACT_GELU = 0, 1
 HEAD_CURL, HEAD_MAE = 0, 1

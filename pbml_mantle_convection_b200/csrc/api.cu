@@ -108,7 +108,8 @@ static int validate_conv(const pbmc_conv_desc& d) {
     if (S.nblk <= 0) return PBMC_ERR_BAD_SHAPE;
     if ((S.xform == PBMC_XFORM_GN_GELU || S.xform == PBMC_XFORM_GN) && (!S.stats || !S.gamma || !S.beta))
       return PBMC_ERR_NULL_POINTER;
-    if (S.xform < PBMC_XFORM_NONE || S.xform > PBMC_XFORM_GELU) return PBMC_ERR_UNSUPPORTED;
+    if (S.xform < PBMC_XFORM_NONE || S.xform > PBMC_XFORM_SCALE) return PBMC_ERR_UNSUPPORTED;
+    if (S.xform == PBMC_XFORM_SCALE && !S.stats) return PBMC_ERR_NULL_POINTER;
   }
   return PBMC_OK;
 }
@@ -132,6 +133,11 @@ static int conv_enqueue(const pbmc_conv_desc& d, cudaStream_t st, bool pdl) {
            : (d.wpk_row && conv_row_supported(d))   ? PBMC_CONV_ROW_F16X2
            : (d.wpk_umma && conv_umma_supported(d)) ? PBMC_CONV_UMMA_F16X2
                                                     : PBMC_CONV_FFMA;
+  // a SCALE source is understood by the mux kernel only
+  for (int s = 0; s < d.nsrc; ++s)
+    if (d.src[s].xform == PBMC_XFORM_SCALE &&
+        ((impl != PBMC_CONV_MUX_F16X2 && impl != PBMC_CONV_MUX_BF16) || !d.wpk_row || !conv_mux_supported(d)))
+      return PBMC_ERR_UNSUPPORTED;
   if (impl == PBMC_CONV_MUX_F16X2 || impl == PBMC_CONV_MUX_BF16) {
     if (!d.wpk_row) return PBMC_ERR_UNSUPPORTED;
     if (conv_mux_supported(d)) {
@@ -213,7 +219,7 @@ struct Plan {
   int Hl[PBMC_MAX_LEVELS], Wl[PBMC_MAX_LEVELS];
   size_t inp, x0, pooled[PBMC_MAX_LEVELS], ping[PBMC_MAX_LEVELS][2], up[PBMC_MAX_LEVELS], h1, h2, h3;
   size_t stats, stats_bytes, chan_sum, sync, uvmax, total;  // sync: [L][B] grid-barrier counters of the persistent trunk kernels
-  // stats slots: 0 = conv0, 1 + l*R + r = trunk, 1 + L*R = conv1
+  // stats slots: 0 = conv0, 1 + l*R + r = trunk, 1 + L*R = conv1, 2 + L*R = conv2
   size_t stat_off(int slot, int B) const { return stats + (size_t)slot * B * CB * 2 * sizeof(double); }
 };
 
@@ -253,7 +259,7 @@ int make_plan(const pbmc_net& n, int B, int H, int W, Plan& P) {
   P.h1 = take((size_t)B * P.CB * px * 16);
   P.h2 = take((size_t)B * P.CB * px * 16);
   P.h3 = take((size_t)B * P.COB3 * px * 16);
-  const int nslots = 2 + P.L * P.R;
+  const int nslots = 3 + P.L * P.R;
   const size_t sync_bytes = ((size_t)P.L * B * sizeof(uint32_t) + 7) & ~(size_t)7;
   P.stats_bytes = (size_t)nslots * B * P.CB * 2 * sizeof(double) + (size_t)B * P.COB3 * 4 * sizeof(double) + sync_bytes +
                   (size_t)2 * B * sizeof(uint32_t);
@@ -556,16 +562,33 @@ static int surrogate_enqueue_on(pbmc_ctx* ctx, const pbmc_net& n, const Plan& P,
   d.src[L] = make_src(inp, P.CIB, PBMC_XFORM_NONE, nullptr, nullptr, 0.0);
   RC(conv_enqueue(d, st, true));
   if (learned) RC(ring_enqueue(d, n.wedge_conv1, st));
+  // conv[3] (:1342) with per-channel sums for the zero-mean (:1343).  Its source is conv[2]'s GELU output, which no
+  // GroupNorm brings to order 1: its scale follows conv[2]'s weights, and an fp16 hi|lo split of it loses relative
+  // precision below 2^-3 (subnormal lo part) and overflows above 65504.  Where conv[3] runs on the fp16 mux kernel, conv[2]
+  // also accumulates its sums of squares and conv[3] reads h2 as a SCALE source (times 2^-s per sample, s from h2's rms;
+  // the epilogue multiplies by 2^s: exact).  Elsewhere, when the fp16 split was asked for, conv[3] runs on the 3xTF32
+  // split, which has fp32's exponent range (FFMA where the tensor-core kernel does not take the shape).
+  pbmc_conv_desc d3;
+  fill_conv(d3, n, n.conv3, B, H, W, F(P.h3), nullptr, chan_sum, PBMC_ACT_NONE);
+  d3.nsrc = 1;
+  d3.src[0] = make_src(F(P.h2), CB, PBMC_XFORM_SCALE, S(2 + L * R), nullptr, 0.0);
+  const bool conv3_scaled = !learned && d3.wpk_row && conv_mux_supported(d3) &&
+                            (d3.impl == PBMC_CONV_MUX_F16X2 || (d3.impl == PBMC_CONV_AUTO && conv_mux_one_wave(d3)));
+  if (conv3_scaled) {
+    d3.impl = PBMC_CONV_MUX_F16X2;
+  } else {
+    d3.src[0].xform = PBMC_XFORM_NONE;
+    d3.src[0].stats = nullptr;
+    if (d3.impl == PBMC_CONV_AUTO || d3.impl == PBMC_CONV_UMMA_F16X2 || d3.impl == PBMC_CONV_ROW_F16X2 || d3.impl == PBMC_CONV_MUX_F16X2)
+      d3.impl = (d3.wpk_umma && conv_umma_supported(d3)) ? PBMC_CONV_UMMA_3XTF32 : PBMC_CONV_FFMA;
+  }
   // gn[0] + act folded into conv[2]'s load; conv[2] + act (:1336-1340)
-  fill_conv(d, n, n.conv2, B, H, W, F(P.h2), nullptr, nullptr, PBMC_ACT_GELU);
+  fill_conv(d, n, n.conv2, B, H, W, F(P.h2), conv3_scaled ? S(2 + L * R) : nullptr, nullptr, PBMC_ACT_GELU);
   d.nsrc = 1;
   d.src[0] = make_src(F(P.h1), CB, PBMC_XFORM_GN_GELU, S(1 + L * R), &n.conv1, 1.0 / (4.0 * H * W));
   RC(conv_enqueue(d, st, true));
   if (learned) RC(ring_enqueue(d, n.wedge_conv2, st));
-  // conv[3] (:1342) with per-channel sums for the zero-mean (:1343)
-  fill_conv(d, n, n.conv3, B, H, W, F(P.h3), nullptr, chan_sum, PBMC_ACT_NONE);
-  d.nsrc = 1;
-  d.src[0] = make_src(F(P.h2), CB, PBMC_XFORM_NONE, nullptr, nullptr, 0.0);
+  d = d3;
   RC(conv_enqueue(d, st, true));
   if (learned) RC(ring_enqueue(d, n.wedge_conv3, st));
   return head_enqueue(F(P.h3), chan_sum, members, n.a_bound, n.head_kind, n.p_pred, u, v, p, uvmax, B, H, W, st, true);

@@ -171,6 +171,16 @@ __device__ __forceinline__ void gn_coeffs(const double* stats2, double inv_count
   b = (float)((double)beta - mean * ad);
 }
 
+// PBMC_XFORM_SCALE: 2^-s with 2^(s-1) <= rms < 2^s, rms over all nblk*4 channels of one sample from its (sum, sum^2) per
+// block; 1 for an all-zero source.  A power of two, so scaling the source by it (and the output back) is exact.
+__device__ __forceinline__ float scale_src_factor(const double* st, int nblk, size_t plane_px) {
+  double ss = 0.0;
+  for (int k = 0; k < nblk; ++k) ss += __ldcg(st + 2 * k + 1);
+  int ex = 0;
+  frexp(sqrt(ss / ((double)nblk * 4.0 * (double)plane_px)), &ex);
+  ex = ex < -64 ? -64 : (ex > 64 ? 64 : ex);
+  return ldexpf(1.f, -ex);
+}
 __device__ __forceinline__ float4 xform4(float4 v, const float* a4, const float* b4, int xform) {
   if (xform == PBMC_XFORM_NONE) return v;
   if (xform != PBMC_XFORM_GELU) {

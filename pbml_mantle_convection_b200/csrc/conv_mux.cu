@@ -52,6 +52,7 @@ struct ConvMuxParams {
   int cout_blks, pad_mode, epi_act;
   int rpc;           // output rows per CTA (<= CM_MAXR - 2)
   const void* wpk;   // [dx][part][2 K-chunks][48 rows (dy, c_out)][8 c_in] 16-bit
+  const float* wscale;  // 2^-e: the image holds the filters times 2^e (ops.prescale_pow2)
   const float* bias;
   float* out;
   double* out_stats;
@@ -88,6 +89,7 @@ __global__ void __maxnreg__(CM_MAXNREG) conv_mux_kernel(const __grid_constant__ 
   float* bias_s = reinterpret_cast<float*>(smem + 1792);      // 16 floats (zero padded)
   float* xf_a = reinterpret_cast<float*>(smem + 1856);        // GroupNorm scale / shift of the 16 input channels
   float* xf_b = reinterpret_cast<float*>(smem + 1920);
+  float* wsc_s = reinterpret_cast<float*>(smem + 1984);       // epilogue factor 2^-e (times 2^s for a SCALE source)
   unsigned char* Bs = smem + CM_HDR;
   unsigned char* As = Bs + B_GROUP;
 
@@ -165,8 +167,10 @@ __global__ void __maxnreg__(CM_MAXNREG) conv_mux_kernel(const __grid_constant__ 
   if (tid < 16) {
     float a = 1.f, bb = 0.f;
     if (do_x && tid < nb * 4) gn_coeffs(p.stats + ((size_t)b * p.nblk + (tid >> 2)) * 2, p.inv_count, p.gamma[tid], p.beta[tid], a, bb);
+    if (p.xform == PBMC_XFORM_SCALE) a = scale_src_factor(p.stats + (size_t)b * p.nblk * 2, p.nblk, plane_px);
     xf_a[tid] = a;
     xf_b[tid] = bb;
+    if (tid == 0) *wsc_s = p.xform == PBMC_XFORM_SCALE ? __ldg(p.wscale) / a : __ldg(p.wscale);  // powers of two: exact
   }
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   fence_proxy_async_smem();
@@ -197,6 +201,12 @@ __global__ void __maxnreg__(CM_MAXNREG) conv_mux_kernel(const __grid_constant__ 
       float v[16] = {R.v0.x, R.v0.y, R.v0.z, R.v0.w, R.v1.x, R.v1.y, R.v1.z, R.v1.w,
                      R.v2.x, R.v2.y, R.v2.z, R.v2.w, R.v3.x, R.v3.y, R.v3.z, R.v3.w};
       float hv = R.h;
+      if (p.xform == PBMC_XFORM_SCALE) {  // exact power-of-two scale: out-of-image taps stay zero
+        const float s_a = xf_a[0];
+#pragma unroll
+        for (int e = 0; e < 16; ++e) v[e] *= s_a;
+        hv *= s_a;
+      }
       if (do_x) {
         // GroupNorm + GELU, branch-free: out-of-image taps are masked back to zero afterwards
         const bool keep = R.ok && col_ok;
@@ -274,6 +284,7 @@ __global__ void __maxnreg__(CM_MAXNREG) conv_mux_kernel(const __grid_constant__ 
     const int cout_blks = p.cout_blks;
     const bool epi_gelu = p.epi_act == PBMC_ACT_GELU;
     const uint32_t bias_addr = smem_u32(bias_s);
+    const uint32_t wsc_addr = smem_u32(wsc_s);
     float* const obase = p.out + (((size_t)b * cout_blks) * plane_px + (size_t)y0 * W + gx) * 4;
     const size_t blk_stride = plane_px * 4;
     const bool col_in = gx < W;
@@ -330,13 +341,15 @@ __global__ void __maxnreg__(CM_MAXNREG) conv_mux_kernel(const __grid_constant__ 
                 float4 bq;
                 asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(bq.x), "=f"(bq.y), "=f"(bq.z), "=f"(bq.w) : "r"(bias_addr + qb * 16));
                 const float bias4[4] = {bq.x, bq.y, bq.z, bq.w};
+                float wsc;  // re-read per block: a register held across the loop spills under the register cap
+                asm volatile("ld.shared.f32 %0, [%1];" : "=f"(wsc) : "r"(wsc_addr));
                 float o[4];
 #pragma unroll
                 for (int e = 0; e < 4; ++e) {
                   float a = __uint_as_float(r[0][qh * 4 + e]);
 #pragma unroll
                   for (int dy = 1; dy < KS; ++dy) a += __uint_as_float(r[dy][qh * 4 + e]);
-                  a += bias4[e];
+                  a = fmaf(a, wsc, bias4[e]);
                   if (!LEAN && epi_gelu) a = gelu_erf(a);
                   o[e] = a;
                 }
@@ -495,13 +508,13 @@ bool conv_mux_one_wave(const pbmc_conv_desc& d) {
 bool conv_mux_supported(const pbmc_conv_desc& d) {
   if (d.ksize != 3 || d.cout > 16 || d.nsrc != 1 || d.src[0].layout != PBMC_LAYOUT_BLOCKED) return false;
   if (d.src[0].nblk < 1 || d.src[0].nblk > 4) return false;
-  if (d.src[0].xform != PBMC_XFORM_NONE && d.src[0].xform != PBMC_XFORM_GN_GELU) return false;
+  if (d.src[0].xform != PBMC_XFORM_NONE && d.src[0].xform != PBMC_XFORM_GN_GELU && d.src[0].xform != PBMC_XFORM_SCALE) return false;
   if (d.out_chan_sum != nullptr && d.cout > 4) return false;  // per-channel sums: head conv only
   return true;
 }
 
-// wpk_row holds two operand images back to back (ops.pack_conv_weight_row), one 16-channel group here:
-//   [fp16 hi|lo : 3 * 2 * 1536 B][bf16 : 3 * 1536 B]
+// wpk_row holds two operand images back to back (ops.pack_conv_weight_row), one 16-channel group here, then the prescale tail:
+//   [fp16 hi|lo : 3 * 2 * 1536 B][bf16 : 3 * 1536 B][float 2^-e, 0, 0, 0]
 int conv_mux_dispatch(const pbmc_conv_desc& d, cudaStream_t st, bool pdl) {
   ConvMuxParams p;
   const pbmc_src& S = d.src[0];
@@ -520,6 +533,7 @@ int conv_mux_dispatch(const pbmc_conv_desc& d, cudaStream_t st, bool pdl) {
   if (!base) return PBMC_ERR_NULL_POINTER;
   if (!aligned16(base)) return PBMC_ERR_MISALIGNED;
   const size_t off_bf16 = (size_t)3 * 2 * (2 * CM_N * 16);
+  p.wscale = reinterpret_cast<const float*>(base + off_bf16 + (size_t)3 * (2 * CM_N * 16));
   if (d.impl == PBMC_CONV_MUX_F16X2) {
     p.wpk = base;
     return launch_mux<2>(p, d.max_ctas, st, pdl);

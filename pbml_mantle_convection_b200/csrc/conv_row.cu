@@ -66,6 +66,7 @@ struct ConvRowParams {
   int max_ctas; // CTA budget (0 = whole GPU)
   int has_staged;  // some source is an operand image: the bulk-copy ring is allocated
   const void* wpk;  // [group][dx][part][2 K-chunks][N = k*16 rows (dy, c_out)][8 c_in] 16-bit
+  const float* wscale;  // 2^-e: the image holds the filters times 2^e (ops.prescale_pow2)
   const float* bias;
   float* out;
   double* out_stats;
@@ -269,6 +270,7 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
     const int cout_blks = p.cout_blks;
     const bool epi_gelu = p.epi_act == PBMC_ACT_GELU;
     const uint32_t bias_addr = smem_u32(bias_s);
+    const float wsc = __ldg(p.wscale);
     float* orow = p.out + (((size_t)b * cout_blks) * plane_px + (size_t)(y0 + eset) * W + gx) * 4;
     const size_t blk_stride = plane_px * 4, row_stride = (size_t)EPI_SETS * W * 4;
     const bool col_in = gx < W;
@@ -316,7 +318,7 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
                 float a = __uint_as_float(r[0][qb * 4 + e]);
 #pragma unroll
                 for (int dy = 1; dy < KS; ++dy) a += __uint_as_float(r[dy][qb * 4 + e]);
-                a += bias4[e];
+                a = fmaf(a, wsc, bias4[e]);
                 if (!LEAN && epi_gelu) a = gelu_erf(a);
                 o[e] = a;
               }
@@ -380,7 +382,7 @@ __global__ void __launch_bounds__(CR_THREADS, 1) conv_row_kernel(const __grid_co
                     a += __uint_as_float(ra[dy][qh * 4 + e]);
                     c += __uint_as_float(rb[dy][qh * 4 + e]);
                   }
-                  a = (a + c) + bias4[e];
+                  a = fmaf(a + c, wsc, bias4[e]);
                   if (epi_gelu) a = gelu_erf(a);
                   o[e] = a;
                 }
@@ -1060,8 +1062,8 @@ bool conv_row_supported(const pbmc_conv_desc& d) {
   return smem <= 227 * 1024;
 }
 
-// wpk_row holds two operand images back to back (ops.pack_conv_weight_row):
-//   [fp16 hi|lo : groups * k * 2 * (2*N*16) B][bf16 : groups * k * (2*N*16) B]
+// wpk_row holds two operand images back to back (ops.pack_conv_weight_row), then the prescale tail:
+//   [fp16 hi|lo : groups * k * 2 * (2*N*16) B][bf16 : groups * k * (2*N*16) B][float 2^-e, 0, 0, 0]
 int conv_row_dispatch(const pbmc_conv_desc& d, cudaStream_t st, bool pdl) {
   ConvRowParams p;
   int cin = 0;
@@ -1097,6 +1099,7 @@ int conv_row_dispatch(const pbmc_conv_desc& d, cudaStream_t st, bool pdl) {
   if (!aligned16(base)) return PBMC_ERR_MISALIGNED;
   const size_t n = (size_t)d.ksize * 16;
   const size_t off_bf16 = (size_t)p.ngroups * d.ksize * 2 * (2 * n * 16);
+  p.wscale = reinterpret_cast<const float*>(base + off_bf16 + (size_t)p.ngroups * d.ksize * (2 * n * 16));
   if (d.impl == PBMC_CONV_ROW_F16X2) {
     p.wpk = base;
     return d.ksize == 3 ? launch_row<3, 2>(p, st, pdl) : launch_row<5, 2>(p, st, pdl);

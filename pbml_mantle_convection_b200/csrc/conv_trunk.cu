@@ -49,6 +49,7 @@ struct TrunkLayerDev {
   const float* gamma;    // [16] affine of `in`'s GroupNorm
   const float* beta;
   const void* wpk;       // this layer's filters, row-kernel operand image (one 16-channel group)
+  const float* wscale;   // 2^-e: the image holds the filters times 2^e (ops.prescale_pow2)
   const float* bias;     // [16]
   float* out;            // [B][4][H][W][4] raw output
   double* out_stats;     // [B][4][2], zeroed before the launch
@@ -339,6 +340,7 @@ __global__ void __maxnreg__(CT_SETS <= 5 ? 80 : 72) conv_trunk_kernel(const __gr
 
       float s1[4] = {0.f, 0.f, 0.f, 0.f}, s2[4] = {0.f, 0.f, 0.f, 0.f};
       float* const obase = Ld.out + o_off;
+      const float wsc = __ldg(Ld.wscale);
       // Output row yo reads D_yo .. D_{yo+KS-1} (running indices gb + ...).  Each issuer commits its own rows in order,
       // so the last CT_NMMA of them (one per issuer) cover all KS.
       auto dfull_bar = [&](int r) { return d_full((uint32_t)(gb + r) % ND); };
@@ -396,7 +398,7 @@ __global__ void __maxnreg__(CT_SETS <= 5 ? 80 : 72) conv_trunk_kernel(const __gr
                 float a = __uint_as_float(r[0][qh * 4 + e]);
 #pragma unroll
                 for (int dy = 1; dy < KS; ++dy) a += __uint_as_float(r[dy][qh * 4 + e]);
-                o[e] = a + bias4[e];
+                o[e] = fmaf(a, wsc, bias4[e]);
               }
               *reinterpret_cast<float4*>(orow + qb * blk_stride) = make_float4(o[0], o[1], o[2], o[3]);
               s1[qb] += (o[0] + o[1]) + (o[2] + o[3]);
@@ -568,7 +570,8 @@ static int launch_trunk(ConvTrunkParams& p, cudaStream_t st, bool pdl) {
   return PBMC_OK;
 }
 
-// wpk_row of a layer: [fp16 hi|lo : 3 * 2 * 1536 B][bf16 : 3 * 1536 B] (ops.pack_conv_weight_row, one 16-channel group)
+// wpk_row of a layer: [fp16 hi|lo : 3 * 2 * 1536 B][bf16 : 3 * 1536 B][float 2^-e, 0, 0, 0] (ops.pack_conv_weight_row, one
+// 16-channel group)
 int conv_trunk_dispatch(const pbmc_trunk_desc& t, cudaStream_t st, bool pdl) {
   if (!conv_trunk_supported(t)) return PBMC_ERR_UNSUPPORTED;
   if (!t.src0.ptr || !t.ping[0] || !t.ping[1] || !t.stats || !t.sync) return PBMC_ERR_NULL_POINTER;
@@ -595,6 +598,7 @@ int conv_trunk_dispatch(const pbmc_trunk_desc& t, cudaStream_t st, bool pdl) {
       Ld.in = t.ping[(r - 1) & 1]; Ld.stats = t.stats + (size_t)(r - 1) * t.B * 8; Ld.gamma = Lp.gamma; Ld.beta = Lp.beta;
     }
     Ld.wpk = reinterpret_cast<const char*>(Lh.wpk_row) + (bf16 ? off_bf16 : 0);
+    Ld.wscale = reinterpret_cast<const float*>(reinterpret_cast<const char*>(Lh.wpk_row) + off_bf16 + (size_t)3 * (2 * CT_N * 16));
     Ld.bias = Lh.bias;
     Ld.out = t.ping[r & 1];
     Ld.out_stats = t.stats + (size_t)r * t.B * 8;

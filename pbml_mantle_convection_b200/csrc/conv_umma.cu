@@ -51,6 +51,7 @@ struct ConvUmmaParams {
   int nsrc, B, H, W;
   int cout_blks, cin_blks, pad_mode, epi_act;
   const void* wpk;  // [parts][cin chunks][taps][16 c_out][16 B of c_in]
+  const float* wscale;  // 2^-e: the image holds the filters times 2^e (ops.prescale_pow2)
   const float* bias;
   float* out;
   double* out_stats;
@@ -245,6 +246,7 @@ __global__ void __launch_bounds__(CU_THREADS, (MODE == CU_TF32X3 ? 1 : (NMT <= 4
 #pragma unroll
   for (int c = 0; c < 16; ++c) cs[c] = 0.f;
   float bias[16];
+  const float wsc = __ldg(p.wscale);
 #pragma unroll
   for (int q = 0; q < 4; ++q) {
     float4 bq = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -261,8 +263,8 @@ __global__ void __launch_bounds__(CU_THREADS, (MODE == CU_TF32X3 ? 1 : (NMT <= 4
 #pragma unroll
       for (int qb = 0; qb < 4; ++qb) {
         if (qb < p.cout_blks) {
-          float4 o = make_float4(v[qb * 4 + 0] + bias[qb * 4 + 0], v[qb * 4 + 1] + bias[qb * 4 + 1],
-                                 v[qb * 4 + 2] + bias[qb * 4 + 2], v[qb * 4 + 3] + bias[qb * 4 + 3]);
+          float4 o = make_float4(fmaf(v[qb * 4 + 0], wsc, bias[qb * 4 + 0]), fmaf(v[qb * 4 + 1], wsc, bias[qb * 4 + 1]),
+                                 fmaf(v[qb * 4 + 2], wsc, bias[qb * 4 + 2]), fmaf(v[qb * 4 + 3], wsc, bias[qb * 4 + 3]));
           if (p.epi_act == PBMC_ACT_GELU) {
             o.x = gelu_erf(o.x); o.y = gelu_erf(o.y); o.z = gelu_erf(o.z); o.w = gelu_erf(o.w);
           }
@@ -346,12 +348,13 @@ int conv_umma_dispatch(const pbmc_conv_desc& d, cudaStream_t st) {
   p.cin_blks = cin;
   p.pad_mode = d.pad_mode; p.epi_act = d.epi_act;
   p.bias = d.bias; p.out = d.out; p.out_stats = d.out_stats; p.out_chan_sum = d.out_chan_sum;
-  // wpk_umma holds three operand images back to back (see ops.pack_conv_weight_umma):
-  //   [tf32 hi|lo : 2*cin*taps*256 B][fp16 hi|lo : cin/2*taps*512 B][bf16 : cin/2*taps*256 B]
+  // wpk_umma holds three operand images back to back (see ops.pack_conv_weight_umma), then the prescale tail:
+  //   [tf32 hi|lo : 2*cin*taps*256 B][fp16 hi|lo : cin/2*taps*512 B][bf16 : cin/2*taps*256 B][float 2^-e, 0, 0, 0]
   const size_t taps = (size_t)d.ksize * d.ksize;
   const char* base = reinterpret_cast<const char*>(d.wpk_umma);
   if (!aligned16(base)) return PBMC_ERR_MISALIGNED;
   const size_t off_f16 = 2 * (size_t)cin * taps * 256, off_bf16 = off_f16 + (size_t)(cin / 2) * taps * 512;
+  p.wscale = reinterpret_cast<const float*>(base + off_bf16 + (size_t)(cin / 2) * taps * 256);
   if (d.impl == PBMC_CONV_UMMA_3XTF32) {
     p.wpk = base;
     return d.ksize == 3 ? launch_umma<3, 64, 15, 8, CU_TF32X3>(p, st) : launch_umma<5, 64, 15, 8, CU_TF32X3>(p, st);

@@ -276,6 +276,7 @@ extern "C" int pbmc_finalize_nchw(const pbmc_src* S, float* dst, int B, int C, i
   if (!S || !S->ptr || !dst) return PBMC_ERR_NULL_POINTER;
   if (S->layout != PBMC_LAYOUT_BLOCKED) return PBMC_ERR_UNSUPPORTED;
   if ((S->xform == PBMC_XFORM_GN_GELU || S->xform == PBMC_XFORM_GN) && (!S->stats || !S->gamma || !S->beta)) return PBMC_ERR_NULL_POINTER;
+  if (S->xform < PBMC_XFORM_NONE || S->xform > PBMC_XFORM_GELU) return PBMC_ERR_UNSUPPORTED;
   if (B <= 0 || C <= 0 || H <= 0 || W <= 0 || S->nblk != (C + 3) / 4) return PBMC_ERR_BAD_SHAPE;
   if (!aligned16(S->ptr)) return PBMC_ERR_MISALIGNED;
   const size_t plane = (size_t)H * W;
@@ -309,6 +310,7 @@ extern "C" int pbmc_avgpool2(const pbmc_src* S, float* dst, int B, int H, int W,
   if (!S || !S->ptr || !dst) return PBMC_ERR_NULL_POINTER;
   if (S->layout != PBMC_LAYOUT_BLOCKED) return PBMC_ERR_UNSUPPORTED;
   if ((S->xform == PBMC_XFORM_GN_GELU || S->xform == PBMC_XFORM_GN) && (!S->stats || !S->gamma || !S->beta)) return PBMC_ERR_NULL_POINTER;
+  if (S->xform < PBMC_XFORM_NONE || S->xform > PBMC_XFORM_GELU) return PBMC_ERR_UNSUPPORTED;
   const int Ho = H / 2, Wo = W / 2;
   if (B <= 0 || Ho <= 0 || Wo <= 0 || S->nblk <= 0) return PBMC_ERR_BAD_SHAPE;
   if (!aligned16(S->ptr) || !aligned16(dst)) return PBMC_ERR_MISALIGNED;
@@ -321,6 +323,7 @@ extern "C" int pbmc_avgpool2(const pbmc_src* S, float* dst, int B, int H, int W,
 static int bicubic_launch(const pbmc_src* S, void* dst, int B, int Hs, int Ws, int H, int W, bool staged, void* stream) {
   if (!S || !S->ptr || !dst) return PBMC_ERR_NULL_POINTER;
   if ((S->xform == PBMC_XFORM_GN_GELU || S->xform == PBMC_XFORM_GN) && (!S->stats || !S->gamma || !S->beta)) return PBMC_ERR_NULL_POINTER;
+  if (S->xform < PBMC_XFORM_NONE || S->xform > PBMC_XFORM_GELU) return PBMC_ERR_UNSUPPORTED;
   if (B <= 0 || Hs <= 0 || Ws <= 0 || H < Hs || W < Ws || S->nblk <= 0) return PBMC_ERR_BAD_SHAPE;  // up-sampling only
   if (S->layout != PBMC_LAYOUT_BLOCKED) return PBMC_ERR_UNSUPPORTED;
   if (staged && S->nblk != 4) return PBMC_ERR_UNSUPPORTED;  // the staged image is one 16-channel K group

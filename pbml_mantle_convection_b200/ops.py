@@ -63,6 +63,22 @@ def tf32_round(x: torch.Tensor) -> torch.Tensor:
     return ((bits + 0x1000) & -8192).view(torch.float32)
 
 
+def pow2(e: torch.Tensor) -> torch.Tensor:
+    """2^e as float32, built from the exponent bits (exact; e integer in [-126, 127])."""
+    return ((e.to(torch.int32).reshape(1) + 127) << 23).view(torch.float32)
+
+
+def prescale_pow2(w: torch.Tensor):
+    """Tensor-core weight images hold w * 2^e, one e per layer, so that max|w| * 2^e lies in [2^14, 2^15): the fp16 hi part
+    then uses fp16's whole range and the lo part stays normal for weights down to 2^-18 of the largest, whatever the
+    layer's own scale (all-zero weights: e = 0).  Returns (w * 2^e, the image's 16-byte tail = float32 [2^-e, 0, 0, 0]),
+    which the kernels' epilogues apply as fmaf(acc, 2^-e, bias).  Computed on w's device without a host sync."""
+    mant, ex = torch.frexp(w.abs().amax())
+    e = torch.where(mant > 0, 15 - ex, torch.zeros_like(ex)).clamp(-126, 126)
+    tail = torch.cat([pow2(-e), w.new_zeros(3)])
+    return w * pow2(e), tail
+
+
 def umma_supported(cout: int, src_channels) -> bool:
     """Shapes the tcgen05 conv kernel takes (csrc/conv_umma.cu): <= 16 outputs, every source an even number of 4-channel blocks."""
     return cout <= 16 and all(nblk(c) % 2 == 0 for c in src_channels)
@@ -73,7 +89,8 @@ def pack_conv_weight_umma(w_full: torch.Tensor, src_channels) -> torch.Tensor:
          tf32 : float32  [2 (hi, lo)][cin_blks  ][k*k][16 c_out][4 c_in]   hi = tf32(w),  lo = w - hi
          fp16 : float16  [2 (hi, lo)][cin_blks/2][k*k][16 c_out][8 c_in]   hi = fp16(w),  lo = fp16(w - hi)
          bf16 : bfloat16 [1         ][cin_blks/2][k*k][16 c_out][8 c_in]
-       back to back (offsets are multiples of 256 B)."""
+         tail : float32  [4] = [2^-e, 0, 0, 0]
+       back to back (offsets are multiples of 16 B); w here is the layer's filters times 2^e (prescale_pow2)."""
     Co, Ci, k, _ = w_full.shape
     assert Co <= 16 and sum(src_channels) == Ci
     parts, c0 = [], 0
@@ -84,7 +101,7 @@ def pack_conv_weight_umma(w_full: torch.Tensor, src_channels) -> torch.Tensor:
             wpart = torch.cat([wpart, wpart.new_zeros(Co, pad, k, k)], 1)
         parts.append(wpart)
         c0 += c
-    w = torch.cat(parts, 1).float()
+    w, tail = prescale_pow2(torch.cat(parts, 1).float())
     if Co < 16:
         w = torch.cat([w, w.new_zeros(16 - Co, w.shape[1], k, k)], 0)
     cb = w.shape[1] // 4
@@ -97,7 +114,7 @@ def pack_conv_weight_umma(w_full: torch.Tensor, src_channels) -> torch.Tensor:
     img_f16 = torch.stack([h16, (w8 - h16.float()).half()], 0).contiguous()
     img_bf16 = w8.bfloat16().contiguous()
     as_bytes = lambda t: t.view(torch.uint8).reshape(-1)
-    return torch.cat([as_bytes(img_tf32), as_bytes(img_f16), as_bytes(img_bf16)]).contiguous()
+    return torch.cat([as_bytes(img_tf32), as_bytes(img_f16), as_bytes(img_bf16), as_bytes(tail)]).contiguous()
 
 
 def row_supported(cout: int, ksize: int, src_channels) -> bool:
@@ -116,8 +133,10 @@ def pack_conv_weight_row(w_full: torch.Tensor, src_channels) -> torch.Tensor:
     """[Co<=16, Ci, k, k] -> uint8 buffer with the two K-major B-operand images of csrc/conv_row.cu:
          fp16 : [group][dx][2 (hi, lo)][2 K-chunks][N = k*16 rows (dy, c_out)][8 c_in]   hi = fp16(w), lo = fp16(w - hi)
          bf16 : [group][dx][1         ][2 K-chunks][N rows][8 c_in]
-       back to back.  A group is 16 input channels of ONE source (each source is zero-padded to a
-       multiple of 16 channels), in concat order; the vertical tap dy rides in the MMA's N dimension."""
+         tail : float32 [4] = [2^-e, 0, 0, 0]
+       back to back, w here being the layer's filters times 2^e (prescale_pow2).  A group is 16 input channels of ONE
+       source (each source is zero-padded to a multiple of 16 channels), in concat order; the vertical tap dy rides in the
+       MMA's N dimension."""
     Co, Ci, k, _ = w_full.shape
     assert Co <= 16 and sum(src_channels) == Ci
     parts, c0 = [], 0
@@ -128,7 +147,7 @@ def pack_conv_weight_row(w_full: torch.Tensor, src_channels) -> torch.Tensor:
             wpart = torch.cat([wpart, wpart.new_zeros(Co, pad, k, k)], 1)
         parts.append(wpart)
         c0 += c
-    w = torch.cat(parts, 1).float()
+    w, tail = prescale_pow2(torch.cat(parts, 1).float())
     if Co < 16:
         w = torch.cat([w, w.new_zeros(16 - Co, w.shape[1], k, k)], 0)
     G = w.shape[1] // 16
@@ -138,7 +157,7 @@ def pack_conv_weight_row(w_full: torch.Tensor, src_channels) -> torch.Tensor:
     img_f16 = torch.stack([h16, (w6 - h16.float()).half()], 2).contiguous()  # (g, dx, part, chunk, dy, co, e)
     img_bf16 = w6.bfloat16().contiguous()
     as_bytes = lambda t: t.view(torch.uint8).reshape(-1)
-    return torch.cat([as_bytes(img_f16), as_bytes(img_bf16)]).contiguous()
+    return torch.cat([as_bytes(img_f16), as_bytes(img_bf16), as_bytes(tail)]).contiguous()
 
 
 def pad_vec(v, c: int, device, fill=0.0) -> torch.Tensor:

@@ -68,7 +68,9 @@ def conv_module_forward(m: nn.Conv2d, x: torch.Tensor) -> torch.Tensor:
     """Stand-alone forward of an nn.Conv2d-shaped module on an NCHW tensor through libpbmc.
     Images of at least TENSOR_CORE_MIN_SIDE rows and columns with c_in, c_out <= 16 go to the tensor-core kernels (fp16 hi+lo, fp32-grade; the library
     picks the time-multiplexed or the row-streaming one), thin strips (the edge regions of the learned-boundary conv,
-    reference :1022-1065) and wide outputs to the FFMA kernel."""
+    reference :1022-1065) and wide outputs to the FFMA kernel.
+    The input may have any magnitude: it is scaled by 2^-s with 2^(s-1) <= max|x| < 2^s (the bias with it) and the output
+    by 2^s, exact in float32, so the kernels' fp16 split always sees |x| < 1.  s is computed on the device (no sync)."""
     _check_conv_supported(m)
     if not x.is_cuda:
         raise L.PbmcError("this layer has no CPU implementation; move the module and input to a CUDA device")
@@ -82,11 +84,13 @@ def conv_module_forward(m: nn.Conv2d, x: torch.Tensor) -> torch.Tensor:
     # k=5, 7->16 at k=3; wider inputs stay on the FFMA kernel here, the fused network path feeds conv[1] itself)
     tensor_core = m.out_channels <= 16 and m.in_channels <= 16 and min(x.shape[-2:]) >= TENSOR_CORE_MIN_SIDE
     wpk, wrow, bias = _packed_filters(m, x.device, tensor_core)
-    xb = ops.pack_nchw(x)
+    mant, s = torch.frexp(x.abs().amax().float())
+    s = torch.where(mant > 0, s, torch.zeros_like(s)).clamp(-126, 126)
+    xb = ops.pack_nchw(x * ops.pow2(-s).to(x.dtype))
     mode = m.padding_mode if pad != (0, 0) else "zeros"
-    yb, _, _ = ops.conv_fwd([ops.Source(xb)], wpk, bias, m.out_channels, k, mode, impl="auto" if tensor_core else "ffma",
-                            wpk_row=wrow)
-    y = ops.unpack_nchw(yb, m.out_channels)
+    yb, _, _ = ops.conv_fwd([ops.Source(xb)], wpk, bias * ops.pow2(-s), m.out_channels, k, mode,
+                            impl="auto" if tensor_core else "ffma", wpk_row=wrow)
+    y = ops.unpack_nchw(yb, m.out_channels) * ops.pow2(s)
     # 'same' geometry is computed; smaller paddings are a crop of it (exact for zeros / valid)
     cy, cx = k // 2 - pad[0], k // 2 - pad[1]
     if cy < 0 or cx < 0 or ((cy or cx) and mode != "zeros"):
