@@ -221,10 +221,11 @@ class _FluidNetBase(nn.Module):
             else:
                 self.conv.append(BoundaryLearnedConvolution2D(c_h, co, k=f, use_symm=use_symm))
         self._engines = {}
+        self._fused_ok = {}
         self.conv_impl = "auto"  # "auto" | "ffma" | "umma_3xtf32" | "umma_bf16"
         self.trunk_mode = "auto"  # "auto": one persistent launch per pyramid level where it fits | "per_layer"
         self.up_staged = False    # True: conv[1] stages the up-sampled levels with TMA bulk copies (see include/pbmc.h)
-        self.use_cuda_graph = True  # learned-boundary networks: replay the module-level forward as one CUDA graph
+        self.use_cuda_graph = True  # learned-boundary networks: replay the whole forward as one CUDA graph
 
     # nn.Module bookkeeping: engines hold device buffers, never parameters
     def _engine(self, device) -> SurrogateEngine:
@@ -237,6 +238,17 @@ class _FluidNetBase(nn.Module):
         if eng.trunk_mode != self.trunk_mode or eng.up_staged != bool(self.up_staged):
             eng.set_trunk_mode(self.trunk_mode, self.up_staged)
         return eng
+
+    def _fused_supported(self, device, B, H, W):
+        """Whether the fused engine takes a call of this size on `device`.  It runs on CUDA devices only; the shape part is
+        engine.fused_supported, remembered per (B, H, W): the query builds a descriptor and calls into the library, and the
+        network's shape does not change after construction."""
+        if device.type != "cuda":
+            return False
+        ok = self._fused_ok.get((B, H, W))
+        if ok is None:
+            ok = self._fused_ok[(B, H, W)] = fused_supported(self, B, H, W)
+        return ok
 
     def __getstate__(self):  # engines are not picklable / deep-copyable
         d = dict(self.__dict__)
@@ -264,10 +276,15 @@ class NewFluidNet(_FluidNetBase):
         self._check_fused(inputs)
         if self.r_p == "learned":
             return _forward_learned_replayed(self, inputs, head_bc=1, wall_bcs=True)
-        eng = self._engine(inputs.device)
-        eng.net_module = self
-        u, v, p, _ = eng.forward_blocked(ops.pack_nchw(inputs))
-        return _shape_outputs(self, u, v, p, inputs.dtype)
+        return _forward_engine(self, inputs)
+
+
+def _forward_engine(net, inputs):
+    """The fused engine's forward of a NewFluidNet (pbmc_surrogate_forward: the DAG that TS and EnsembleRollout run)."""
+    eng = net._engine(inputs.device)
+    eng.net_module = net
+    u, v, p, _ = eng.forward_blocked(ops.pack_nchw(inputs))
+    return _shape_outputs(net, u, v, p, inputs.dtype)
 
 
 def _shape_outputs(net, u, v, p, dtype):
@@ -299,16 +316,17 @@ class _LearnedPlan:
 
 
 def _forward_learned_replayed(net, inputs, head_bc, wall_bcs):
-    """The module-level forward of a learned-boundary network is ~1000 small launches (9 region convs + stitching per
-    layer): 26 ms of host time per call for the paper's network at 128x506 whatever the kernels do.  From the third
-    call with the same input shape, dtype and parameter versions the whole forward is replayed as ONE CUDA graph
-    (call 1 runs eagerly and fills the packed-filter caches, call 2 captures); the result is what the eager path
-    returns, bit for bit.  Any parameter update (in place or by re-assignment) starts over.  If capture is impossible
-    the eager path stays in use -- the same kernels, launched one by one."""
+    """A learned-boundary forward is many small launches (two per layer on the engine, which also forks and joins the
+    pyramid levels' streams; more per layer in the module-level composition), so its host time can exceed its device
+    time.  From the third call with the same input shape, dtype, parameter versions and kernel choices the whole forward
+    is replayed as ONE CUDA graph (call 1 runs eagerly and fills the packed-filter caches and the workspace, call 2
+    captures); the result is what the eager path returns, bit for bit.  Any parameter update (in place or by
+    re-assignment) or a change of `conv_impl` starts over.  If capture is impossible the eager path stays in use -- the
+    same kernels, launched one by one."""
     if not net.use_cuda_graph or torch.cuda.is_current_stream_capturing():
         return _forward_learned(net, inputs, head_bc, wall_bcs)
     key = (tuple(inputs.shape), inputs.dtype, str(inputs.device), head_bc, wall_bcs, net.training,
-           tuple((q.data_ptr(), q._version) for q in net.parameters()))
+           (net.conv_impl, net.trunk_mode, bool(net.up_staged)), tuple((q.data_ptr(), q._version) for q in net.parameters()))
     pl = net.__dict__.get("_learned_plan")
     if pl is None or pl.key != key:
         pl = _LearnedPlan()
@@ -334,61 +352,21 @@ def _forward_learned_replayed(net, inputs, head_bc, wall_bcs):
     return tuple(None if o is None else o.clone() for o in pl.out)  # callers own what they get
 
 
-def _learned_blocked_ok(net, H, W, head_bc, wall_bcs):
-    """The all-blocked kernel path of a learned-boundary NewFluidNet: every layer's 9-region conv as two launches."""
-    if head_bc != 1 or not wall_bcs or net.c_h % 4 or net.c_h > 16 or net.c_o > 4:
-        return False
-    h, w = H, W
-    for l in range(net.levels):
-        if not net.convs[l][0].layers[0].kernel_path_ok(h, w, [net.c_h]):
-            return False
-        h, w = h // 2, w // 2
-    return net.conv[1].kernel_path_ok(H, W, [net.c_h] * net.levels + [net.c_i])
-
-
-def _forward_learned_blocked(net, inputs):
-    """NewFluidNet with learned boundaries (reference :1315-1388 with BoundaryLearnedConvolution2D layers, SURVEY.md 8f N1):
-    activations stay in the blocked layout from the first conv to the head; every FluidLayer is TWO launches (interior
-    conv with the producer's GroupNorm + GELU fused into its load and the statistics in its epilogue, then the ring
-    kernel); pooling is incremental, the up-sampled levels and the raw input are conv[1]'s source list (never
-    concatenated); zero-mean + curl + wall BCs are the head kernel."""
-    B, _, H, W = inputs.shape
-    dev, c_h, c_i = inputs.device, net.c_h, net.c_i
-    gnp = lambda gn, c: (ops.pad_vec(gn.weight, c, dev, 1.0), ops.pad_vec(gn.bias, c, dev))
-
-    def fluid(fl, sources, chans):
-        yb, st, _ = fl.layers[0].forward_blocked(sources, chans)
-        g, b_ = gnp(fl.layers[1], c_h)
-        return ops.Source(yb, L.XFORM_GN_GELU, st, g, b_)
-
-    inp_b = ops.pack_nchw(inputs)
-    x_in = fluid(net.conv[0], [ops.Source(inp_b)], [c_i])
-    srcs, level_in = [], x_in
-    for l in range(net.levels):
-        if l > 0:
-            level_in = ops.Source(ops.avgpool2(level_in))  # pool^l(x_in), incrementally (identical composition, :1321-1322)
-        y1 = level_in
-        for r in range(net.repeats):
-            y1 = fluid(net.convs[l][r], [y1], [c_h])
-        srcs.append(y1 if l == 0 else ops.Source(ops.bicubic_up(y1, H, W)))
-    srcs.append(ops.Source(inp_b))
-    y1b, st1, _ = net.conv[1].forward_blocked(srcs, [c_h] * net.levels + [c_i])
-    g0, b0 = gnp(net.gn[0], c_h)
-    y2b, _, _ = net.conv[2].forward_blocked([ops.Source(y1b, L.XFORM_GN_GELU, st1, g0, b0)], [c_h], epi_act=L.ACT_GELU,
-                                            want_stats=False)
-    y3b, _, csum = net.conv[3].forward_blocked([ops.Source(y2b)], [c_h], want_stats=False, want_chan_sum=True)
-    u, v, p, _ = ops.head(y3b, csum, None, net.a_bound, L.HEAD_CURL if net.loss_type == "curl" else L.HEAD_MAE, net.p_pred,
-                          want_uvmax=False)
-    return _shape_outputs(net, u, v, p, inputs.dtype)
-
-
 def _forward_learned(net, inputs, head_bc, wall_bcs):
-    """Learned-boundary networks (SURVEY.md section 8f N1).  NewFluidNet on grids every level of which holds the
-    reference's boundary strips runs all-blocked (two launches per layer, `_forward_learned_blocked`); FluidNet (head
-    conv enlarged by bc_x = bc_y = 2) and degenerate sizes run layer by layer through the module-level forwards."""
+    """Learned-boundary networks (SURVEY.md section 8f N1).  A NewFluidNet at a shape the fused engine takes runs there,
+    on the DAG that TS and EnsembleRollout run; FluidNet (head conv enlarged by bc_x = bc_y = 2) and the shapes the engine
+    refuses run through `_forward_learned_modules`."""
     B, _, H, W = inputs.shape
-    if _learned_blocked_ok(net, H, W, head_bc, wall_bcs):
-        return _forward_learned_blocked(net, inputs)
+    if head_bc == 1 and wall_bcs and net._fused_supported(inputs.device, B, H, W):
+        return _forward_engine(net, inputs)
+    return _forward_learned_modules(net, inputs, head_bc, wall_bcs)
+
+
+def _forward_learned_modules(net, inputs, head_bc, wall_bcs):
+    """The learned-boundary forward composed layer by layer from the module-level forwards (reference :1315-1388):
+    pyramid, concatenation, head conv enlarged by `head_bc`, then the curl head with wall BCs (NewFluidNet) or plain
+    central differences of the enlarged stream function (FluidNet, `wall_bcs=False`)."""
+    B, _, H, W = inputs.shape
     dev = inputs.device
     x_in = net.conv[0](inputs)
     feats = []
@@ -744,7 +722,7 @@ class TS(nn.Module):
         advect = self.ad is not None and self.net == "newfluidnet"
         # learned-boundary nets: where the engine's ring kernel takes every level (else the per-step path below)
         fused = (isinstance(stokes, NewFluidNet) and grid.separable
-                 and (stokes.r_p != "learned" or fused_supported(stokes, B, H, W)))
+                 and (stokes.r_p != "learned" or stokes._fused_supported(dev, B, H, W)))
         cn_max = self.ad.CN_max if advect else 0.0
         n = self.ts
         if fused and advect:

@@ -393,11 +393,18 @@ def test_learned_network_with_scaled_weights(k):
                         use_symm=False, a_bound=spec.a_bound, repeats=spec.repeats, f=spec.f, p_pred=spec.p_pred).double()
     net.load_state_dict({n: torch.tensor(v) for n, v in sd.items()})
     net = net.to(DEV).eval()
-    u, v, _, _ = net._engine(torch.device(DEV)).forward_blocked(ops.pack_nchw(torch.tensor(inp, device=DEV)))
+    x = torch.tensor(inp, device=DEV)
+    u, v, _, _ = net._engine(torch.device(DEV)).forward_blocked(ops.pack_nchw(x))
     errs = {"u": relerr(u.cpu().numpy(), u64), "v": relerr(v.cpu().numpy(), v64)}
     print(f"[learned_k5 2^{k}] fused engine rel-L2 {errs}; reference fp32 noise {noise}")
     for n in errs:
         assert errs[n] <= field_bound(noise[n]), (n, errs[n], noise[n])
+    for call in range(3):  # the module call: eager, capture + replay, replay
+        u, v, _ = net(x)
+        errs = {"u": relerr(u.cpu().numpy(), u64), "v": relerr(v.cpu().numpy(), v64)}
+        print(f"[learned_k5 2^{k}] net(x) call {call} rel-L2 {errs}")
+        for n in errs:
+            assert errs[n] <= field_bound(noise[n]), (call, n, errs[n], noise[n])
 
 
 def test_ts_rollout_with_scaled_weights():

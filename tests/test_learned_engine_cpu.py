@@ -121,3 +121,67 @@ def test_python_support_query_and_slab_refusal(lib):
     assert not engine.fused_supported(net, 1, 64, 506)
     with pytest.raises(NotImplementedError, match="learned"):
         SlabSurrogate(net, 128, 506, None, None, (1.0, 1.0, 1.0), None, "cpu")
+
+
+def test_learned_forward_dispatch(lib, monkeypatch):
+    """A learned NewFluidNet's forward runs on the fused engine wherever the engine plans its shape; the shapes it refuses
+    and FluidNet (whose enlarged head has no engine form) take the module-level composition.  The engine is stubbed (its
+    context needs a GPU); the support query is the library's, asked once per (B, H, W)."""
+    import torch
+
+    import pbml_mantle_convection_b200 as P
+    from pbml_mantle_convection_b200 import engine, ops
+    from pbml_mantle_convection_b200 import pytorch_networks_convae as M
+    from tests._util import load_learned_case
+
+    reached, queries = [], []
+
+    class StubEngine:
+        def forward_blocked(self, inp):
+            reached.append("engine")
+            B, _, H, W, _ = inp.shape
+            return torch.zeros(B, H, W), torch.zeros(B, H, W), None, None
+
+    monkeypatch.setattr(torch.Tensor, "is_cuda", property(lambda self: True))
+    cpu_device = torch.Tensor.device
+    monkeypatch.setattr(torch.Tensor, "device", property(lambda self: torch.device("cuda:0")))
+    monkeypatch.setattr(ops, "pack_nchw", lambda x: x[..., None])
+    monkeypatch.setattr(M, "_forward_learned_modules",
+                        lambda net, x, head_bc, wall_bcs: reached.append(("modules", head_bc, wall_bcs)))
+    monkeypatch.setattr(M, "fused_supported", lambda m, B, H, W: queries.append((B, H, W)) or engine.fused_supported(m, B, H, W))
+
+    def mk(spec, cls=P.NewFluidNet):
+        net = cls(spec.levels, spec.c_i, spec.c_h, spec.c_o, "cpu", act_fn="gelu", r_p="learned", loss_type="curl",
+                  use_symm=False, a_bound=spec.a_bound, repeats=spec.repeats, f=spec.f, p_pred=spec.p_pred).eval()
+        monkeypatch.setattr(net, "_engine", lambda dev: StubEngine())
+        net.use_cuda_graph = False
+        return net
+
+    def route(net, B, H, W):
+        reached.clear()
+        net(torch.zeros(B, net.c_i, H, W))
+        assert len(reached) == 1
+        return reached[0]
+
+    from oracle import ref_numpy as RN
+
+    paper = mk(RN.NetSpec(levels=5, c_i=7, c_h=16, c_o=1, r_p="learned", loss_type="curl", use_symm=False, a_bound=10.0,
+                          repeats=6, f=5, p_pred=False))
+    assert route(paper, 1, 128, 506) == "engine" and route(paper, 1, 128, 506) == "engine"
+    assert queries == [(1, 128, 506)]
+    assert route(paper, 2, 128, 506) == "engine" and queries == [(1, 128, 506), (2, 128, 506)]
+    assert route(paper, 1, 64, 506) == ("modules", 1, True)  # coarsest level shorter than the k = 5 strip
+    with monkeypatch.context() as mp:  # the engine runs on CUDA devices only
+        mp.setattr(torch.Tensor, "device", cpu_device)
+        assert route(paper, 1, 128, 506) == ("modules", 1, True)
+
+    k5 = mk(load_learned_case("learned_k5")[0])  # 3 levels, k = 5
+    assert route(k5, 2, 40, 56) == "engine"
+    assert route(k5, 1, 20, 28) == ("modules", 1, True)  # coarsest level 5 x 7: shorter than the 6-row strip
+    wide = mk(RN.NetSpec(levels=2, c_i=7, c_h=32, c_o=1, r_p="learned", loss_type="curl", use_symm=False, a_bound=10.0,
+                         repeats=1, f=5, p_pred=False))
+    assert route(wide, 1, 40, 56) == ("modules", 1, True)  # one ring-kernel tile holds 16 output channels
+
+    fluid = mk(load_learned_case("learned_fluidnet")[0], P.FluidNet)
+    assert engine.fused_supported(fluid, 2, 36, 44)  # the engine would plan the shape ...
+    assert route(fluid, 2, 36, 44) == ("modules", 2, False)  # ... but FluidNet's head is enlarged

@@ -1,7 +1,7 @@
 """Time step of the paper's learned-boundary network (SURVEY.md section 8f N1: NewFluidNet(levels=5, r_p="learned",
 repeats=6, f=5, c_o=1, p_pred=False), 2.13 M parameters) on the fused device-resident rollout, against the per-step
-composition TS.forward used for it before (input build, module-level forward replayed as a CUDA graph, uvmax reduction,
-stencil -- each issued from Python), plus the ring kernel (pbmc_conv_edge9) alone.
+composition TS.forward used for it before (input build, `net(x)` replayed as a CUDA graph, uvmax reduction, stencil --
+each issued from Python), plus the ring kernel (pbmc_conv_edge9) alone.
 
 All times are CUDA-event times over many back-to-back steps after a warm-up.  The L2 is NOT flushed between steps: a
 rollout runs its steps back to back, and one step's working set (under 60 MB at 128 x 506, B = 1) stays in the 126 MB
@@ -88,8 +88,9 @@ def ts_ms_per_step(net, H, W, steps):
 
 
 def per_step_composition_ms(net, H, W, steps):
-    """What TS.forward ran per step for a learned net before: build_input -> net(...) (module-level forward, CUDA-graph
-    replay) -> un-scale -> uvmax -> advect_diffuse, every call issued from Python."""
+    """What TS.forward ran per step for a learned net before the fused rollout (and still runs on non-separable grids,
+    there with the general stencil): build_input -> net(...) (the fused engine's forward, CUDA-graph replay) -> un-scale
+    -> uvmax -> advect_diffuse, every call issued from Python."""
     xc, yc = synthetic_grid(H, W)
     grid = engine.Grid(torch.tensor(xc), torch.tensor(yc), torch.tensor(yc), DEV)
     members = ops.make_members([PARAMS], DEV)
