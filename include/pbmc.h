@@ -465,6 +465,57 @@ int pbmc_rollout_queued(pbmc_ctx* ctx, const pbmc_net* net_h, pbmc_member* membe
                         pbmc_member_clock* clock, double* meanT_seq, float* snap_ring, double* snap_meta, int snap_slots,
                         const pbmc_member_queue* queue_h, void* stream);
 
+/* ------------------------------------------------------------------ per-step wall heat flux, rms velocity, steady stop
+ * Computed by the same apply / commit launches behind every step, for every member that takes the step (float64, sums in
+ * a fixed order: per-CTA partials in apply, a fixed-order sum in commit, so a replay gives the same bits):
+ *   q_bot = -(Tm(1) - Tm(0)) / (y[1] - y[0]),  q_top = -(Tm(H-1) - Tm(H-2)) / (y[H-1] - y[H-2])
+ *     Tm(i) = plain mean over the W columns of row i of the step's new T (pbmc_diagnostics' prof), y = the row
+ *     coordinates with the walls forced to 0 and 1 (ADNet, pytorch_networks_convae.py:532-545): the negated end values
+ *     of the notebook's dTm/dy (load_advection_results :322-323); positive = heat flowing upward
+ *   vrms  = sqrt(mean over the interior cells (rows 1..H-2, cols 1..W-2) of u^2 + v^2), u, v = the step's un-scaled
+ *     velocities (those the stencil advanced T with and the snapshot ring stores)
+ * Steady criterion (window = 0: off).  A member is steady after step s when it has taken at least `window` steps since
+ * it entered its slot (or since the clock was started) and, for each of its series meanT, q_top and vrms, the last
+ * `window` logged values are finite and satisfy (mx - mn) <= rtol * max(|mx|, |mn|) (mx, mn: their max and min; one
+ * rounded subtraction, one rounded multiplication, so a host replay on the logged doubles decides the same bit for bit).
+ * Stop rule: a member found steady after step s takes step s + 1 and then stops (in a sweep its slot is refilled by the
+ * queue's rank rule at that step, in the same launches).  A member that reaches t_end or max_steps at step s + 1 or
+ * earlier stops as without the criterion and is not reported steady.
+ *   flux_seq   [dt_seq_rows][B][2] = (q_bot, q_top), vrms_seq [dt_seq_rows][B]: indexed like dt_seq; rows of frozen
+ *              members are written as 0
+ *   inv_dy_bot = 1 / (y[1] - y[0]), inv_dy_top = 1 / (y[H-1] - y[H-2])
+ *   hist       [B][window][3] ring of the last (meanT, q_top, vrms) of each slot, hist_n [B] values pushed since the
+ *              slot's member started (NULL allowed when window = 0); the caller zeroes hist_n when it starts a clock
+ *   steady     [B]: PBMC_STEADY_* of the slot's member (the caller zeroes it when it starts a clock; a refill resets it)
+ *   part       [B][5][PBMC_CLOCK_PARTS] doubles: device scratch of the per-CTA partial sums */
+#define PBMC_STEADY_MAX_WINDOW 1024
+enum { PBMC_STEADY_NONE = 0, PBMC_STEADY_FOUND = 1, PBMC_STEADY_STOPPED = 2 };
+typedef struct {
+  double* flux_seq;
+  double* vrms_seq;
+  double inv_dy_bot, inv_dy_top;
+  int window;
+  int reserved;
+  double rtol;
+  double* hist;
+  int64_t* hist_n;
+  int* steady;
+  double* part;
+} pbmc_diag_desc;
+
+/* pbmc_rollout_queued (queue_h may be NULL: pbmc_rollout_clocked) plus the per-step diagnostics and the steady stop of
+ * diag_h (host struct of device pointers).  Same launches, none added.  Refused before any CUDA call: what
+ * pbmc_rollout_clocked / pbmc_rollout_queued refuse, a NULL diag_h or NULL array in it (PBMC_ERR_NULL_POINTER; hist and
+ * hist_n may be NULL when window = 0), window < 0 or > PBMC_STEADY_MAX_WINDOW, rtol negative or not finite
+ * (PBMC_ERR_BAD_SHAPE), H < 3 or W < 3 (PBMC_ERR_BAD_SHAPE: no interior). */
+int pbmc_rollout_diagnosed(pbmc_ctx* ctx, const pbmc_net* net_h, pbmc_member* members, const float* xc, const float* yc,
+                           const float* ycc, const float* xcoef, const float* ycoef, double dx_min, double cn_max,
+                           int per_member_dt, float* T_seq, int nslots, int first_step, int n_steps, double* dt_seq,
+                           int dt_seq_rows, float* u, float* v, float* p, float* V, void* workspace, size_t workspace_bytes,
+                           int B, int H, int W, pbmc_member_clock* clock, double* meanT_seq, float* snap_ring,
+                           double* snap_meta, int snap_slots, const pbmc_member_queue* queue_h,
+                           const pbmc_diag_desc* diag_h, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -94,7 +94,17 @@ class MemberQueue(C.Structure):
                 ("member_seq", C.c_void_p), ("snap_member", C.c_void_p), ("Q", C.c_int64)]
 
 
-_STRUCTS = {"pbmc_member_queue": MemberQueue, "pbmc_member_clock": MemberClock, "pbmc_edge9_desc": Edge9Desc, "pbmc_trunk_desc": TrunkDesc, "pbmc_slab_sync": SlabSync, "pbmc_member": Member, "pbmc_src": Src, "pbmc_conv_desc": ConvDesc, "pbmc_layer": Layer, "pbmc_net": Net}
+STEADY_MAX_WINDOW = 1024
+STEADY_NONE, STEADY_FOUND, STEADY_STOPPED = 0, 1, 2
+
+
+class DiagDesc(C.Structure):
+    _fields_ = [("flux_seq", C.c_void_p), ("vrms_seq", C.c_void_p), ("inv_dy_bot", C.c_double), ("inv_dy_top", C.c_double),
+                ("window", C.c_int), ("reserved", C.c_int), ("rtol", C.c_double), ("hist", C.c_void_p), ("hist_n", C.c_void_p),
+                ("steady", C.c_void_p), ("part", C.c_void_p)]
+
+
+_STRUCTS = {"pbmc_diag_desc": DiagDesc, "pbmc_member_queue": MemberQueue, "pbmc_member_clock": MemberClock, "pbmc_edge9_desc": Edge9Desc, "pbmc_trunk_desc": TrunkDesc, "pbmc_slab_sync": SlabSync, "pbmc_member": Member, "pbmc_src": Src, "pbmc_conv_desc": ConvDesc, "pbmc_layer": Layer, "pbmc_net": Net}
 
 # name -> (restype, argtypes); every symbol declared in include/pbmc.h
 _vp, _i, _d, _f, _sz = C.c_void_p, C.c_int, C.c_double, C.c_float, C.c_size_t
@@ -139,6 +149,9 @@ SIGNATURES = {
                                   _vp, _vp, _vp, _vp, _sz, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _vp]),
     "pbmc_rollout_queued": (_i, [_vp, C.POINTER(Net), _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _vp, _i, _i, _i, _vp, _i, _vp,
                                  _vp, _vp, _vp, _vp, _sz, _i, _i, _i, _vp, _vp, _vp, _vp, _i, C.POINTER(MemberQueue), _vp]),
+    "pbmc_rollout_diagnosed": (_i, [_vp, C.POINTER(Net), _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _vp, _i, _i, _i, _vp, _i,
+                                    _vp, _vp, _vp, _vp, _vp, _sz, _i, _i, _i, _vp, _vp, _vp, _vp, _i, C.POINTER(MemberQueue),
+                                    C.POINTER(DiagDesc), _vp]),
 }
 
 _lib = None

@@ -11,6 +11,13 @@ afterwards (`.ipynb_checkpoints/load_advection_results-checkpoint.ipynb:243-326`
     T_vec_<mode>.pkl       mean temperature after every step (first entry: initial mean)     (:547, :647)
     TS_vec_<mode>.pkl      wall-clock seconds of every step                                  (:650-652)
 
+and, with `attempt_ensemble(..., diagnostics=True)` / `attempt_sweep(..., diagnostics=True)` (or `steady=(window,
+rtol)`), the per-step quantities of the converged-state analysis, computed on the device:
+
+    Nu_vec_<mode>.pkl      wall heat fluxes np.array([q_bot, q_top]) after every step (include/pbmc.h, pbmc_diag_desc)
+    vrms_vec_<mode>.pkl    rms velocity of every step (float)
+                           both one entry per step, aligned with t_vec[1:] (no initial entry: vrms needs a step)
+
 with the same cadence rules: a snapshot whenever `t > save_t` (then `save_t = t + save_every`), the pickles rewritten
 whenever `t > write_t` and once more at the end (`:654-677`).
 
@@ -61,6 +68,14 @@ def write_logs(out_dir, mode, snapshots, TS_vec, t_vec, T_vec):
     """The four pickles of `advect_wi_gaia.py:659-677`, same names, same objects."""
     os.makedirs(out_dir, exist_ok=True)
     for name, obj in (("snapshots_", snapshots[mode]), ("TS_vec_", TS_vec[mode]), ("t_vec_", t_vec[mode]), ("T_vec_", T_vec[mode])):
+        with open(os.path.join(out_dir, name + mode + ".pkl"), "wb") as fh:
+            pickle.dump(obj, fh)
+
+
+def write_diag_logs(out_dir, mode, Nu_vec, vrms_vec):
+    """The two diagnostics pickles next to write_logs' four: Nu_vec_<mode>.pkl, vrms_vec_<mode>.pkl."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, obj in (("Nu_vec_", Nu_vec), ("vrms_vec_", vrms_vec)):
         with open(os.path.join(out_dir, name + mode + ".pkl"), "wb") as fh:
             pickle.dump(obj, fh)
 
@@ -175,7 +190,7 @@ def attempt_resident(ens, xcc, ycc, t_end, out_dir, save_every=0.0, write_every=
 
 
 def attempt_ensemble(ens, xcc, ycc, t_end, out_dir, save_every=0.0, write_every=0.0, mode="ML", t=0.0, n_step=0,
-                     check_every=10, max_steps=None):
+                     check_every=10, max_steps=None, diagnostics=False, steady=None):
     """`attempt` for every member of a device-resident `EnsembleRollout` at once.  Member m runs `while t < t_end[m]` (and
     n_step < max_steps) on its own device-side clock; t_end, save_every, t and n_step are scalars or one value per member.
     Writes the reference's four pickles of member m into `out_dir/member_<m>/` with `attempt`'s cadence: the initial entry
@@ -183,7 +198,8 @@ def attempt_ensemble(ens, xcc, ycc, t_end, out_dir, save_every=0.0, write_every=
     `check_every` steps run as one CUDA-graph replay each, then the block's logs are drained; `t > write_t` is evaluated at
     block ends (it decides when intermediate pickles are written, not their final content).  A TS_vec entry is the block's
     wall time over the steps the member took in it.  Returns (t [B], n_step [B], [logs of member m]) with logs as in
-    `attempt`."""
+    `attempt`.  diagnostics=True (or steady=(window, rtol), which also stops a member at a statistical steady state:
+    `EnsembleRollout.start_clock`) adds Nu_vec_<mode>.pkl and vrms_vec_<mode>.pkl next to the four pickles."""
     B, H, W = ens.B, ens.H, ens.W
     n = H * W
     k = int(check_every)
@@ -192,17 +208,18 @@ def attempt_ensemble(ens, xcc, ycc, t_end, out_dir, save_every=0.0, write_every=
     T0 = ens.T.double().cpu().numpy().reshape(B, n)
     t0 = np.broadcast_to(np.asarray(t, dtype=np.float64), (B,)).copy()
     _initial_entries(logs, T0, t0, xcc, ycc, mode, n)
-    ens.start_clock(t_end, save_every=save_every, t0=t0, max_steps=max_steps, n_step=n_step, snap_slots=k)
-    return _run_blocks(ens, k, logs, dirs, t0, n_step, write_every, mode, n)
+    ens.start_clock(t_end, save_every=save_every, t0=t0, max_steps=max_steps, n_step=n_step, snap_slots=k,
+                    **_diag_kwargs(diagnostics, steady))
+    return _run_blocks(ens, k, logs, dirs, t0, n_step, write_every, mode, n, _diag_logs(B, diagnostics, steady))
 
 
 def attempt_sweep(ens, T0, params, xcc, ycc, t_end, out_dir, save_every=0.0, write_every=0.0, mode="ML", t=0.0, n_step=0,
-                  check_every=10, max_steps=None):
+                  check_every=10, max_steps=None, diagnostics=False, steady=None):
     """`attempt` for each of Q members run through the B slots of a device-resident `EnsembleRollout`
     (`EnsembleRollout.start_sweep`; Q may be larger or smaller than B).  T0: [Q, H, W]; params: Q tuples (RaQ, gamma,
     beta); t_end, save_every, t, n_step, max_steps: scalars or one value per member.  Member q's pickles go to
     `out_dir/member_<q>/`, with `attempt_ensemble`'s cadence and content: the slot a member ran in, and when, make no
-    difference.  Returns (t [Q], n_step [Q], [logs of member q])."""
+    difference.  Returns (t [Q], n_step [Q], [logs of member q]).  diagnostics / steady: as in `attempt_ensemble`."""
     Q, H, W = len(params), ens.H, ens.W
     n = H * W
     k = int(check_every)
@@ -211,8 +228,18 @@ def attempt_sweep(ens, T0, params, xcc, ycc, t_end, out_dir, save_every=0.0, wri
     T0 = torch.as_tensor(T0).to("cpu", torch.float32).reshape(Q, H, W)  # what the device runs from
     _initial_entries(logs, T0.double().numpy().reshape(Q, n), t, xcc, ycc, mode, n)
     ens.start_sweep(T0, params, t_end, save_every=save_every, t0=t, max_steps=max_steps, n_step=n_step, snap_slots=k,
-                    steps_per_graph=k)
-    return _run_blocks(ens, k, logs, dirs, t, n_step, write_every, mode, n)
+                    steps_per_graph=k, **_diag_kwargs(diagnostics, steady))
+    return _run_blocks(ens, k, logs, dirs, t, n_step, write_every, mode, n, _diag_logs(Q, diagnostics, steady))
+
+
+def _diag_kwargs(diagnostics, steady):
+    """start_clock / start_sweep's diagnostics arguments (none when off, so the call is the one without them)."""
+    return {"diagnostics": True, "steady": steady} if diagnostics or steady is not None else {}
+
+
+def _diag_logs(N, diagnostics, steady):
+    """Per member (Nu_vec, vrms_vec) lists, or None without diagnostics."""
+    return [([], []) for _ in range(N)] if diagnostics or steady is not None else None
 
 
 def _initial_entries(logs, T0, t, xcc, ycc, mode, n):
@@ -225,11 +252,18 @@ def _initial_entries(logs, T0, t, xcc, ycc, mode, n):
         snapshots[mode]["xcc"], snapshots[mode]["ycc"] = xcc, ycc
 
 
-def _run_blocks(ens, k, logs, dirs, t, n_step, write_every, mode, n):
+def _run_blocks(ens, k, logs, dirs, t, n_step, write_every, mode, n, diag=None):
     """Blocks of k steps (one graph replay each) until no member of the running clock or sweep is left; each drained
     block (a list over the members, or a sweep's dict keyed by member) goes into the logs of its members.  A
     TS_vec entry is the block's wall time over the steps the member took in it; `t > write_t` is evaluated at block
-    ends.  Writes every member's pickles at the end; returns (t, n_step, logs) per member."""
+    ends.  Writes every member's pickles at the end; returns (t, n_step, logs) per member.  diag: per member
+    (Nu_vec, vrms_vec) lists filled from the blocks' q_bot, q_top, vrms and written with the other pickles."""
+
+    def write(m):
+        write_logs(dirs[m], mode, *logs[m])
+        if diag is not None:
+            write_diag_logs(dirs[m], mode, *diag[m])
+
     N = len(logs)
     t_now = np.broadcast_to(np.asarray(t, dtype=np.float64), (N,)).copy()
     n_now = np.broadcast_to(np.asarray(n_step, dtype=np.int64), (N,)).copy()
@@ -253,12 +287,17 @@ def _run_blocks(ens, k, logs, dirs, t, n_step, write_every, mode, n):
                                            np.zeros((n, 1))), axis=1),
                       "P": sn["p"].astype(np.float64).reshape(n) if sn["p"] is not None else np.zeros(n)}
                 _snapshot(snapshots[mode], st)
+            if diag is not None:
+                Nu_vec, vrms_vec = diag[m]
+                for qb, qt, vr in zip(d["q_bot"], d["q_top"], d["vrms"]):
+                    Nu_vec.append(np.array([qb, qt]))
+                    vrms_vec.append(float(vr))
             if taken:
                 t_now[m], n_now[m] = d["t"][-1], d["steps"][-1]
             if taken and t_now[m] > write_t[m]:
                 write_t[m] = t_now[m] + write_every[m]
-                write_logs(dirs[m], mode, *logs[m])
+                write(m)
     for m in range(N):
-        write_logs(dirs[m], mode, *logs[m])
+        write(m)
     ens.stop_clock()
     return t_now, n_now, logs

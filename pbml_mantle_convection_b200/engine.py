@@ -228,10 +228,11 @@ class SurrogateEngine:
                                                 L.stream_ptr(dev)), "pbmc_surrogate_forward")
         return u, v, p, uvmax
 
-    def rollout(self, state, first_step, n_steps, clock=None, queue=None):
+    def rollout(self, state, first_step, n_steps, clock=None, queue=None, diag=None):
         """Enqueue n_steps time steps on `state` (a RolloutState).  No host sync.  clock: a rollout.MemberClocks (the
         per-member run-to-time clock, pbmc_rollout_clocked) or None (pbmc_rollout); queue (with a clock only): a
-        rollout.SweepQueue whose members refill the slots that stop (pbmc_rollout_queued)."""
+        rollout.SweepQueue whose members refill the slots that stop (pbmc_rollout_queued); diag (with a clock only): a
+        rollout.MemberDiagnostics, per-step wall fluxes / rms velocity and the steady stop (pbmc_rollout_diagnosed)."""
         self.refresh()
         s = state
         ws = self.workspace(s.B, s.H, s.W)
@@ -240,15 +241,19 @@ class SurrogateEngine:
                 int(first_step), int(n_steps), L.ptr(s.dt_seq), int(s.dt_seq.shape[0]), L.ptr(s.u), L.ptr(s.v), L.ptr(s.p),
                 L.ptr(s.V), L.ptr(ws), ws.numel(), s.B, s.H, s.W)
         if clock is None:
+            if diag is not None:
+                raise ValueError("diagnostics need a clock")
             L.check(L.load().pbmc_rollout(*args, L.stream_ptr(self.device)), "pbmc_rollout")
+            return
+        clk = (L.ptr(clock.clock), L.ptr(clock.meanT_seq), L.ptr(clock.ring), L.ptr(clock.meta), int(clock.slots))
+        if diag is not None:
+            L.check(L.load().pbmc_rollout_diagnosed(*args, *clk, C.byref(queue.desc) if queue is not None else None,
+                                                    C.byref(diag.desc), L.stream_ptr(self.device)), "pbmc_rollout_diagnosed")
         elif queue is not None:
-            L.check(L.load().pbmc_rollout_queued(*args, L.ptr(clock.clock), L.ptr(clock.meanT_seq), L.ptr(clock.ring),
-                                                 L.ptr(clock.meta), int(clock.slots), C.byref(queue.desc),
-                                                 L.stream_ptr(self.device)), "pbmc_rollout_queued")
+            L.check(L.load().pbmc_rollout_queued(*args, *clk, C.byref(queue.desc), L.stream_ptr(self.device)),
+                    "pbmc_rollout_queued")
         else:
-            L.check(L.load().pbmc_rollout_clocked(*args, L.ptr(clock.clock), L.ptr(clock.meanT_seq), L.ptr(clock.ring),
-                                                  L.ptr(clock.meta), int(clock.slots), L.stream_ptr(self.device)),
-                    "pbmc_rollout_clocked")
+            L.check(L.load().pbmc_rollout_clocked(*args, *clk, L.stream_ptr(self.device)), "pbmc_rollout_clocked")
 
 
 class Grid:

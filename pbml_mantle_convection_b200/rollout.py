@@ -14,10 +14,16 @@ once stopped it is frozen (T bit-identical, dt rows 0) while the others go on.  
 Sweeps larger than the batch (`start_sweep`): Q members run through the B slots; when a slot's member stops, the device
 puts the next queued member into it inside the same graph (pbmc_rollout_queued), so no slot idles while the queue holds
 members.
+
+Per-step diagnostics and the steady stop (`start_clock(..., diagnostics=True)` or `steady=(window, rtol)`, the same for
+`start_sweep`): the same launches also log the wall heat fluxes q_bot / q_top and the rms velocity of every step
+(pbmc_rollout_diagnosed; include/pbmc.h defines them), and with `steady` a member stops one step after its meanT, q_top
+and vrms have each varied by at most rtol (relative) over the last `window` steps.
 """
 from __future__ import annotations
 
 import ctypes as C
+import math
 
 import numpy as np
 import torch
@@ -99,6 +105,50 @@ class SweepQueue:
                 d.member_seq, d.snap_member, d.Q)
 
 
+class MemberDiagnostics:
+    """Device buffers of the per-step diagnostics and the steady criterion (pbmc_diag_desc): flux_seq [rows, B, 2] =
+    (q_bot, q_top) and vrms_seq [rows, B], indexed like dt_seq; each slot's history ring of (meanT, q_top, vrms) with its
+    count, the PBMC_STEADY_* state per slot and the partials scratch.  window = 0: diagnostics only.  `desc` is the C
+    struct."""
+
+    def __init__(self, B, rows, window, rtol, grid, device):
+        f64 = lambda *n: torch.zeros(n, dtype=torch.float64, device=device)
+        self.window, self.rtol = int(window), float(rtol)
+        self.flux_seq, self.vrms_seq = f64(rows, B, 2), f64(rows, B)
+        self.hist = f64(B, self.window, 3) if self.window else None
+        self.hist_n = torch.zeros(B, dtype=torch.int64, device=device)
+        self.steady = torch.zeros(B, dtype=torch.int32, device=device)
+        self.part = f64(B, 5, L.CLOCK_PARTS)
+        y = grid.y1d64  # row coordinates, walls forced to 0 and 1
+        d = self.desc = L.DiagDesc()
+        d.inv_dy_bot, d.inv_dy_top = 1.0 / float(y[1] - y[0]), 1.0 / float(y[-1] - y[-2])
+        d.window, d.rtol = self.window, self.rtol
+        for name in ("flux_seq", "vrms_seq", "hist", "hist_n", "steady", "part"):
+            setattr(d, name, L.ptr(getattr(self, name)))
+
+    def reset(self):
+        """A clock starts: no history, nobody steady."""
+        self.hist_n.zero_()
+        self.steady.zero_()
+
+    def key(self):
+        d = self.desc
+        return ("diag", d.flux_seq, d.vrms_seq, d.hist, d.hist_n, d.steady, d.part, self.window, self.rtol)
+
+
+def _steady_args(diagnostics, steady):
+    """(window, rtol) of start_clock / start_sweep's arguments, None without diagnostics."""
+    if steady is None:
+        return (0, 0.0) if diagnostics else None
+    window, rtol = steady
+    if isinstance(window, bool) or int(window) != window or not 1 <= int(window) <= L.STEADY_MAX_WINDOW:
+        raise ValueError(f"steady window must be an integer in [1, {L.STEADY_MAX_WINDOW}], got {window!r}")
+    rtol = float(rtol)
+    if not (math.isfinite(rtol) and rtol >= 0.0):
+        raise ValueError(f"steady rtol must be finite and >= 0, got {rtol!r}")
+    return int(window), rtol
+
+
 class EnsembleRollout:
     """B members on one GPU.  `params`: list of (RaQ, gamma=fkt, beta=fkp), one per member."""
 
@@ -125,6 +175,8 @@ class EnsembleRollout:
         self._pending = None  # (first dt_seq row, steps) of the block not drained yet
         self._queue = None    # SweepQueue of the last sweep (its buffers, and so its graphs, serve the next one of that shape)
         self._sweep = None    # host bookkeeping while a sweep runs (start_sweep)
+        self._diag = None     # MemberDiagnostics while a clock runs with diagnostics
+        self._diags = {}      # (window, rtol) -> MemberDiagnostics: buffers, and so graphs, kept for the next clock
 
     # ------------------------------------------------------------------ state
     def set_T(self, T0):
@@ -149,7 +201,7 @@ class EnsembleRollout:
             first = 1 + (self.n_done % 2)
             k = min(n - done, self.max_steps)
             self._begin_block(first - 1, k)
-            self.engine.rollout(self.state, first, k, clock=self._clk, queue=self._run_queue())
+            self.engine.rollout(self.state, first, k, clock=self._clk, queue=self._run_queue(), diag=self._diag)
             self.time += self.state.dt_seq[first - 1:first - 1 + k].sum(0)
             self.n_done += k
             done += k
@@ -164,23 +216,26 @@ class EnsembleRollout:
         par = self.n_done % 2
         # the graph bakes in packed-weight and workspace addresses and the conv implementation: key on them too
         key = (k, par) + self.engine.graph_key(self.B, self.H, self.W)
-        clk, qu = self._clk, self._run_queue()
+        clk, qu, dg = self._clk, self._run_queue(), self._diag
         if clk is not None:
             key = key + clk.key()  # a clocked graph: its own entry (t_end, save_every live in device memory)
         if qu is not None:
             key = key + qu.key()  # a sweep's graph: refills only rewrite device memory
+        if dg is not None:
+            key = key + dg.key()  # window and rtol are launch arguments
         if key not in self._graphs:
             # eager warm-up (module load + func attributes outside capture) on saved state: what a step may rewrite
             saved = [self.state.T_seq] + ([clk.clock] if clk is not None else []) + \
-                    ([self.members, qu.next, qu.slot_member] if qu is not None else [])
+                    ([self.members, qu.next, qu.slot_member] if qu is not None else []) + \
+                    ([t for t in (dg.hist, dg.hist_n, dg.steady) if t is not None] if dg is not None else [])
             copies = [t.clone() for t in saved]
-            self.engine.rollout(self.state, 1 + par, 1, clock=clk, queue=qu)
+            self.engine.rollout(self.state, 1 + par, 1, clock=clk, queue=qu, diag=dg)
             for t, c in zip(saved, copies):
                 t.copy_(c)
             torch.cuda.synchronize(self.device)
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
-                self.engine.rollout(self.state, 1 + par, k, clock=clk, queue=qu)
+                self.engine.rollout(self.state, 1 + par, k, clock=clk, queue=qu, diag=dg)
             self._graphs[key] = g
         return self._graphs[key]
 
@@ -226,16 +281,22 @@ class EnsembleRollout:
     def _per_member(self, x, dtype=np.float64):
         return np.broadcast_to(np.asarray(x, dtype=dtype), (self.B,)).copy()
 
-    def start_clock(self, t_end, save_every=0.0, t0=None, max_steps=None, n_step=0, snap_slots=None, steps_per_graph=10):
+    def start_clock(self, t_end, save_every=0.0, t0=None, max_steps=None, n_step=0, snap_slots=None, steps_per_graph=10,
+                    diagnostics=False, steady=None):
         """Give every member a clock (each argument a scalar or one value per member): the following steps run member m
         `while t[m] < t_end[m] and steps[m] < max_steps[m]` (advect_wi_gaia.py:583), log mean-T after every step and take a
         snapshot (T, u, v, p) whenever t > save_t (save_t = 0 at the start, then t + save_every).
           t0         start time (default: `self.time`; given, it also becomes `self.time`)
           n_step     step count at the start (the reference's n_step), max_steps an absolute limit on it (None: none)
           snap_slots snapshot-ring slots per member (default steps_per_graph: a ring drained once per block never fills)
+          diagnostics  also log the wall heat fluxes q_bot, q_top and the rms velocity of every step (drain())
+          steady     (window, rtol), 1 <= window <= 1024, rtol finite >= 0: diagnostics, and a member stops one step after
+                     the last `window` values of each of its meanT, q_top and vrms satisfy max - min <= rtol * max(|max|,
+                     |min|) (include/pbmc.h, pbmc_diag_desc); a member stopped so is reported `steady`
         Then alternate `run(k, steps_per_graph=k)` (or `step(n)`) and `drain()` until `any_active()` is False.
         The clock's device buffers (and so its captured graphs) outlive stop_clock(): the next start_clock() or
         start_sweep() with the same ring size reuses them, re-initialised, and captures nothing new."""
+        dg = self._new_diag(diagnostics, steady)
         clk = self._new_clock(snap_slots, steps_per_graph)
         if t0 is None:
             t0 = self.time.cpu().numpy()
@@ -251,7 +312,7 @@ class EnsembleRollout:
         c.view(torch.int32)[:, _ACTIVE] = torch.from_numpy(active.astype(np.int32))
         clk.clock.copy_(c)
         self.time.copy_(torch.from_numpy(t0))
-        self._clk = clk
+        self._clk, self._diag = clk, dg
         self._pending = None
         self._sweep = None
         self._host_t, self._host_steps, self._host_active = t0, steps0, active
@@ -272,8 +333,19 @@ class EnsembleRollout:
             self._clocks = clk
         return clk
 
+    def _new_diag(self, diagnostics, steady):
+        """The MemberDiagnostics of start_clock / start_sweep's arguments (None: none), reset; cached per (window, rtol)."""
+        wr = _steady_args(diagnostics, steady)
+        if wr is None:
+            return None
+        dg = self._diags.get(wr)
+        if dg is None:
+            dg = self._diags[wr] = MemberDiagnostics(self.B, self.state.dt_seq.shape[0], wr[0], wr[1], self.grid, self.device)
+        dg.reset()
+        return dg
+
     def start_sweep(self, T0, params, t_end, save_every=0.0, t0=0.0, max_steps=None, n_step=0, snap_slots=None,
-                    steps_per_graph=10):
+                    steps_per_graph=10, diagnostics=False, steady=None):
         """Run Q members (`params`: Q tuples (RaQ, gamma, beta); T0: [Q, H, W]) through this ensemble's B slots, each
         `while t < t_end and steps < max_steps` on its own clock as in start_clock (t_end, save_every, t0, max_steps,
         n_step: scalars or one value per member).  When a slot's member stops, the device puts the next queued member
@@ -283,7 +355,9 @@ class EnsembleRollout:
         and with fewer queued members than slots the other slots stay frozen.  Then alternate `run(k, steps_per_graph=k)` and `drain()` until `any_active()` is False.
         The slots' T and member rows are rewritten by the sweep (`members` holds the last members afterwards), and
         `time` keeps summing each slot's dt rows: per-member times come from drain().  A second sweep with the same
-        number of queued members and ring size reuses the buffers and the captured graphs."""
+        number of queued members and ring size reuses the buffers and the captured graphs.
+        diagnostics / steady: as in start_clock; a slot's history and steady state start afresh with each member."""
+        dg = self._new_diag(diagnostics, steady)
         Qa = len(params)
         T0 = torch.as_tensor(T0).to(torch.float32).reshape(Qa, self.H, self.W)
         bc = lambda x, dt=np.float64: np.broadcast_to(np.asarray(x, dtype=dt), (Qa,)).copy()
@@ -322,15 +396,16 @@ class EnsembleRollout:
         c.view(torch.int32)[:, _ACTIVE] = torch.from_numpy(active.astype(np.int32))
         clk.clock.copy_(c)
         self.time.copy_(c[:, _T])
-        self._clk = clk
+        self._clk, self._diag = clk, dg
         self._pending = None
-        self._sweep = {"index": index, "Q": Q, "next": n0, "t": t0, "steps": steps0}
+        self._sweep = {"index": index, "Q": Q, "next": n0, "t": t0, "steps": steps0, "t_end": t_end, "max_steps": max_steps}
         self._host_active = active
 
     def stop_clock(self):
         """Back to unclocked stepping.  Also ends a sweep.  The clock's buffers and graphs stay cached for the next
         start_clock() / start_sweep() with the same ring size."""
         self._clk = None
+        self._diag = None
         self._pending = None
         self._sweep = None
 
@@ -340,10 +415,12 @@ class EnsembleRollout:
 
     def set_t_end(self, t_end):
         """New end time(s) between blocks: written to the device clock, no re-capture.  A stopped member whose t is now
-        below its t_end takes steps again."""
+        below its t_end takes steps again, unless the steady criterion stopped it."""
         self._require_clock(sweep=False)
         self._t_end = self._per_member(t_end)
         self._host_active = (self._host_t < self._t_end) & (self._host_steps < self._max_steps)
+        if self._diag is not None:
+            self._host_active &= self._diag.steady.cpu().numpy() != L.STEADY_STOPPED
         self._clk.clock[:, _T_END].copy_(torch.from_numpy(self._t_end))
         self._clk.clock.view(torch.int32)[:, _ACTIVE].copy_(torch.from_numpy(self._host_active.astype(np.int32)))
 
@@ -362,13 +439,15 @@ class EnsembleRollout:
     def read_clock(self):
         """The device clocks as numpy arrays: t, t_end, save_t, steps, snaps, drained, active, overflow (synchronises).
         In a sweep (one clock per slot) also slot_member (the member in each slot, -1: none) and next (queued members
-        placed so far)."""
+        placed so far).  With diagnostics also steady (the slot's member was stopped by the steady criterion)."""
         self._require_clock()
         c = self._clk.clock[:, :_HDR].cpu()
         ci, ci32 = c.view(torch.int64), c.view(torch.int32)
         out = {"t": c[:, _T].numpy(), "t_end": c[:, _T_END].numpy(), "save_t": c[:, _SAVE_T].numpy(),
                "steps": ci[:, _STEPS].numpy(), "snaps": ci[:, _SNAPS].numpy(), "drained": ci[:, _DRAINED].numpy(),
                "active": ci32[:, _ACTIVE].numpy() != 0, "overflow": ci32[:, _OVERFLOW].numpy() != 0}
+        if self._diag is not None:
+            out["steady"] = self._diag.steady.cpu().numpy() == L.STEADY_STOPPED
         if self._sweep is not None:
             qu = self._run_queue()
             out["slot_member"] = self._member_of(qu.slot_member.cpu().numpy() if qu is not None else np.full(self.B, -1))
@@ -387,7 +466,9 @@ class EnsembleRollout:
         Copies only the counters, the block's rows and the filled ring slots to the host.  Raises if a member's snapshot
         ring overflowed (a snapshot was due while every slot held an undrained one: drain more often or use more slots).
         In a sweep: a dict {member index: logs} over the members that took a step in the block, each with the fields
-        above plus `finished` (the member has stopped); t is the cumsum of the member's dt from its own t0."""
+        above plus `finished` (the member has stopped); t is the cumsum of the member's dt from its own t0.
+        With diagnostics, also q_bot, q_top, vrms (float64 [n], one per step taken) and steady (the member has been
+        stopped by the steady criterion)."""
         self._require_clock()
         clk = self._clk
         ck = self.read_clock()
@@ -405,6 +486,9 @@ class EnsembleRollout:
             lo = self._pending[0]
             dts = self.state.dt_seq[lo:lo + nmax].cpu().numpy()
             mts = clk.meanT_seq[lo:lo + nmax].cpu().numpy()
+            if self._diag is not None:
+                fls = self._diag.flux_seq[lo:lo + nmax].cpu().numpy()
+                vrs = self._diag.vrms_seq[lo:lo + nmax].cpu().numpy()
         _, ring, meta = self._ring_entries(ck)
         out, r = [], 0
         for m in range(self.B):
@@ -420,6 +504,11 @@ class EnsembleRollout:
                               "p": f[3] if clk.nch == 4 else None})
                 r += 1
             d["snapshots"] = snaps
+            if self._diag is not None:
+                d["q_bot"] = fls[:k, m, 0].copy() if k else np.zeros(0)
+                d["q_top"] = fls[:k, m, 1].copy() if k else np.zeros(0)
+                d["vrms"] = vrs[:k, m].copy() if k else np.zeros(0)
+                d["steady"] = bool(ck["steady"][m])
             out.append(d)
         clk.clock.view(torch.int64)[:, _DRAINED].copy_(torch.from_numpy(ck["snaps"].copy()))
         self._host_t, self._host_steps, self._host_active = ck["t"].copy(), ck["steps"].copy(), ck["active"].copy()
@@ -437,7 +526,7 @@ class EnsembleRollout:
         return pairs, clk.ring[si, mi].cpu().numpy(), clk.meta[si, mi].cpu().numpy()
 
     def _drain_sweep(self, ck):
-        sw, clk, qu = self._sweep, self._clk, self._run_queue()
+        sw, clk, qu, dg = self._sweep, self._clk, self._run_queue(), self._diag
         out = {}
         if qu is None:
             self._pending = None
@@ -449,9 +538,13 @@ class EnsembleRollout:
             seq = self._member_of(qu.member_seq[lo:lo + k].cpu().numpy())
             dts = self.state.dt_seq[lo:lo + k].cpu().numpy()
             mts = clk.meanT_seq[lo:lo + k].cpu().numpy()
+            if dg is not None:
+                fls, vrs = dg.flux_seq[lo:lo + k].cpu().numpy(), dg.vrms_seq[lo:lo + k].cpu().numpy()
             for m in np.unique(seq[seq >= 0]):
                 j, s = np.nonzero(seq == m)  # row-major: in step order (a member runs in one slot)
                 steps[int(m)] = (dts[j, s].copy(), mts[j, s].copy())
+                if dg is not None:
+                    steps[int(m)] += (fls[j, s, 0].copy(), fls[j, s, 1].copy(), vrs[j, s].copy())
         snaps = {}
         if pairs:
             owner = self._member_of(qu.snap_member.cpu().numpy())
@@ -462,7 +555,7 @@ class EnsembleRollout:
                      "p": f[3] if clk.nch == 4 else None})
         running = set(ck["slot_member"][ck["active"]].tolist())
         for m in sorted(set(steps) | set(snaps)):
-            dt, mt = steps.get(m, (np.zeros(0), np.zeros(0)))
+            dt, mt = steps.get(m, (np.zeros(0), np.zeros(0)))[:2]
             h_t, h_n = sw["t"][m], sw["steps"][m]
             d = {"dt": dt, "meanT": mt, "steps": np.arange(h_n + 1, h_n + 1 + len(dt), dtype=np.int64)}
             d["t"] = np.cumsum(np.concatenate(([h_t], dt)))[1:]  # the device's own additions: == its clock bit for bit
@@ -470,6 +563,11 @@ class EnsembleRollout:
             d["finished"] = m not in running
             if len(dt):
                 sw["t"][m], sw["steps"][m] = d["t"][-1], d["steps"][-1]
+            if dg is not None:
+                d["q_bot"], d["q_top"], d["vrms"] = steps[m][2:] if m in steps else (np.zeros(0),) * 3
+                # a refill resets the slot's steady state, so it is read from the clock: a member stops either at its
+                # t_end / max_steps or, before both, by the criterion (the limits take precedence at the same step)
+                d["steady"] = bool(d["finished"] and sw["t"][m] < sw["t_end"][m] and sw["steps"][m] < sw["max_steps"][m])
             out[m] = d
         occupied = ck["slot_member"] >= 0
         who = ck["slot_member"][occupied]
