@@ -516,6 +516,45 @@ int pbmc_rollout_diagnosed(pbmc_ctx* ctx, const pbmc_net* net_h, pbmc_member* me
                            double* snap_meta, int snap_slots, const pbmc_member_queue* queue_h,
                            const pbmc_diag_desc* diag_h, void* stream);
 
+/* ------------------------------------------------------------------ parameter-continuation chains
+ * Members of a queue may continue from the state their predecessor stopped in.  succ[p] = q (p < q; each entry has at
+ * most one successor and one predecessor) means: entry q starts from the T that entry p had after its last step, in the
+ * slot p ran in, handed over at p's stop step whatever stopped p.  Entries
+ * that are nobody's successor are chain heads; heads[0 .. K-1] lists them in entry order, and `next` counts heads.
+ * Rule at step i, fixed so that it can be tested:
+ *   - a slot whose member p stops after step i and has a successor q = succ[p] hands over: from step i + 1, q runs in
+ *     the slot with
+ *       T (the step's output slot) unchanged bit for bit, members[s] = params[q] bit for bit,
+ *       clock: t = t0[q], t_end[q], save_t = 0, save_every[q], steps = n_step0[q], max_steps[q], active = 1,
+ *       steady state and history ring reset (as a refill sets them);
+ *     the same launches store that T into T0[q] (so the queue's T0 must be writable: it holds q's start field afterwards,
+ *     and T0[q] is never read for a successor);
+ *   - of the slots that stop after step i and whose member has NO successor, the one with rank r (r = how many such
+ *     slots with a lower index) takes head heads[next + r] if next + r < K, as pbmc_rollout_queued's refill; then next +=
+ *     the number of such slots (at most K).  A slot with a successor never takes a head.
+ * The finishing member's mean-T, diagnostics and a due snapshot are taken before the hand-off.  The caller places
+ * heads[0 .. min(B, K) - 1] into slots 0 .. in order (next = min(B, K), slot_member = those entries); successors never
+ * start in the initial placement.  Every member of a chain must be able to take a step (t0 < t_end, n_step0 <
+ * max_steps).  slot_member / member_seq / snap_member hold entries, as in pbmc_member_queue.
+ *   heads [K], succ [Q] (-1: none): int64 device arrays. */
+typedef struct {
+  const int64_t* heads;
+  const int64_t* succ;
+  int64_t K;
+} pbmc_member_chain;
+
+/* pbmc_rollout_diagnosed (diag_h may be NULL: no diagnostics) with a queue whose members may continue from their
+ * predecessors (chain_h, host struct of device pointers).  Same launches, none added.  Refused before any CUDA call:
+ * what pbmc_rollout_queued / pbmc_rollout_diagnosed refuse, a NULL queue_h or chain_h or a NULL array in the chain
+ * (PBMC_ERR_NULL_POINTER), K < 1 or K > Q (PBMC_ERR_BAD_SHAPE). */
+int pbmc_rollout_chained(pbmc_ctx* ctx, const pbmc_net* net_h, pbmc_member* members, const float* xc, const float* yc,
+                         const float* ycc, const float* xcoef, const float* ycoef, double dx_min, double cn_max,
+                         int per_member_dt, float* T_seq, int nslots, int first_step, int n_steps, double* dt_seq,
+                         int dt_seq_rows, float* u, float* v, float* p, float* V, void* workspace, size_t workspace_bytes,
+                         int B, int H, int W, pbmc_member_clock* clock, double* meanT_seq, float* snap_ring,
+                         double* snap_meta, int snap_slots, const pbmc_member_queue* queue_h, const pbmc_diag_desc* diag_h,
+                         const pbmc_member_chain* chain_h, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -104,7 +104,11 @@ class DiagDesc(C.Structure):
                 ("steady", C.c_void_p), ("part", C.c_void_p)]
 
 
-_STRUCTS = {"pbmc_diag_desc": DiagDesc, "pbmc_member_queue": MemberQueue, "pbmc_member_clock": MemberClock, "pbmc_edge9_desc": Edge9Desc, "pbmc_trunk_desc": TrunkDesc, "pbmc_slab_sync": SlabSync, "pbmc_member": Member, "pbmc_src": Src, "pbmc_conv_desc": ConvDesc, "pbmc_layer": Layer, "pbmc_net": Net}
+class MemberChain(C.Structure):
+    _fields_ = [("heads", C.c_void_p), ("succ", C.c_void_p), ("K", C.c_int64)]
+
+
+_STRUCTS = {"pbmc_member_chain": MemberChain, "pbmc_diag_desc": DiagDesc, "pbmc_member_queue": MemberQueue, "pbmc_member_clock": MemberClock, "pbmc_edge9_desc": Edge9Desc, "pbmc_trunk_desc": TrunkDesc, "pbmc_slab_sync": SlabSync, "pbmc_member": Member, "pbmc_src": Src, "pbmc_conv_desc": ConvDesc, "pbmc_layer": Layer, "pbmc_net": Net}
 
 # name -> (restype, argtypes); every symbol declared in include/pbmc.h
 _vp, _i, _d, _f, _sz = C.c_void_p, C.c_int, C.c_double, C.c_float, C.c_size_t
@@ -152,6 +156,9 @@ SIGNATURES = {
     "pbmc_rollout_diagnosed": (_i, [_vp, C.POINTER(Net), _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _vp, _i, _i, _i, _vp, _i,
                                     _vp, _vp, _vp, _vp, _vp, _sz, _i, _i, _i, _vp, _vp, _vp, _vp, _i, C.POINTER(MemberQueue),
                                     C.POINTER(DiagDesc), _vp]),
+    "pbmc_rollout_chained": (_i, [_vp, C.POINTER(Net), _vp, _vp, _vp, _vp, _vp, _vp, _d, _d, _i, _vp, _i, _i, _i, _vp, _i,
+                                  _vp, _vp, _vp, _vp, _vp, _sz, _i, _i, _i, _vp, _vp, _vp, _vp, _i, C.POINTER(MemberQueue),
+                                  C.POINTER(DiagDesc), C.POINTER(MemberChain), _vp]),
 }
 
 _lib = None

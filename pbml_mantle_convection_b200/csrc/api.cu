@@ -41,7 +41,7 @@ int advect_diffuse_enqueue(const float* T, const float* u, const float* v, const
 int clock_enqueue(pbmc_member_clock* clk, const float* Tin, float* Tout, const float* u, const float* v, const float* p,
                   double* dt_row, double* meanT_row, float* ring, double* meta, int slots, int B, int H, int W,
                   const pbmc_member_queue* queue, pbmc_member* members, int64_t* seq_row, const pbmc_diag_desc* diag,
-                  cudaStream_t st);  // clock.cu
+                  const pbmc_member_chain* chain, cudaStream_t st);  // clock.cu
 
 }  // namespace pbmc
 
@@ -83,6 +83,7 @@ extern "C" size_t pbmc_sizeof(const char* name) {
   if (!strcmp(name, "pbmc_member_clock")) return sizeof(pbmc_member_clock);
   if (!strcmp(name, "pbmc_member_queue")) return sizeof(pbmc_member_queue);
   if (!strcmp(name, "pbmc_diag_desc")) return sizeof(pbmc_diag_desc);
+  if (!strcmp(name, "pbmc_member_chain")) return sizeof(pbmc_member_chain);
   return 0;
 }
 
@@ -638,15 +639,16 @@ struct ClockArgs {
 };
 }  // namespace
 
-// pbmc_rollout, pbmc_rollout_clocked, pbmc_rollout_queued and pbmc_rollout_diagnosed: the same launches in the same
-// order; a clock adds its two launches behind every step's stencil, a queue (NULL except for pbmc_rollout_queued /
-// _diagnosed, whose members are mutable) and a diagnostics descriptor (NULL except for pbmc_rollout_diagnosed) none
+// pbmc_rollout, pbmc_rollout_clocked, pbmc_rollout_queued, pbmc_rollout_diagnosed and pbmc_rollout_chained: the same
+// launches in the same order; a clock adds its two launches behind every step's stencil, a queue (NULL except for
+// pbmc_rollout_queued / _diagnosed / _chained, whose members are mutable), a diagnostics descriptor (NULL except for
+// pbmc_rollout_diagnosed / _chained) and chains (NULL except for pbmc_rollout_chained) none
 static int rollout_impl(pbmc_ctx* ctx, const pbmc_net* net, const pbmc_member* members, const float* xc, const float* yc,
                         const float* ycc, const float* xcoef, const float* ycoef, double dx_min, double cn_max,
                         int per_member_dt, float* T_seq, int nslots, int first_step, int n_steps, double* dt_seq,
                         int dt_seq_rows, float* u, float* v, float* p, float* V, void* workspace, size_t workspace_bytes,
                         int B, int H, int W, const ClockArgs& clk, const pbmc_member_queue* queue, const pbmc_diag_desc* diag,
-                        void* stream) {
+                        const pbmc_member_chain* chain, void* stream) {
   if (!ctx || !net || !members || !xc || !yc || !ycc || !xcoef || !ycoef || !T_seq || !u || !v || !workspace) return PBMC_ERR_NULL_POINTER;
   if (nslots < 2 || first_step < 1 || n_steps < 0 || !(dx_min > 0.0)) return PBMC_ERR_BAD_SHAPE;
   if (dt_seq != nullptr && dt_seq_rows < first_step + n_steps - 1) return PBMC_ERR_BAD_SHAPE;  // step i writes row i - 1
@@ -694,7 +696,7 @@ static int rollout_impl(pbmc_ctx* ctx, const pbmc_net* net, const pbmc_member* m
       if (clk.clock)
         RC(clock_enqueue(clk.clock, Tin, Tout, u, v, p, dt_seq + (size_t)(i - 1) * B, clk.meanT_seq + (size_t)(i - 1) * B,
                          clk.snap_ring, clk.snap_meta, clk.snap_slots, B, H, W, queue, const_cast<pbmc_member*>(members),
-                         queue ? queue->member_seq + (size_t)(i - 1) * B : nullptr, diag ? &dg : nullptr, st));
+                         queue ? queue->member_seq + (size_t)(i - 1) * B : nullptr, diag ? &dg : nullptr, chain, st));
     }
     return PBMC_OK;
   };
@@ -714,7 +716,7 @@ extern "C" int pbmc_rollout(pbmc_ctx* ctx, const pbmc_net* net, const pbmc_membe
   const ClockArgs none = {nullptr, nullptr, nullptr, nullptr, 0};
   return rollout_impl(ctx, net, members, xc, yc, ycc, xcoef, ycoef, dx_min, cn_max, per_member_dt, T_seq, nslots, first_step,
                       n_steps, dt_seq, dt_seq_rows, u, v, p, V, workspace, workspace_bytes, B, H, W, none, nullptr, nullptr,
-                      stream);
+                      nullptr, stream);
 }
 
 // the refusals of a clocked rollout, shared by pbmc_rollout_clocked and pbmc_rollout_queued
@@ -736,10 +738,10 @@ extern "C" int pbmc_rollout_clocked(pbmc_ctx* ctx, const pbmc_net* net, const pb
   const ClockArgs clk = {clock, meanT_seq, snap_ring, snap_meta, snap_slots};
   return rollout_impl(ctx, net, members, xc, yc, ycc, xcoef, ycoef, dx_min, cn_max, per_member_dt, T_seq, nslots, first_step,
                       n_steps, dt_seq, dt_seq_rows, u, v, p, V, workspace, workspace_bytes, B, H, W, clk, nullptr, nullptr,
-                      stream);
+                      nullptr, stream);
 }
 
-// the refusals of a member queue, shared by pbmc_rollout_queued and pbmc_rollout_diagnosed
+// the refusals of a member queue, shared by pbmc_rollout_queued, pbmc_rollout_diagnosed and pbmc_rollout_chained
 static int validate_queue(const pbmc_member_queue* queue, int B) {
   if (!queue) return PBMC_ERR_NULL_POINTER;
   const pbmc_member_queue& q = *queue;
@@ -764,7 +766,17 @@ extern "C" int pbmc_rollout_queued(pbmc_ctx* ctx, const pbmc_net* net, pbmc_memb
   const ClockArgs clk = {clock, meanT_seq, snap_ring, snap_meta, snap_slots};
   return rollout_impl(ctx, net, members, xc, yc, ycc, xcoef, ycoef, dx_min, cn_max, per_member_dt, T_seq, nslots, first_step,
                       n_steps, dt_seq, dt_seq_rows, u, v, p, V, workspace, workspace_bytes, B, H, W, clk, queue, nullptr,
-                      stream);
+                      nullptr, stream);
+}
+
+// the refusals of a diagnostics descriptor, shared by pbmc_rollout_diagnosed and pbmc_rollout_chained
+static int validate_diag(const pbmc_diag_desc& d, int H, int W) {
+  if (!d.flux_seq || !d.vrms_seq || !d.steady || !d.part) return PBMC_ERR_NULL_POINTER;
+  if (d.window < 0 || d.window > PBMC_STEADY_MAX_WINDOW) return PBMC_ERR_BAD_SHAPE;
+  if (d.window > 0 && (!d.hist || !d.hist_n)) return PBMC_ERR_NULL_POINTER;
+  if (!(d.rtol >= 0.0) || !std::isfinite(d.rtol)) return PBMC_ERR_BAD_SHAPE;  // NaN fails the first test
+  if (H < 3 || W < 3) return PBMC_ERR_BAD_SHAPE;  // vrms averages over the interior cells
+  return PBMC_OK;
 }
 
 extern "C" int pbmc_rollout_diagnosed(pbmc_ctx* ctx, const pbmc_net* net, pbmc_member* members, const float* xc,
@@ -777,13 +789,27 @@ extern "C" int pbmc_rollout_diagnosed(pbmc_ctx* ctx, const pbmc_net* net, pbmc_m
   RC(validate_clock(clock, dt_seq, meanT_seq, snap_ring, snap_meta, snap_slots, per_member_dt, B));
   if (queue) RC(validate_queue(queue, B));
   if (!diag) return PBMC_ERR_NULL_POINTER;
-  const pbmc_diag_desc& d = *diag;
-  if (!d.flux_seq || !d.vrms_seq || !d.steady || !d.part) return PBMC_ERR_NULL_POINTER;
-  if (d.window < 0 || d.window > PBMC_STEADY_MAX_WINDOW) return PBMC_ERR_BAD_SHAPE;
-  if (d.window > 0 && (!d.hist || !d.hist_n)) return PBMC_ERR_NULL_POINTER;
-  if (!(d.rtol >= 0.0) || !std::isfinite(d.rtol)) return PBMC_ERR_BAD_SHAPE;  // NaN fails the first test
-  if (H < 3 || W < 3) return PBMC_ERR_BAD_SHAPE;  // vrms averages over the interior cells
+  RC(validate_diag(*diag, H, W));
   const ClockArgs clk = {clock, meanT_seq, snap_ring, snap_meta, snap_slots};
   return rollout_impl(ctx, net, members, xc, yc, ycc, xcoef, ycoef, dx_min, cn_max, per_member_dt, T_seq, nslots, first_step,
-                      n_steps, dt_seq, dt_seq_rows, u, v, p, V, workspace, workspace_bytes, B, H, W, clk, queue, diag, stream);
+                      n_steps, dt_seq, dt_seq_rows, u, v, p, V, workspace, workspace_bytes, B, H, W, clk, queue, diag, nullptr,
+                      stream);
+}
+
+extern "C" int pbmc_rollout_chained(pbmc_ctx* ctx, const pbmc_net* net, pbmc_member* members, const float* xc,
+                                    const float* yc, const float* ycc, const float* xcoef, const float* ycoef, double dx_min,
+                                    double cn_max, int per_member_dt, float* T_seq, int nslots, int first_step, int n_steps,
+                                    double* dt_seq, int dt_seq_rows, float* u, float* v, float* p, float* V, void* workspace,
+                                    size_t workspace_bytes, int B, int H, int W, pbmc_member_clock* clock, double* meanT_seq,
+                                    float* snap_ring, double* snap_meta, int snap_slots, const pbmc_member_queue* queue,
+                                    const pbmc_diag_desc* diag, const pbmc_member_chain* chain, void* stream) {
+  RC(validate_clock(clock, dt_seq, meanT_seq, snap_ring, snap_meta, snap_slots, per_member_dt, B));
+  RC(validate_queue(queue, B));
+  if (diag) RC(validate_diag(*diag, H, W));
+  if (!chain || !chain->heads || !chain->succ) return PBMC_ERR_NULL_POINTER;
+  if (chain->K < 1 || chain->K > queue->Q) return PBMC_ERR_BAD_SHAPE;
+  const ClockArgs clk = {clock, meanT_seq, snap_ring, snap_meta, snap_slots};
+  return rollout_impl(ctx, net, members, xc, yc, ycc, xcoef, ycoef, dx_min, cn_max, per_member_dt, T_seq, nslots, first_step,
+                      n_steps, dt_seq, dt_seq_rows, u, v, p, V, workspace, workspace_bytes, B, H, W, clk, queue, diag, chain,
+                      stream);
 }

@@ -25,6 +25,11 @@
 // vrms) into the slot's history ring and scans the ring with the member's warp.  A member found steady after step s
 // stops at step s + 1 through clock_stops, so the queue's refill rule needs nothing new.  Without a descriptor
 // (dg.part == NULL, block-uniform) neither kernel touches any of this.
+//
+// With chains (pbmc_rollout_chained) a stopping slot whose member has a successor hands its T over in place: apply
+// skips the T0 overwrite and stores the slot's new T into the successor's T0 row on the same pass; commit loads the
+// successor's clock and member row.  The refill rank counts only the stopping slots without a successor, and queue
+// entries come from the heads list.  Without chains (ch.succ == NULL, block-uniform) neither kernel touches any of this.
 #include <string.h>
 
 #include "common.cuh"
@@ -49,6 +54,14 @@ __device__ __forceinline__ bool clock_ring_full(const pbmc_member_clock& c, int 
 __device__ __forceinline__ bool clock_stops(const pbmc_member_clock& c, double dt, int st) {
   return clock_active(c, st) && (st == PBMC_STEADY_FOUND || !(c.t + dt < c.t_end && c.steps + 1 < c.max_steps));
 }
+// the successor of the member in slot m (-1: none, or no chains)
+__device__ __forceinline__ int64_t chain_succ(const pbmc_member_chain& ch, const pbmc_member_queue& qu, int m) {
+  if (!ch.succ) return -1;
+  const int64_t w = qu.slot_member[m];
+  return w < 0 ? -1 : ch.succ[w];
+}
+// the queue entry that head rank j (next + r) stands for
+__device__ __forceinline__ int64_t head_entry(const pbmc_member_chain& ch, int64_t j) { return ch.succ ? ch.heads[j] : j; }
 
 // cell e (column col) of a member plane into the descriptor's sums; rb / rt = first cell of rows H-2 / H-1 (H >= 3:
 // for H = 3 row 1 goes into both r1 and rb)
@@ -70,7 +83,7 @@ __global__ void __launch_bounds__(CLK_THREADS, 4)
     clock_apply_kernel(pbmc_member_clock* __restrict__ clk, const float* __restrict__ Tin, float* __restrict__ Tout,
                        const float* __restrict__ u, const float* __restrict__ v, const float* __restrict__ p,
                        const double* __restrict__ dt_row, float* __restrict__ ring, int slots, int nch, size_t n, size_t chunk,
-                       int W, const pbmc_member_queue qu, const pbmc_diag_desc dg) {
+                       int W, const pbmc_member_queue qu, const pbmc_diag_desc dg, const pbmc_member_chain ch) {
   __shared__ double red[1 + DIAG_SUMS][CLK_THREADS / 32];
   const int m = blockIdx.y, part = blockIdx.x;
   const int B = gridDim.y;
@@ -93,17 +106,26 @@ __global__ void __launch_bounds__(CLK_THREADS, 4)
   const double t_new = c.t + dt_row[m];
   const bool snap = t_new > c.save_t && !clock_ring_full(c, slots);
   float* dst = snap ? ring + ((size_t)(c.snaps % slots) * B + m) * nch * n : nullptr;
-  // queue: this member stops here and the queue holds an entry for the slot -> its T0 replaces the new T once read
-  // (block-uniform: every thread reads the same clocks, dt row and next)
-  const float* T0q = nullptr;
+  // queue: this member stops here.  With a successor its new T stays and is also stored into the successor's T0 row
+  // (hand = true); otherwise, when the queue holds a head for the slot, that head's T0 replaces the new T once read
+  // (block-uniform: every thread reads the same clocks, dt row, slot members and next).  One pointer for both: the
+  // kernel has no register to spare
+  float* T0q = nullptr;
+  bool hand = false;
   if (qu.Q > 0 && clock_stops(c, dt_row[m], st)) {
-    int r = 0;
-    for (int b0 = 0; b0 < m; b0 += CLK_THREADS) {
-      const int o = b0 + (int)threadIdx.x;
-      r += __syncthreads_count(o < m && clock_stops(clk[o], dt_row[o], steady_of(dg, o)));
+    const int64_t succ = chain_succ(ch, qu, m);
+    if (succ >= 0) {
+      T0q = const_cast<float*>(qu.T0) + (size_t)succ * n;  // written for chains only (include/pbmc.h)
+      hand = true;
+    } else {
+      int r = 0;
+      for (int b0 = 0; b0 < m; b0 += CLK_THREADS) {
+        const int o = b0 + (int)threadIdx.x;
+        r += __syncthreads_count(o < m && clock_stops(clk[o], dt_row[o], steady_of(dg, o)) && chain_succ(ch, qu, o) < 0);
+      }
+      const int64_t j = *qu.next + r;
+      if (j < (ch.succ ? ch.K : qu.Q)) T0q = const_cast<float*>(qu.T0) + (size_t)head_entry(ch, j) * n;
     }
-    const int64_t q = *qu.next + r;
-    if (q < qu.Q) T0q = qu.T0 + (size_t)q * n;
   }
   double s = 0.0;
   double a[DIAG_SUMS] = {0.0, 0.0, 0.0, 0.0, 0.0};  // descriptor sums (diag only)
@@ -115,6 +137,7 @@ __global__ void __launch_bounds__(CLK_THREADS, 4)
     for (size_t i = i0; i < hi; i += 4 * CLK_THREADS) {
       const float4 t4 = *reinterpret_cast<const float4*>(Tout + base + i);
       s += ((double)t4.x + (double)t4.y) + ((double)t4.z + (double)t4.w);
+      if (hand) *reinterpret_cast<float4*>(T0q + i) = t4;  // here: t4 is not kept live across the diagnostics
       float4 u4, v4;
       if (snap || diag) {
         u4 = *reinterpret_cast<const float4*>(u + base + i);
@@ -137,7 +160,7 @@ __global__ void __launch_bounds__(CLK_THREADS, 4)
         col += col_step;
         if (col >= W) col -= W;
       }
-      if (T0q) *reinterpret_cast<float4*>(Tout + base + i) = *reinterpret_cast<const float4*>(T0q + i);
+      if (T0q && !hand) *reinterpret_cast<float4*>(Tout + base + i) = *reinterpret_cast<const float4*>(T0q + i);
     }
   } else {
     const size_t i0 = lo + threadIdx.x;
@@ -146,6 +169,7 @@ __global__ void __launch_bounds__(CLK_THREADS, 4)
     for (size_t i = i0; i < hi; i += CLK_THREADS) {
       const float t1 = Tout[base + i];
       s += (double)t1;
+      if (hand) T0q[i] = t1;
       if (snap) {
         dst[i] = t1;
         dst[n + i] = u[base + i];
@@ -157,7 +181,7 @@ __global__ void __launch_bounds__(CLK_THREADS, 4)
         col += col_step;
         if (col >= W) col -= W;
       }
-      if (T0q) Tout[base + i] = T0q[i];
+      if (T0q && !hand) Tout[base + i] = T0q[i];
     }
   }
   // fixed-order block reduction: warp tree, then warp 0 over the warp sums
@@ -191,14 +215,15 @@ __global__ void __launch_bounds__(CLK_THREADS, 4)
 }
 
 // one warp per member (strided), lane 0 writes.  Queue (qu.Q > 0): `stops` (dynamic shared memory, [B]) holds
-// clock_stops of every slot, taken before any clock is written; members / seq_row are the member rows and this step's
-// member_seq row.  Descriptor (dg.part != NULL): dg.flux_seq / dg.vrms_seq are this step's rows.
+// clock_stops of every slot, taken before any clock is written (1: the slot takes a head, 2: its member has a successor);
+// members / seq_row are the member rows and this step's member_seq row.  Descriptor (dg.part != NULL): dg.flux_seq /
+// dg.vrms_seq are this step's rows.
 __global__ void __launch_bounds__(CLK_THREADS) clock_commit_kernel(pbmc_member_clock* __restrict__ clk, double* __restrict__ dt_row,
                                                                    double* __restrict__ meanT_row, double* __restrict__ meta, int slots,
                                                                    int parts, double inv_n, int H, int W, int B,
                                                                    const pbmc_member_queue qu,
                                                                    pbmc_member* __restrict__ members, int64_t* __restrict__ seq_row,
-                                                                   const pbmc_diag_desc dg) {
+                                                                   const pbmc_diag_desc dg, const pbmc_member_chain ch) {
   extern __shared__ int stops[];
   const int lane = threadIdx.x & 31;
   const bool queued = qu.Q > 0;
@@ -206,7 +231,8 @@ __global__ void __launch_bounds__(CLK_THREADS) clock_commit_kernel(pbmc_member_c
   int64_t next = 0;
   if (queued) {
     next = *qu.next;
-    for (int m = threadIdx.x; m < B; m += CLK_THREADS) stops[m] = clock_stops(clk[m], dt_row[m], steady_of(dg, m)) ? 1 : 0;
+    for (int m = threadIdx.x; m < B; m += CLK_THREADS)
+      stops[m] = clock_stops(clk[m], dt_row[m], steady_of(dg, m)) ? (chain_succ(ch, qu, m) >= 0 ? 2 : 1) : 0;
     __syncthreads();
   }
   for (int m = threadIdx.x >> 5; m < B; m += CLK_THREADS / 32) {
@@ -236,9 +262,9 @@ __global__ void __launch_bounds__(CLK_THREADS) clock_commit_kernel(pbmc_member_c
         a[k] = warp_sum(a[k]);
       }
     }
-    int r = 0;  // rank among the slots that stop at this step (the apply kernel's count)
-    if (queued && stops[m]) {
-      for (int o = lane; o < m; o += 32) r += stops[o];
+    int r = 0;  // rank among the slots that stop at this step and take a head (the apply kernel's count)
+    if (queued && stops[m] == 1) {
+      for (int o = lane; o < m; o += 32) r += stops[o] == 1;
       r = __reduce_add_sync(0xffffffffu, r);
     }
     int scan = 0;  // the member goes on and its history ring holds `window` values: evaluate the criterion
@@ -278,8 +304,10 @@ __global__ void __launch_bounds__(CLK_THREADS) clock_commit_kernel(pbmc_member_c
         running = false;
       }
       c->active = running ? 1 : 0;
-      if (queued && stops[m] && next + r < qu.Q) {
-        const int64_t q = next + r;  // the slot's next member, from step i + 1 on
+      int64_t q = -1;  // the slot's next member, from step i + 1 on: the successor, or the head of rank r
+      if (queued && stops[m] == 2) q = ch.succ[who];
+      else if (queued && stops[m] == 1 && next + r < (ch.succ ? ch.K : qu.Q)) q = head_entry(ch, next + r);
+      if (q >= 0) {
         c->t = qu.t0[q];
         c->t_end = qu.t_end[q];
         c->save_t = 0.0;
@@ -334,8 +362,9 @@ __global__ void __launch_bounds__(CLK_THREADS) clock_commit_kernel(pbmc_member_c
     __syncthreads();  // every thread has read next
     if (threadIdx.x == 0) {
       int64_t k = 0;
-      for (int m = 0; m < B; ++m) k += stops[m];
-      *qu.next = next + k < qu.Q ? next + k : qu.Q;
+      for (int m = 0; m < B; ++m) k += stops[m] == 1;
+      const int64_t K = ch.succ ? ch.K : qu.Q;
+      *qu.next = next + k < K ? next + k : K;
     }
   }
 }
@@ -351,10 +380,11 @@ int clock_parts(size_t n) {
 // meanT_row the step's rows ([B] each) of dt_seq / meanT_seq.
 // queue (NULL: none): the rollout's member queue, members its member rows, seq_row the step's row of member_seq.
 // diag (NULL: none): the diagnostics descriptor with flux_seq / vrms_seq pointing at the step's rows.
+// chain (NULL: none; only with a queue): the queue's successor and head lists.
 int clock_enqueue(pbmc_member_clock* clk, const float* Tin, float* Tout, const float* u, const float* v, const float* p,
                   double* dt_row, double* meanT_row, float* ring, double* meta, int slots, int B, int H, int W,
                   const pbmc_member_queue* queue, pbmc_member* members, int64_t* seq_row, const pbmc_diag_desc* diag,
-                  cudaStream_t st) {
+                  const pbmc_member_chain* chain, cudaStream_t st) {
   const size_t n = (size_t)H * W;
   const int parts = clock_parts(n);
   size_t chunk = (n + parts - 1) / parts;
@@ -366,12 +396,15 @@ int clock_enqueue(pbmc_member_clock* clk, const float* Tin, float* Tout, const f
   pbmc_diag_desc dg;
   memset(&dg, 0, sizeof(dg));  // part = NULL: no diagnostics
   if (diag) dg = *diag;
+  pbmc_member_chain ch;
+  memset(&ch, 0, sizeof(ch));  // succ = NULL: no chains
+  if (chain) ch = *chain;
   const size_t smem = queue ? (size_t)B * sizeof(int) : 0;
   clock_apply_kernel<<<dim3(parts, B), CLK_THREADS, 0, st>>>(clk, Tin, Tout, u, v, p, dt_row, ring, slots, nch, n, chunk, W, qu,
-                                                             dg);
+                                                             dg, ch);
   PBMC_CHECK_LAUNCH("clock_apply_kernel");
   clock_commit_kernel<<<1, CLK_THREADS, smem, st>>>(clk, dt_row, meanT_row, meta, slots, parts, 1.0 / (double)n, H, W, B, qu, members,
-                                                     seq_row, dg);
+                                                     seq_row, dg, ch);
   PBMC_CHECK_LAUNCH("clock_commit_kernel");
   return PBMC_OK;
 }

@@ -31,7 +31,8 @@ Three ways to advance:
     read back once per block of `check_every` steps.
   * `attempt_sweep(ens, T0, params, ...)` -- the same for a sweep of Q members run through the B slots of an
     `EnsembleRollout` (`EnsembleRollout.start_sweep`): a slot whose member stops takes the next queued member on the
-    device, so Q may exceed B and no slot idles while members wait.
+    device, so Q may exceed B and no slot idles while members wait.  With `continue_from`, a member starts from the
+    field its predecessor stopped with (parameter continuation), handed over on the device.
 
 External energy solver (the `ML_STOKES` / `ML_PRE` modes and the `intervene_TS` interventions of mode "ML", `:486-505`,
 `:618-630`): the reference calls GAIA's `sim.doTimestep()` with the surrogate's velocities already written into the state
@@ -214,22 +215,29 @@ def attempt_ensemble(ens, xcc, ycc, t_end, out_dir, save_every=0.0, write_every=
 
 
 def attempt_sweep(ens, T0, params, xcc, ycc, t_end, out_dir, save_every=0.0, write_every=0.0, mode="ML", t=0.0, n_step=0,
-                  check_every=10, max_steps=None, diagnostics=False, steady=None):
+                  check_every=10, max_steps=None, diagnostics=False, steady=None, continue_from=None):
     """`attempt` for each of Q members run through the B slots of a device-resident `EnsembleRollout`
     (`EnsembleRollout.start_sweep`; Q may be larger or smaller than B).  T0: [Q, H, W]; params: Q tuples (RaQ, gamma,
     beta); t_end, save_every, t, n_step, max_steps: scalars or one value per member.  Member q's pickles go to
     `out_dir/member_<q>/`, with `attempt_ensemble`'s cadence and content: the slot a member ran in, and when, make no
-    difference.  Returns (t [Q], n_step [Q], [logs of member q]).  diagnostics / steady: as in `attempt_ensemble`."""
+    difference.  Returns (t [Q], n_step [Q], [logs of member q]).  diagnostics / steady: as in `attempt_ensemble`.
+    continue_from: as in `EnsembleRollout.start_sweep`; a continued member's pickles are those of `attempt` run alone
+    from the field its predecessor stopped with (its initial entries are written when it starts)."""
     Q, H, W = len(params), ens.H, ens.W
     n = H * W
     k = int(check_every)
     logs = [_new_logs(mode) for _ in range(Q)]
     dirs = [os.path.join(out_dir, f"member_{q}") for q in range(Q)]
     T0 = torch.as_tensor(T0).to("cpu", torch.float32).reshape(Q, H, W)  # what the device runs from
-    _initial_entries(logs, T0.double().numpy().reshape(Q, n), t, xcc, ycc, mode, n)
+    t0 = np.broadcast_to(np.asarray(t, dtype=np.float64), (Q,)).copy()
+    chain = {} if continue_from is None else {"continue_from": continue_from}
     ens.start_sweep(T0, params, t_end, save_every=save_every, t0=t, max_steps=max_steps, n_step=n_step, snap_slots=k,
-                    steps_per_graph=k, **_diag_kwargs(diagnostics, steady))
-    return _run_blocks(ens, k, logs, dirs, t, n_step, write_every, mode, n, _diag_logs(Q, diagnostics, steady))
+                    steps_per_graph=k, **_diag_kwargs(diagnostics, steady), **chain)
+    heads = [q for q in range(Q) if continue_from is None or continue_from[q] == -1]
+    _initial_entries([logs[q] for q in heads], T0[heads].double().numpy().reshape(len(heads), n), t0[heads], xcc, ycc,
+                     mode, n)
+    start = lambda m, T: _initial_entries([logs[m]], T.astype(np.float64).reshape(1, n), t0[m:m + 1], xcc, ycc, mode, n)
+    return _run_blocks(ens, k, logs, dirs, t, n_step, write_every, mode, n, _diag_logs(Q, diagnostics, steady), start)
 
 
 def _diag_kwargs(diagnostics, steady):
@@ -252,12 +260,13 @@ def _initial_entries(logs, T0, t, xcc, ycc, mode, n):
         snapshots[mode]["xcc"], snapshots[mode]["ycc"] = xcc, ycc
 
 
-def _run_blocks(ens, k, logs, dirs, t, n_step, write_every, mode, n, diag=None):
+def _run_blocks(ens, k, logs, dirs, t, n_step, write_every, mode, n, diag=None, start=None):
     """Blocks of k steps (one graph replay each) until no member of the running clock or sweep is left; each drained
     block (a list over the members, or a sweep's dict keyed by member) goes into the logs of its members.  A
     TS_vec entry is the block's wall time over the steps the member took in it; `t > write_t` is evaluated at block
     ends.  Writes every member's pickles at the end; returns (t, n_step, logs) per member.  diag: per member
-    (Nu_vec, vrms_vec) lists filled from the blocks' q_bot, q_top, vrms and written with the other pickles."""
+    (Nu_vec, vrms_vec) lists filled from the blocks' q_bot, q_top, vrms and written with the other pickles.  start:
+    start(m, start_T) writes a continued member's initial entries when its first block carries start_T."""
 
     def write(m):
         write_logs(dirs[m], mode, *logs[m])
@@ -275,6 +284,8 @@ def _run_blocks(ens, k, logs, dirs, t, n_step, write_every, mode, n, diag=None):
         blk = ens.drain()
         wall = time.time() - w0
         for m, d in (blk.items() if isinstance(blk, dict) else enumerate(blk)):
+            if "start_T" in d:
+                start(m, d["start_T"])
             snapshots, TS_vec, t_vec, T_vec = logs[m]
             taken = len(d["dt"])
             for tm, mt in zip(d["t"], d["meanT"]):

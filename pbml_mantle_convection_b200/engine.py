@@ -228,11 +228,13 @@ class SurrogateEngine:
                                                 L.stream_ptr(dev)), "pbmc_surrogate_forward")
         return u, v, p, uvmax
 
-    def rollout(self, state, first_step, n_steps, clock=None, queue=None, diag=None):
+    def rollout(self, state, first_step, n_steps, clock=None, queue=None, diag=None, chain=None):
         """Enqueue n_steps time steps on `state` (a RolloutState).  No host sync.  clock: a rollout.MemberClocks (the
         per-member run-to-time clock, pbmc_rollout_clocked) or None (pbmc_rollout); queue (with a clock only): a
         rollout.SweepQueue whose members refill the slots that stop (pbmc_rollout_queued); diag (with a clock only): a
-        rollout.MemberDiagnostics, per-step wall fluxes / rms velocity and the steady stop (pbmc_rollout_diagnosed)."""
+        rollout.MemberDiagnostics, per-step wall fluxes / rms velocity and the steady stop (pbmc_rollout_diagnosed);
+        chain (with a queue only): a _lib.MemberChain whose members continue from their predecessors
+        (pbmc_rollout_chained)."""
         self.refresh()
         s = state
         ws = self.workspace(s.B, s.H, s.W)
@@ -246,7 +248,11 @@ class SurrogateEngine:
             L.check(L.load().pbmc_rollout(*args, L.stream_ptr(self.device)), "pbmc_rollout")
             return
         clk = (L.ptr(clock.clock), L.ptr(clock.meanT_seq), L.ptr(clock.ring), L.ptr(clock.meta), int(clock.slots))
-        if diag is not None:
+        if chain is not None:
+            L.check(L.load().pbmc_rollout_chained(*args, *clk, C.byref(queue.desc),
+                                                  C.byref(diag.desc) if diag is not None else None, C.byref(chain),
+                                                  L.stream_ptr(self.device)), "pbmc_rollout_chained")
+        elif diag is not None:
             L.check(L.load().pbmc_rollout_diagnosed(*args, *clk, C.byref(queue.desc) if queue is not None else None,
                                                     C.byref(diag.desc), L.stream_ptr(self.device)), "pbmc_rollout_diagnosed")
         elif queue is not None:

@@ -19,6 +19,10 @@ Per-step diagnostics and the steady stop (`start_clock(..., diagnostics=True)` o
 `start_sweep`): the same launches also log the wall heat fluxes q_bot / q_top and the rms velocity of every step
 (pbmc_rollout_diagnosed; include/pbmc.h defines them), and with `steady` a member stops one step after its meanT, q_top
 and vrms have each varied by at most rtol (relative) over the last `window` steps.
+
+Parameter continuation (`start_sweep(..., continue_from=...)`): a member may start from the T its predecessor stopped
+with, handed over on the device in the predecessor's slot (pbmc_rollout_chained), so a ladder of parameters follows one
+branch of steady states without a host round-trip between rungs.
 """
 from __future__ import annotations
 
@@ -81,7 +85,8 @@ class MemberClocks:
 
 class SweepQueue:
     """Device buffers of a sweep's member queue (pbmc_member_queue): the queued members' T0, parameter rows and clock
-    starts, `next`, the slot each member is in and the member_seq / snap_member tags.  `desc` is the C struct."""
+    starts, `next`, the slot each member is in and the member_seq / snap_member tags.  `desc` is the C struct.  With
+    chains also the heads and successors of pbmc_member_chain; `chain` is that C struct (its K is set per sweep)."""
 
     def __init__(self, Q, B, H, W, rows, slots, device):
         f64 = lambda n: torch.zeros(n, dtype=torch.float64, device=device)
@@ -98,11 +103,17 @@ class SweepQueue:
                      "snap_member"):
             setattr(d, name, L.ptr(getattr(self, name)))
         d.Q = self.Q
+        self.heads, self.succ = i64(Q), i64(Q)
+        self.chain = L.MemberChain()
+        self.chain.heads, self.chain.succ = L.ptr(self.heads), L.ptr(self.succ)
 
     def key(self):
         d = self.desc
         return ("queue", d.T0, d.params, d.t0, d.t_end, d.save_every, d.n_step0, d.max_steps, d.next, d.slot_member,
                 d.member_seq, d.snap_member, d.Q)
+
+    def chain_key(self):
+        return ("chain", self.chain.heads, self.chain.succ, self.chain.K)  # K is a launch argument
 
 
 class MemberDiagnostics:
@@ -147,6 +158,30 @@ def _steady_args(diagnostics, steady):
     if not (math.isfinite(rtol) and rtol >= 0.0):
         raise ValueError(f"steady rtol must be finite and >= 0, got {rtol!r}")
     return int(window), rtol
+
+
+def _continue_from(continue_from, Q, can_step):
+    """start_sweep's continue_from checked against the Q members (can_step: whether each could take a step): int64 [Q]."""
+    if len(continue_from) != Q:
+        raise ValueError(f"continue_from has {len(continue_from)} entries for {Q} members")
+    cf = np.empty(Q, dtype=np.int64)
+    for q, p in enumerate(continue_from):
+        if isinstance(p, (bool, np.bool_)) or not isinstance(p, (int, np.integer)):
+            raise ValueError(f"continue_from[{q}] must be an integer member index or -1, got {p!r}")
+        if not -1 <= p < q:
+            raise ValueError(f"continue_from[{q}] = {p}: a member continues from an earlier member (0 <= p < {q}) or -1")
+        cf[q] = p
+    preds = cf[cf >= 0]
+    if len(np.unique(preds)) != len(preds):
+        dup = sorted({int(p) for p in preds if (preds == p).sum() > 1})
+        raise ValueError(f"members {dup} are continued by more than one member")
+    chained = cf >= 0
+    chained[preds] = True
+    bad = np.flatnonzero(chained & ~can_step)
+    if len(bad):
+        raise ValueError(f"members {bad.tolist()} are in a chain but would take no step (t0 >= t_end or n_step >= "
+                         "max_steps): the chain would break")
+    return cf
 
 
 class EnsembleRollout:
@@ -201,7 +236,8 @@ class EnsembleRollout:
             first = 1 + (self.n_done % 2)
             k = min(n - done, self.max_steps)
             self._begin_block(first - 1, k)
-            self.engine.rollout(self.state, first, k, clock=self._clk, queue=self._run_queue(), diag=self._diag)
+            self.engine.rollout(self.state, first, k, clock=self._clk, queue=self._run_queue(), diag=self._diag,
+                                chain=self._run_chain())
             self.time += self.state.dt_seq[first - 1:first - 1 + k].sum(0)
             self.n_done += k
             done += k
@@ -216,26 +252,29 @@ class EnsembleRollout:
         par = self.n_done % 2
         # the graph bakes in packed-weight and workspace addresses and the conv implementation: key on them too
         key = (k, par) + self.engine.graph_key(self.B, self.H, self.W)
-        clk, qu, dg = self._clk, self._run_queue(), self._diag
+        clk, qu, dg, ch = self._clk, self._run_queue(), self._diag, self._run_chain()
         if clk is not None:
             key = key + clk.key()  # a clocked graph: its own entry (t_end, save_every live in device memory)
         if qu is not None:
             key = key + qu.key()  # a sweep's graph: refills only rewrite device memory
         if dg is not None:
             key = key + dg.key()  # window and rtol are launch arguments
+        if ch is not None:
+            key = key + qu.chain_key()
         if key not in self._graphs:
             # eager warm-up (module load + func attributes outside capture) on saved state: what a step may rewrite
             saved = [self.state.T_seq] + ([clk.clock] if clk is not None else []) + \
                     ([self.members, qu.next, qu.slot_member] if qu is not None else []) + \
-                    ([t for t in (dg.hist, dg.hist_n, dg.steady) if t is not None] if dg is not None else [])
+                    ([t for t in (dg.hist, dg.hist_n, dg.steady) if t is not None] if dg is not None else []) + \
+                    ([qu.T0] if ch is not None else [])  # a hand-off writes the successor's T0 row
             copies = [t.clone() for t in saved]
-            self.engine.rollout(self.state, 1 + par, 1, clock=clk, queue=qu, diag=dg)
+            self.engine.rollout(self.state, 1 + par, 1, clock=clk, queue=qu, diag=dg, chain=ch)
             for t, c in zip(saved, copies):
                 t.copy_(c)
             torch.cuda.synchronize(self.device)
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
-                self.engine.rollout(self.state, 1 + par, k, clock=clk, queue=qu, diag=dg)
+                self.engine.rollout(self.state, 1 + par, k, clock=clk, queue=qu, diag=dg, chain=ch)
             self._graphs[key] = g
         return self._graphs[key]
 
@@ -345,7 +384,7 @@ class EnsembleRollout:
         return dg
 
     def start_sweep(self, T0, params, t_end, save_every=0.0, t0=0.0, max_steps=None, n_step=0, snap_slots=None,
-                    steps_per_graph=10, diagnostics=False, steady=None):
+                    steps_per_graph=10, diagnostics=False, steady=None, continue_from=None):
         """Run Q members (`params`: Q tuples (RaQ, gamma, beta); T0: [Q, H, W]) through this ensemble's B slots, each
         `while t < t_end and steps < max_steps` on its own clock as in start_clock (t_end, save_every, t0, max_steps,
         n_step: scalars or one value per member).  When a slot's member stops, the device puts the next queued member
@@ -356,22 +395,39 @@ class EnsembleRollout:
         The slots' T and member rows are rewritten by the sweep (`members` holds the last members afterwards), and
         `time` keeps summing each slot's dt rows: per-member times come from drain().  A second sweep with the same
         number of queued members and ring size reuses the buffers and the captured graphs.
-        diagnostics / steady: as in start_clock; a slot's history and steady state start afresh with each member."""
+        diagnostics / steady: as in start_clock; a slot's history and steady state start afresh with each member.
+        continue_from: None, or one entry per member: p (0 <= p < q, no p twice) makes member q start from the T member p
+        had after its last step, in p's slot, at p's stop step whatever stopped p (include/pbmc.h, pbmc_member_chain);
+        -1 starts q from T0[q] as without it.  T0[q] of a continued member is ignored.  Members with -1 are chain heads
+        and go through the queue rule above among themselves; a member in a chain must be able to take a step
+        (ValueError otherwise: it would break the chain).  A continued member's first drained block also carries
+        `start_T`, its float32 start field."""
         dg = self._new_diag(diagnostics, steady)
         Qa = len(params)
-        T0 = torch.as_tensor(T0).to(torch.float32).reshape(Qa, self.H, self.W)
         bc = lambda x, dt=np.float64: np.broadcast_to(np.asarray(x, dtype=dt), (Qa,)).copy()
         t0, t_end, save_every = bc(t0), bc(t_end), bc(save_every)
         steps0 = bc(n_step, np.int64)
         max_steps = bc(_NO_LIMIT if max_steps is None else max_steps, np.int64)
-        index = np.flatnonzero((t0 < t_end) & (steps0 < max_steps))  # queue entry -> member
+        can_step = (t0 < t_end) & (steps0 < max_steps)
+        cf = None if continue_from is None else _continue_from(continue_from, Qa, can_step)
+        T0 = torch.as_tensor(T0).to(torch.float32).reshape(Qa, self.H, self.W)
+        index = np.flatnonzero(can_step)  # queue entry -> member
         Q = len(index)
+        heads = np.arange(Q)  # queue entries of the chain heads (all entries without chains)
+        if cf is not None and Q:
+            entry = np.full(Qa, -1, dtype=np.int64)
+            entry[index] = np.arange(Q)
+            pred = cf[index]  # each entry's predecessor member, -1: a head
+            heads = np.flatnonzero(pred < 0)
+            succ = np.full(Q, -1, dtype=np.int64)
+            succ[entry[pred[pred >= 0]]] = np.flatnonzero(pred >= 0)
         clk = self._new_clock(snap_slots, steps_per_graph)
         qu = self._queue
         if Q and (qu is None or qu.Q != Q or qu.slots != clk.slots):
             self._graphs = {k: g for k, g in self._graphs.items() if "queue" not in k}
             qu = self._queue = SweepQueue(Q, self.B, self.H, self.W, self.state.dt_seq.shape[0], clk.slots, self.device)
-        n0 = min(self.B, Q)
+        K = len(heads)
+        n0 = min(self.B, K)
         active = np.arange(self.B) < n0
         c = torch.zeros(clk.clock.shape, dtype=torch.float64)
         if Q:
@@ -381,14 +437,18 @@ class EnsembleRollout:
             for name, a in (("t0", t0), ("t_end", t_end), ("save_every", save_every), ("n_step0", steps0), ("max_steps", max_steps)):
                 getattr(qu, name).copy_(torch.from_numpy(a[index]))
             qu.next.fill_(n0)
-            qu.slot_member.copy_(torch.from_numpy(np.where(active, np.arange(self.B), -1)))
+            qu.slot_member.copy_(torch.from_numpy(np.where(active, heads[np.minimum(np.arange(self.B), n0 - 1)], -1)))
             qu.member_seq.fill_(-1)
             qu.snap_member.fill_(-1)
-            # slots without a member keep entry 0's T and row (finite input to the surrogate); their clocks stay inactive
-            fill = torch.from_numpy(np.minimum(np.arange(self.B), n0 - 1)).to(self.device)
+            if cf is not None:
+                qu.heads[:K].copy_(torch.from_numpy(heads))
+                qu.succ.copy_(torch.from_numpy(succ))
+                qu.chain.K = K
+            # slots without a member keep head 0's T and row (finite input to the surrogate); their clocks stay inactive
+            fill = torch.from_numpy(heads[np.minimum(np.arange(self.B), n0 - 1)]).to(self.device)
             self.state.T_seq[self.n_done % 2].copy_(qu.T0[fill])
             self.members.copy_(qu.params[fill])
-            first = index[:n0]
+            first = index[heads[:n0]]
             c[:n0, _T], c[:n0, _T_END] = torch.from_numpy(t0[first]), torch.from_numpy(t_end[first])
             c[:n0, _SAVE_EVERY] = torch.from_numpy(save_every[first])
             ci = c.view(torch.int64)
@@ -398,7 +458,10 @@ class EnsembleRollout:
         self.time.copy_(c[:, _T])
         self._clk, self._diag = clk, dg
         self._pending = None
-        self._sweep = {"index": index, "Q": Q, "next": n0, "t": t0, "steps": steps0, "t_end": t_end, "max_steps": max_steps}
+        self._sweep = {"index": index, "Q": Q, "K": K, "next": n0, "t": t0, "steps": steps0, "t_end": t_end,
+                       "max_steps": max_steps, "chained": cf is not None and Q > 0,
+                       # continued members whose start field drain() has not reported yet: member -> queue entry
+                       "unstarted": {int(index[e]): int(e) for e in range(Q) if cf is not None and cf[index[e]] >= 0}}
         self._host_active = active
 
     def stop_clock(self):
@@ -412,6 +475,10 @@ class EnsembleRollout:
     def _run_queue(self):
         """The SweepQueue the next steps run with (None: no sweep, or a sweep whose members all finished on the host)."""
         return self._queue if self._sweep is not None and self._sweep["Q"] else None
+
+    def _run_chain(self):
+        """The MemberChain the next steps run with (None: no sweep, or a sweep without continue_from)."""
+        return self._queue.chain if self._sweep is not None and self._sweep["chained"] else None
 
     def set_t_end(self, t_end):
         """New end time(s) between blocks: written to the device clock, no re-capture.  A stopped member whose t is now
@@ -434,12 +501,13 @@ class EnsembleRollout:
         read (no device access)."""
         self._require_clock()
         sw = self._sweep
-        return bool(self._host_active.any()) or (sw is not None and sw["next"] < sw["Q"])
+        return bool(self._host_active.any()) or (sw is not None and sw["next"] < sw["K"])
 
     def read_clock(self):
         """The device clocks as numpy arrays: t, t_end, save_t, steps, snaps, drained, active, overflow (synchronises).
         In a sweep (one clock per slot) also slot_member (the member in each slot, -1: none) and next (queued members
-        placed so far).  With diagnostics also steady (the slot's member was stopped by the steady criterion)."""
+        placed so far; with continue_from, chain heads placed so far).  With diagnostics also steady (the slot's member
+        was stopped by the steady criterion)."""
         self._require_clock()
         c = self._clk.clock[:, :_HDR].cpu()
         ci, ci32 = c.view(torch.int64), c.view(torch.int32)
@@ -468,7 +536,8 @@ class EnsembleRollout:
         In a sweep: a dict {member index: logs} over the members that took a step in the block, each with the fields
         above plus `finished` (the member has stopped); t is the cumsum of the member's dt from its own t0.
         With diagnostics, also q_bot, q_top, vrms (float64 [n], one per step taken) and steady (the member has been
-        stopped by the steady criterion)."""
+        stopped by the steady criterion).  In a sweep with continue_from, a continued member's first dict also has
+        start_T: the float32 [H,W] field it started from (its predecessor's T after its last step)."""
         self._require_clock()
         clk = self._clk
         ck = self.read_clock()
@@ -569,6 +638,11 @@ class EnsembleRollout:
                 # t_end / max_steps or, before both, by the criterion (the limits take precedence at the same step)
                 d["steady"] = bool(d["finished"] and sw["t"][m] < sw["t_end"][m] and sw["steps"][m] < sw["max_steps"][m])
             out[m] = d
+        started = [m for m in out if m in sw["unstarted"]]
+        if started:  # written by the hand-off into the member's T0 row, which nothing overwrites afterwards
+            rows = qu.T0[torch.tensor([sw["unstarted"].pop(m) for m in started], device=self.device)].cpu().numpy()
+            for m, f in zip(started, rows):
+                out[m]["start_T"] = f
         occupied = ck["slot_member"] >= 0
         who = ck["slot_member"][occupied]
         if not (np.array_equal(sw["steps"][who], ck["steps"][occupied]) and np.array_equal(sw["t"][who], ck["t"][occupied])):
